@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- headline benchmark of the B200-native multigrid engine.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[3] at N=1, the configuration the metric is quoted on): 3D Poisson
 1025^3 fp64, V(2,2) cycles on the reference problem (f = -3 pi^2 sin sin sin, v = 0 on the boundary).
@@ -20,7 +20,11 @@ One JSON line on stdout (rank 0):
              GPUs, holds the reference's bits.
   other_configs  (N=1) the remaining BASELINE.json configurations, measured in the same process: 1D N=1025, 2D Lyapunov
              1025^2, 3D 257^3, and a non-cubic 3D grid (1025 x 513 x 257); (N=8) the 2049^3 capacity run of configs[4]
-`--impl reference` times that CPU solver as the measured arm instead (no GPU work at all): 513^3, at most 3 cycles.
+`--impl reference` times that CPU solver as the measured arm instead (no GPU work at all): 513^3, K cycles.
+`--dump-outputs DIR` (N=1) writes what the last timed V-cycle left to its caller: v on every level as DIR/v_level<l>.npy (a level of
+more than 2^20 points as a fixed, seeded sample of 2^20 of them; 36 MB in all at 1025^3 fp64) and the level-0 residual norms
+(l2, max) as DIR/residual_norm_level0.npy.  The inputs depend on the arguments only, so two builds can be compared file by file;
+bench_outputs/ (e.g. --dump-outputs bench_outputs/<build>) is git-ignored for such dumps.
 `--profile-traffic` re-measures roofline.traffic with ncu (one launch of the dominant kernel) into profiles/roofline_traffic.json.
 
 Only this file's cpu_baseline / --impl reference legs touch oracle/; the GPU arm never does.
@@ -166,6 +170,23 @@ def parity_block(eng, n, dtype_tag):
                              "(tests/golden/make_hash.py)"}
 
 
+DUMP_POINTS = 1 << 20
+
+
+def dump_outputs(eng, out_dir, norms):
+    """v of every level and (l2, max) of the level-0 residual, as the timed V-cycles left them.  A level of more than DUMP_POINTS
+    points is sampled at DUMP_POINTS flat indices (x fastest) drawn by a generator seeded with the level number, so the same
+    arguments always sample the same points."""
+    os.makedirs(out_dir, exist_ok=True)
+    for l in range(eng.numGrids):
+        v = eng.get_v(l)
+        if v.size > DUMP_POINTS:
+            idx = np.sort(np.random.default_rng(l).choice(v.size, DUMP_POINTS, replace=False))
+            v = v.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, "v_level%d.npy" % l), v)
+    np.save(os.path.join(out_dir, "residual_norm_level0.npy"), np.array(norms, dtype=np.float64))
+
+
 def bind_to_gpu_numa_node(torch, device_index):
     """Host-side plumbing of the end-to-end leg: run this process (and therefore first-touch and pin its host buffers) on the
     NUMA node the GPU hangs off, so that eight ranks do not pull their PCIe traffic across the socket interconnect.
@@ -230,11 +251,10 @@ def run_reference_arm(args):
     if rank != 0:
         return 0
     # the reference at the headline size needs ~40 GB and ~2 min per cycle (tests/golden/make_hash.py ran it once): the arm
-    # samples 513^3 -- one level below, same code path, 1/8 of the points -- for at most 3 cycles and no warm-up
+    # samples 513^3 -- one level below, same code path, 1/8 of the points -- for --steps cycles and no warm-up
     n_sample = args.ref_n
-    steps = max(1, min(args.steps, 3))
-    sec, kind = time_reference_cpu(n_sample, steps, 0)
-    args.steps, args.warmup = steps, 0
+    sec, kind = time_reference_cpu(n_sample, args.steps, 0)
+    args.warmup = 0
     scale = updates_per_cycle(n_sample) / updates_per_cycle(args.n)
     value = scale / sec
     model, cores = host_cpu_info()
@@ -400,7 +420,7 @@ def main():
                     help="finest grid size per axis (2^k+1); under torchrun spell it --grid (torchrun treats --n as an abbreviation of its own options)")
     ap.add_argument("--dtype", default="f64", choices=["f32", "f64"])
     ap.add_argument("--cpu-n", type=int, default=257, help="grid of the bounded CPU-baseline sample of the GPU arm")
-    ap.add_argument("--ref-n", type=int, default=513, help="grid the --impl reference arm runs (at most 3 cycles)")
+    ap.add_argument("--ref-n", type=int, default=513, help="grid the --impl reference arm runs")
     ap.add_argument("--no-other-configs", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--profile-traffic", action="store_true",
@@ -411,7 +431,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--smoother", default="auto", choices=["auto", "colour", "tma", "fused", "pipe"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write v of every level and the level-0 residual "
+                                                           "norms as DIR/<name>.npy (one GPU only)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     if args.impl == "reference":
@@ -430,6 +454,8 @@ def main():
     if args.gpus > 1 and world == 1:
         raise SystemExit("--gpus %d needs one rank per GPU: launch with python -m torch.distributed.run "
                          "--nproc-per-node %d bench.py --gpus %d ..." % (args.gpus, args.gpus, args.gpus))
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs runs on one GPU: each rank of a z-slab run holds only its own planes")
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device: the engine has no CPU path")
     torch.cuda.set_device(local_rank)
@@ -492,6 +518,8 @@ def main():
         ms_total = float(t.item())
     ms_step = ms_total / args.steps
     r1 = eng.residual_norm(0)
+    if args.dump_outputs:
+        dump_outputs(eng, args.dump_outputs, r1)
 
     # ---- second pass of the same K steps with the per-operator CUDA-event timers on (the timers need eager
     #      launches, the headline pass above replays the same kernels from a CUDA graph) ----

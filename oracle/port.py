@@ -248,6 +248,16 @@ class PortBox3D:
         self._call("interpolate", self._p(fine), nx, ny, nz, self._p(coarse))
         return fine
 
+    def apply_correction(self, fine, err):
+        nz, ny, nx = fine.shape
+        self._call("apply_correction", self._p(fine), self._p(err), nx, ny, nz)
+        return fine
+
+    def set_to_value(self, grid, value, modify_boundaries):
+        nz, ny, nx = grid.shape
+        self._call("set", self._p(grid), nx, ny, nz, float(value), 1 if modify_boundaries else 0)
+        return grid
+
     def vcycle(self, l, v1, v2):
         self._call("vcycle", self._pp(self._v), self._pp(self._f), self.n0, self.num_levels, self.range, int(l), int(v1), int(v2), self.corrected)
 

@@ -5,6 +5,7 @@ import ctypes
 import os
 import re
 import subprocess
+import sys
 
 import pytest
 
@@ -46,16 +47,28 @@ def test_header_compiles_as_c_and_cxx(tmp_path):
                         str(tmp_path / ("t_%s.o" % ext))], check=True)
 
 
+NO_DEVICE = r'''
+import sys
+sys.path.insert(0, sys.argv[1])
+import pde_multigrid_b200 as mg
+assert mg.lib().mg_device_count() == 0
+for ctor in (lambda: mg.MultiGrid3D(17), lambda: mg.MultiGrid2D(17), lambda: mg.MultiGrid1D(17), lambda: mg.MultiGrid3DBox((33, 17, 9))):
+    try:
+        ctor()
+    except mg.MGError as e:
+        assert e.code == 2 and "no CPU fallback" in str(e), e
+    else:
+        raise AssertionError("created an engine without a CUDA device")
+print("NO_FALLBACK_OK")
+'''
+
+
 def test_no_cpu_fallback(mg):
-    """Without a CUDA device create() must fail with MG_ERR_CUDA; with one it must succeed."""
-    L = mg.lib()
-    if L.mg_device_count() > 0:
-        pytest.skip("a GPU is present")
-    for ctor in (lambda: mg.MultiGrid3D(17), lambda: mg.MultiGrid2D(17), lambda: mg.MultiGrid1D(17), lambda: mg.MultiGrid3DBox((33, 17, 9))):
-        with pytest.raises(mg.MGError) as ei:
-            ctor()
-        assert ei.value.code == 2
-        assert "no CPU fallback" in str(ei.value)
+    """Without a CUDA device create() must fail with MG_ERR_CUDA.  Checked in a child process that sees no device, so a
+    machine with a GPU checks it as well."""
+    out = subprocess.run([sys.executable, "-c", NO_DEVICE, ROOT], env=dict(os.environ, CUDA_VISIBLE_DEVICES=""), capture_output=True,
+                         text=True, timeout=300)
+    assert out.returncode == 0 and "NO_FALLBACK_OK" in out.stdout, out.stdout + out.stderr
 
 
 def test_argument_validation_precedes_device_probe(mg):
@@ -95,14 +108,19 @@ def test_compat_shim_headers_compile(tmp_path):
 EXAMPLE = os.path.join(ROOT, "tests", "_build", "example_poisson3d")
 
 
-def test_c_example_builds_and_fails_loudly_without_a_gpu(mg):
-    """examples/poisson3d_vcycle.c: the ABI from plain C.  Built into tests/_build/ (shipped to the GPU box); in a
-    container without a GPU it must stop at mg3d_create with the no-CPU-fallback message, not compute anything."""
-    os.makedirs(os.path.dirname(EXAMPLE), exist_ok=True)
+def build_example(src, exe):
+    """Compile examples/<src> against libmg_b200.so into tests/_build/<exe>; the CPU and the GPU tests both call it."""
+    os.makedirs(os.path.dirname(exe), exist_ok=True)
     subprocess.run(["gcc", "-O2", "-Wall", "-Werror", "-I", os.path.join(ROOT, "include"),
-                    os.path.join(ROOT, "examples", "poisson3d_vcycle.c"), "-o", EXAMPLE,
+                    os.path.join(ROOT, "examples", src), "-o", exe,
                     "-L", os.path.join(ROOT, "pde_multigrid_b200"), "-lmg_b200",
                     "-Wl,-rpath,$ORIGIN/../../pde_multigrid_b200", "-lm"], check=True)
+
+
+def test_c_example_builds_and_fails_loudly_without_a_gpu(mg):
+    """examples/poisson3d_vcycle.c: the ABI from plain C.  On a machine without a GPU it must stop at mg3d_create with
+    the no-CPU-fallback message, not compute anything."""
+    build_example("poisson3d_vcycle.c", EXAMPLE)
     import torch
     if not torch.cuda.is_available():
         out = subprocess.run([EXAMPLE, "33", "1"], capture_output=True, text=True)
@@ -110,9 +128,8 @@ def test_c_example_builds_and_fails_loudly_without_a_gpu(mg):
 
 
 @pytest.mark.gpu
-def test_c_example_runs_on_the_gpu():
-    if not os.path.exists(EXAMPLE):
-        pytest.skip("tests/_build/example_poisson3d not built (the CPU test builds it)")
+def test_c_example_runs_on_the_gpu(mg):
+    build_example("poisson3d_vcycle.c", EXAMPLE)
     out = subprocess.run([EXAMPLE, "65", "3"], capture_output=True, text=True, timeout=300)
     assert out.returncode == 0, out.stderr
     norms = [float(l.split("||r||_2 =")[1].split()[0]) for l in out.stdout.splitlines() if "||r||_2 =" in l]
@@ -125,11 +142,7 @@ EXAMPLE_BOX = os.path.join(ROOT, "tests", "_build", "example_poisson3d_box")
 
 
 def test_c_example_for_a_non_cubic_grid_builds(mg):
-    os.makedirs(os.path.dirname(EXAMPLE_BOX), exist_ok=True)
-    subprocess.run(["gcc", "-O2", "-Wall", "-Werror", "-I", os.path.join(ROOT, "include"),
-                    os.path.join(ROOT, "examples", "poisson3d_box.c"), "-o", EXAMPLE_BOX,
-                    "-L", os.path.join(ROOT, "pde_multigrid_b200"), "-lmg_b200",
-                    "-Wl,-rpath,$ORIGIN/../../pde_multigrid_b200", "-lm"], check=True)
+    build_example("poisson3d_box.c", EXAMPLE_BOX)
     import torch
     if not torch.cuda.is_available():
         out = subprocess.run([EXAMPLE_BOX], capture_output=True, text=True)
@@ -137,9 +150,8 @@ def test_c_example_for_a_non_cubic_grid_builds(mg):
 
 
 @pytest.mark.gpu
-def test_c_example_for_a_non_cubic_grid_runs_on_the_gpu():
-    if not os.path.exists(EXAMPLE_BOX):
-        pytest.skip("tests/_build/example_poisson3d_box not built (the CPU test builds it)")
+def test_c_example_for_a_non_cubic_grid_runs_on_the_gpu(mg):
+    build_example("poisson3d_box.c", EXAMPLE_BOX)
     out = subprocess.run([EXAMPLE_BOX, "129", "65", "33", "6"], capture_output=True, text=True, timeout=300)
     assert out.returncode == 0, out.stderr
     assert "5 levels down to 9 x 5 x 3" in out.stdout, out.stdout

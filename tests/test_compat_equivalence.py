@@ -4,7 +4,7 @@ a result: the text dump PrintDiff() writes to log/diff.txt (N3/Grid3D.cpp:136-15
 tests/compat/drv{1,2,3}d.cpp hold the calls of the reference's main()s with PrintDiff() switched on.  In a container with the
 reference (CPU part) they are built twice: with the reference's unmodified .cpp files -- that run produced the committed
 tests/golden/compat_diff_?d.txt (tests/golden/make_compat_golden.py) and is repeated here -- and against include/compat/ +
-libmg_b200.so (binaries in tests/_build/, shipped to the GPU box).  On the GPU the shim binaries must write the same bytes:
+libmg_b200.so (binaries in tests/_build/).  On the GPU the shim binaries must write the same bytes:
 3D 17^3 FMG(2,3,3) (with the reference's own residual signs the iteration blows up, any deviation would be amplified), 2D 33^2
 FMG(1,20,20), 1D 129 FMG(2,100,100); and a non-cubic 33 x 17 x 9 grid (FMG(2,3,3) plus a hand-made cycle through the free-array
 operators) whose reference side is the same classes compiled with -DNDEBUG.
@@ -38,6 +38,15 @@ def shim_cmd(src, out, cuda_face=False):
     return cmd
 
 
+def build_driver(dim, cuda_face=False):
+    """tests/compat/drv<dim>[_cuda].cpp against the shim -> tests/_build/eq_{shim,cuda}_<dim>; the CPU and the GPU tests both call it."""
+    os.makedirs(BUILD, exist_ok=True)
+    src = os.path.join(ROOT, "tests", "compat", "drv%s%s.cpp" % (dim, "_cuda" if cuda_face else ""))
+    exe = os.path.join(BUILD, "eq_%s_%s" % ("cuda" if cuda_face else "shim", dim))
+    subprocess.run(shim_cmd(src, exe, cuda_face), check=True)
+    return exe
+
+
 @pytest.mark.skipif(not os.path.isdir(REF), reason="reference sources not mounted")
 @pytest.mark.parametrize("dim", ["1d", "2d", "3d", "3d_box"])
 def test_reference_classes_reproduce_the_committed_dump(dim, tmp_path):
@@ -51,23 +60,18 @@ def test_reference_classes_reproduce_the_committed_dump(dim, tmp_path):
 
 @pytest.mark.parametrize("dim", ["1d", "2d", "3d", "3d_box"])
 def test_shim_side_builds(mg, dim):
-    os.makedirs(BUILD, exist_ok=True)
-    subprocess.run(shim_cmd(os.path.join(ROOT, "tests", "compat", "drv%s.cpp" % dim), os.path.join(BUILD, "eq_shim_" + dim)), check=True)
+    build_driver(dim)
 
 
 @pytest.mark.parametrize("dim", ["1d", "2d", "3d"])
 def test_cuda_tesi_faces_build(mg, dim):
-    os.makedirs(BUILD, exist_ok=True)
-    subprocess.run(shim_cmd(os.path.join(ROOT, "tests", "compat", "drv%s_cuda.cpp" % dim), os.path.join(BUILD, "eq_cuda_" + dim), True),
-                   check=True)
+    build_driver(dim, cuda_face=True)
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("dim", ["1d", "2d", "3d", "3d_box"])
-def test_shim_writes_the_reference_dump_byte_for_byte(dim, tmp_path):
-    exe = os.path.join(BUILD, "eq_shim_" + dim)
-    if not os.path.exists(exe):
-        pytest.skip("tests/_build/eq_shim_%s not built (the CPU tests build it)" % dim)
+def test_shim_writes_the_reference_dump_byte_for_byte(mg, dim, tmp_path):
+    exe = build_driver(dim)
     (tmp_path / "log").mkdir()
     out = subprocess.run([exe] + list(ARGS[dim]), cwd=str(tmp_path), capture_output=True, text=True, timeout=600)
     assert out.returncode == 0, out.stderr
@@ -80,9 +84,7 @@ def test_shim_writes_the_reference_dump_byte_for_byte(dim, tmp_path):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("dim", ["1d", "2d", "3d"])
-def test_cuda_tesi_faces_run(dim, tmp_path):
-    exe = os.path.join(BUILD, "eq_cuda_" + dim)
-    if not os.path.exists(exe):
-        pytest.skip("tests/_build/eq_cuda_%s not built (the CPU tests build it)" % dim)
+def test_cuda_tesi_faces_run(mg, dim, tmp_path):
+    exe = build_driver(dim, cuda_face=True)
     out = subprocess.run([exe], cwd=str(tmp_path), capture_output=True, text=True, timeout=600)
     assert out.returncode == 0 and "CUDA_FACE OK" in out.stdout, out.stdout + out.stderr

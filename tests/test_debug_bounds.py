@@ -9,6 +9,8 @@ import sys
 
 import pytest
 
+from pde_multigrid_b200.build import build_debug_bounds
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 DBG = os.path.join(ROOT, "pde_multigrid_b200", "libmg_b200_dbg.so")
 
@@ -31,18 +33,21 @@ print("RETURNED", float(buf[: 2 * hp * n * n].sum()))
 '''
 
 
-def test_checking_build_compiles(mg):
-    from pde_multigrid_b200 import build as b
-    so = b.build_debug_bounds()
+@pytest.fixture(scope="module")
+def dbg(mg):
+    """The checking build, compiled afresh once per run: a library left over from older sources would be tested instead."""
+    return build_debug_bounds()
+
+
+def test_checking_build_compiles(dbg):
+    so = dbg
     assert so == DBG and os.path.exists(DBG)
     syms = subprocess.run(["nm", "-D", "--defined-only", DBG], capture_output=True, text=True).stdout
     assert "mg3d_vcycle" in syms
 
 
 @pytest.mark.gpu
-def test_every_kernel_family_runs_clean_under_the_bounds_checks():
-    if not os.path.exists(DBG):
-        pytest.skip("libmg_b200_dbg.so not built (the CPU test builds it)")
+def test_every_kernel_family_runs_clean_under_the_bounds_checks(dbg):
     env = dict(os.environ, MG_B200_LIB=DBG)
     out = subprocess.run([sys.executable, os.path.join(ROOT, "scripts", "sanitize_smoke.py")], cwd=ROOT, env=env, capture_output=True,
                          text=True, timeout=900)
@@ -50,9 +55,7 @@ def test_every_kernel_family_runs_clean_under_the_bounds_checks():
 
 
 @pytest.mark.gpu
-def test_an_out_of_range_launch_is_reported():
-    if not os.path.exists(DBG):
-        pytest.skip("libmg_b200_dbg.so not built (the CPU test builds it)")
+def test_an_out_of_range_launch_is_reported(dbg):
     env = dict(os.environ, MG_B200_LIB=DBG)
     out = subprocess.run([sys.executable, "-c", BAD], cwd=ROOT, env=env, capture_output=True, text=True, timeout=300)
     # the three planes past the end are reported by every thread that would have written them, and nothing is written there

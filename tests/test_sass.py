@@ -1,6 +1,7 @@
 """CPU test (no GPU needed): the built library really carries the Blackwell data path the design claims -- sm_100a cubins whose
 hot kernels issue TMA tensor loads (UTMALDG) tracked by mbarriers (SYNCS), and no library kernels.  Reads the SASS of
 pde_multigrid_b200/libmg_b200.so with cuobjdump (B200_PROFILING.md names these mnemonics as the proof of TMA use)."""
+import os
 import re
 import shutil
 import subprocess
@@ -10,10 +11,12 @@ import pytest
 
 @pytest.fixture(scope="module")
 def sass(mg):
-    if shutil.which("cuobjdump") is None:
-        pytest.skip("cuobjdump not on PATH")
+    from pde_multigrid_b200 import build
+    cuobjdump = shutil.which("cuobjdump") or os.path.join(os.path.dirname(build.NVCC), "cuobjdump")  # else the toolkit that built the library
+    if not os.path.exists(cuobjdump):
+        pytest.skip("cuobjdump not found")
     import pde_multigrid_b200._lib as L
-    out = subprocess.run(["cuobjdump", "-sass", L.SO_PATH], capture_output=True, text=True, check=True).stdout
+    out = subprocess.run([cuobjdump, "-sass", L.SO_PATH], capture_output=True, text=True, check=True).stdout
     kernels, cur = {}, None
     for line in out.splitlines():
         m = re.search(r"Function : (\S+)", line)
