@@ -141,6 +141,19 @@ int mg3d_interpolate_correct(mg3d_t* mg, int fine_level);           /* Interpola
 int mg3d_set_to_value(mg3d_t* mg, int level, int field, double value, int modify_boundaries); /* setToValue / Set */
 int mg3d_vcycle(mg3d_t* mg, int level, int v1, int v2);             /* VCycle(gridID, v1, v2) */
 int mg3d_fmg(mg3d_t* mg, int level, int v0, int v1, int v2);        /* FullMultiGridVCycle(gridID, v0, v1, v2) */
+/* V-cycles VCycle(level, v1, v2) from the current v of `level` until
+ *     ||r_k||_2 <= max(atol, rtol * ||r_0||_2)
+ * or max_cycles cycles have run.  r_k is the residual after k cycles, the same residual and the same reduction as
+ * mg3d_residual_norm(level) (the reference has no norm: SURVEY.md 8c).
+ * cycles_out: cycles run (0 if r_0 already meets the target).  converged_out: 1 / 0.
+ * history: NULL, or room for 2*(max_cycles+1) doubles, receives (l2, linf) of r_0 .. r_cycles.
+ * A non-finite l2 stops the solve with converged = 0.  Not converging is not an error: MG_OK is returned.
+ * rtol, atol >= 0, max_cycles >= 0, v1, v2 >= 0, otherwise MG_ERR_ARG and nothing runs.
+ * Synchronous: returns when the solve has finished.  On one GPU the loop runs on the device (a CUDA graph with a WHILE
+ * node: one launch and one wait per solve); distributed handles, MG_B200_NO_GRAPH and per-operator profiling drive it
+ * from the host, one read-back per cycle.  Both give the same bits.  The mg3b / mg2d / mg1d versions are the same. */
+int mg3d_solve(mg3d_t* mg, int level, int v1, int v2, double rtol, double atol, int max_cycles,
+               int* cycles_out, int* converged_out, double* history);
 
 /* reference-facing calls on HOST arrays (NOCUDA signatures, N3/MultiGrid3D.h:16-27): upload, run, download */
 int mg3d_restrict_host(mg3d_t* mg, const void* fine, const int fsize_xyz[3], void* coarse, const int csize_xyz[3]);
@@ -189,6 +202,8 @@ int mg3b_interpolate_correct(mg3b_t* mg, int fine_level);            /* Interpol
 int mg3b_set_to_value(mg3b_t* mg, int level, int field, double value, int modify_boundaries);
 int mg3b_vcycle(mg3b_t* mg, int level, int v1, int v2);              /* VCycle */
 int mg3b_fmg(mg3b_t* mg, int level, int v0, int v1, int v2);         /* FullMultiGridVCycle */
+int mg3b_solve(mg3b_t* mg, int level, int v1, int v2, double rtol, double atol, int max_cycles,
+               int* cycles_out, int* converged_out, double* history); /* as mg3d_solve */
 int mg3b_vcycle_host(mg3b_t* mg, void* v_host, const void* f_host, int v1, int v2, int cycles);
 /* the operators on caller-owned HOST arrays (N3/MultiGrid3D.h:16-27 with three different sizes) */
 int mg3b_restrict_host(mg3b_t* mg, const void* fine, const int fsize_xyz[3], void* coarse, const int csize_xyz[3]);
@@ -223,6 +238,8 @@ int mg2d_interpolate_correct(mg2d_t* mg, int fine_level);
 int mg2d_set_to_value(mg2d_t* mg, int level, int field, double value, int modify_boundaries);
 int mg2d_vcycle(mg2d_t* mg, int level, int v1, int v2);
 int mg2d_fmg(mg2d_t* mg, int level, int v0, int v1, int v2);
+int mg2d_solve(mg2d_t* mg, int level, int v1, int v2, double rtol, double atol, int max_cycles,
+               int* cycles_out, int* converged_out, double* history); /* as mg3d_solve */
 int mg2d_mean_abs_error(mg2d_t* mg, double* mae); /* PrintMeanAbsoluteError, C2/Grid2D.cu:123-154 */
 int mg2d_restrict_host(mg2d_t* mg, const void* fine, const int fsize_xy[2], void* coarse, const int csize_xy[2]);
 int mg2d_interpolate_host(mg2d_t* mg, void* fine, const int fsize_xy[2], const void* coarse, const int csize_xy[2]);
@@ -266,6 +283,8 @@ int mg1d_interpolate_correct(mg1d_t* mg, int fine_level);
 int mg1d_set_to_value(mg1d_t* mg, int level, int field, double value, int modify_boundaries);
 int mg1d_vcycle(mg1d_t* mg, int level, int v1, int v2);
 int mg1d_fmg(mg1d_t* mg, int level, int v0, int v1, int v2);
+int mg1d_solve(mg1d_t* mg, int level, int v1, int v2, double rtol, double atol, int max_cycles,
+               int* cycles_out, int* converged_out, double* history); /* as mg3d_solve */
 int mg1d_restrict_host(mg1d_t* mg, const void* fine, int fsize, void* coarse, int csize);
 int mg1d_interpolate_host(mg1d_t* mg, void* fine, int fsize, const void* coarse, int csize);
 int mg1d_apply_correction_host(mg1d_t* mg, void* fine, int fsize, const void* error, int esize);

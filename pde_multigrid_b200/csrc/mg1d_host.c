@@ -26,6 +26,9 @@ struct mg1d_s {
     double* h_out2;
     long long launches;
     mg_prof prof;
+    int use_graphs;   /* 0: MG_B200_NO_GRAPH, mg1d_solve runs host-driven */
+    mg_solver solver; /* mg1d_solve: parameter block and history on the device */
+    mg_solve_slot solves[MG_SOLVE_SLOTS];
 };
 
 #define PROF_BEGIN(mg, level, op) mg_prof_begin(&(mg)->prof, (mg)->stream, (level), (op), (mg)->launches)
@@ -55,6 +58,7 @@ int mg1d_create(mg1d_t** out, int n, const double range[2], int dtype, int resid
     if (!mg) return mg_fail(MG_ERR_NOMEM, "host allocation failed");
     mg->dtype = dtype;
     mg->mode = residual_mode;
+    mg->use_graphs = getenv("MG_B200_NO_GRAPH") ? 0 : 1;
     mg->range[0] = range[0];
     mg->range[1] = range[1];
     mg->H.nlevels = mg_num_levels_for(n);
@@ -88,7 +92,9 @@ int mg1d_create(mg1d_t** out, int n, const double range[2], int dtype, int resid
 int mg1d_destroy(mg1d_t* mg)
 {
     if (!mg) return MG_OK;
-    if (mg->stream) { cudaStreamSynchronize(mg->stream); cudaStreamDestroy(mg->stream); }
+    if (mg->stream) cudaStreamSynchronize(mg->stream);
+    mg_solve_free(&mg->solver, mg->solves);
+    if (mg->stream) cudaStreamDestroy(mg->stream);
     if (mg->arena) cudaFree(mg->arena);
     if (mg->d_out2) cudaFree(mg->d_out2);
     if (mg->h_out2) cudaFreeHost(mg->h_out2);
@@ -269,11 +275,18 @@ int mg1d_abs_error(mg1d_t* mg, int level, double* mean_abs, double* max_abs)
     return MG_OK;
 }
 
+/* the norm pass of mg1d_residual_norm: {sum of r^2, max |r|} into d_out2, nothing read back */
+static int residual_norm_enqueue(mg1d_t* mg, int level)
+{
+    MG_LAUNCH(mg->launches, mgk1d_residual_norm(mg->stream, mg->dtype, mg->arena, mg->H, level, mg->mode == MG_CORRECTED, mg->d_out2));
+    return MG_OK;
+}
+
 int mg1d_residual_norm(mg1d_t* mg, int level, double* l2, double* linf)
 {
     int st = check_level(mg, level);
     if (st) return st;
-    MG_LAUNCH(mg->launches, mgk1d_residual_norm(mg->stream, mg->dtype, mg->arena, mg->H, level, mg->mode == MG_CORRECTED, mg->d_out2));
+    if ((st = residual_norm_enqueue(mg, level))) return st;
     MG_CUDA(cudaMemcpyAsync(mg->h_out2, mg->d_out2, 2 * sizeof(double), cudaMemcpyDeviceToHost, mg->stream));
     MG_CUDA(cudaStreamSynchronize(mg->stream));
     if (l2) *l2 = sqrt(mg->h_out2[0]);
@@ -346,6 +359,31 @@ int mg1d_vcycle(mg1d_t* mg, int level, int v1, int v2)
     MG_LAUNCH(mg->launches, mgk1d_cycle(mg->stream, mg->dtype, mg->arena, mg->H, level, 1, v1, v2, mg->mode == MG_CORRECTED, 0));
     PROF_END(mg);
     return MG_OK;
+}
+
+/* tolerance-driven solve (mg_host_common.c builds and runs it): the body is the one-launch cycle, the norm and the check */
+typedef struct {
+    mg1d_t* mg;
+    int level, v1, v2;
+} solve1d_ctx;
+
+static int s1_norm(void* c) { solve1d_ctx* x = (solve1d_ctx*)c; return residual_norm_enqueue(x->mg, x->level); }
+static int s1_cycle(void* c) { solve1d_ctx* x = (solve1d_ctx*)c; return mg1d_vcycle(x->mg, x->level, x->v1, x->v2); }
+
+int mg1d_solve(mg1d_t* mg, int level, int v1, int v2, double rtol, double atol, int max_cycles, int* cycles_out, int* converged_out,
+               double* history)
+{
+    int st = check_level(mg, level);
+    if (st) return st;
+    if ((st = mg_solve_check_args(rtol, atol, max_cycles, v1, v2))) return st;
+    solve1d_ctx x = {mg, level, v1, v2};
+    const mg_solve_ops ops = {&x, mg->stream, mg->d_out2, &mg->launches, s1_norm, s1_cycle, s1_cycle, NULL, NULL};
+    mg_solve_slot* slot = NULL;
+    if (mg->use_graphs && !mg->prof.enabled) {
+        const int key[MG_SOLVE_KEY] = {level, v1, v2, 0, 0, 0};
+        slot = mg_solve_slot_for(mg->solves, key);
+    }
+    return mg_solve_run(&ops, &mg->solver, slot, rtol, atol, max_cycles, cycles_out, converged_out, history);
 }
 
 /* FullMultiGridVCycle (N1/MultiGrid1D.cpp:132-148): one launch */

@@ -40,6 +40,8 @@ struct mg2d_s {
     double* h_out2;
     long long launches;
     mg_prof prof;
+    mg_solver solver; /* mg2d_solve: parameter block and history on the device */
+    mg_solve_slot solves[MG_SOLVE_SLOTS];
 };
 
 #define PROF_BEGIN(mg, level, op) mg_prof_begin(&(mg)->prof, (mg)->stream, (level), (op), (mg)->launches)
@@ -137,6 +139,7 @@ int mg2d_destroy(mg2d_t* mg)
     if (mg->stream) cudaStreamSynchronize(mg->stream);
     for (int i = 0; i < MG2_GRAPH_SLOTS; i++)
         if (mg->graphs[i].used && mg->graphs[i].exec) cudaGraphExecDestroy(mg->graphs[i].exec);
+    mg_solve_free(&mg->solver, mg->solves);
     if (mg->stream) cudaStreamDestroy(mg->stream);
     if (mg->arena) cudaFree(mg->arena);
     if (mg->d_scratch) cudaFree(mg->d_scratch);
@@ -275,12 +278,19 @@ static int read_out2(mg2d_t* mg)
     return MG_OK;
 }
 
+/* the norm pass of mg2d_residual_norm: {sum of r^2, max |r|} into d_scratch + 2*SCRATCH_PARTS, nothing read back */
+static int residual_norm_enqueue(mg2d_t* mg, int level)
+{
+    mg_level2d* L = &mg->lv[level];
+    MG_LAUNCH(mg->launches, mgk2d_residual_norm(mg->stream, mg->dtype, L->v, L->f, L->g, L->c, mg->d_scratch, mg->d_scratch + 2 * SCRATCH_PARTS));
+    return MG_OK;
+}
+
 int mg2d_residual_norm(mg2d_t* mg, int level, double* l2, double* linf)
 {
     int st = check_level(mg, level);
     if (st) return st;
-    mg_level2d* L = &mg->lv[level];
-    MG_LAUNCH(mg->launches, mgk2d_residual_norm(mg->stream, mg->dtype, L->v, L->f, L->g, L->c, mg->d_scratch, mg->d_scratch + 2 * SCRATCH_PARTS));
+    if ((st = residual_norm_enqueue(mg, level))) return st;
     st = read_out2(mg);
     if (st) return st;
     if (l2) *l2 = sqrt(mg->h_out2[0]);
@@ -414,6 +424,33 @@ int mg2d_vcycle(mg2d_t* mg, int level, int v1, int v2)
     MG_CUDA(cudaGraphLaunch(g->exec, mg->stream));
     mg->launches += g->launches;
     return MG_OK;
+}
+
+/* tolerance-driven solve (mg_host_common.c builds and runs it) */
+typedef struct {
+    mg2d_t* mg;
+    int level, v1, v2;
+} solve2d_ctx;
+
+static int s2_norm(void* c) { solve2d_ctx* x = (solve2d_ctx*)c; return residual_norm_enqueue(x->mg, x->level); }
+static int s2_cycle(void* c) { solve2d_ctx* x = (solve2d_ctx*)c; return mg2d_vcycle(x->mg, x->level, x->v1, x->v2); }
+static int s2_capture(void* c) { solve2d_ctx* x = (solve2d_ctx*)c; return vcycle_rec(x->mg, x->level, x->v1, x->v2); }
+
+int mg2d_solve(mg2d_t* mg, int level, int v1, int v2, double rtol, double atol, int max_cycles, int* cycles_out, int* converged_out,
+               double* history)
+{
+    int st = check_level(mg, level);
+    if (st) return st;
+    if ((st = mg_solve_check_args(rtol, atol, max_cycles, v1, v2))) return st;
+    solve2d_ctx x = {mg, level, v1, v2};
+    const mg_solve_ops ops = {&x, mg->stream, mg->d_scratch + 2 * SCRATCH_PARTS, &mg->launches, s2_norm, s2_cycle, s2_capture, NULL, NULL};
+    mg_solve_slot* slot = NULL;
+    const long long per_cycle = 2LL * (v1 + v2) * (mg->nlevels - level);
+    if (mg->use_graphs && !mg->prof.enabled && per_cycle <= 4096) {
+        const int key[MG_SOLVE_KEY] = {level, v1, v2, 0, 0, 0};
+        slot = mg_solve_slot_for(mg->solves, key);
+    }
+    return mg_solve_run(&ops, &mg->solver, slot, rtol, atol, max_cycles, cycles_out, converged_out, history);
 }
 
 /* FullMultiGridVCycle, N2/MultiGrid2D.cpp:296-312 */

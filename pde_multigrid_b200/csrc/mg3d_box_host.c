@@ -40,6 +40,9 @@ struct mg3b_s {
     double* d_tables;  /* sin tables of InitF: nx + ny + nz doubles of the finest level */
     double* h_out2;    /* pinned */
     long long launches;
+    int use_graphs;    /* 0: MG_B200_NO_GRAPH, mg3b_solve runs host-driven */
+    mg_solver solver;  /* mg3b_solve: parameter block and history on the device */
+    mg_solve_slot solves[MG_SOLVE_SLOTS];
 };
 
 static size_t level_count(const mg_level3b* L) { return (size_t)L->n[0] * (size_t)L->n[1] * (size_t)L->n[2]; }
@@ -105,6 +108,7 @@ int mg3b_destroy(mg3b_t* mg)
 {
     if (!mg) return MG_OK;
     if (mg->stream) cudaStreamSynchronize(mg->stream);
+    mg_solve_free(&mg->solver, mg->solves);
     if (mg->arena) cudaFree(mg->arena);
     if (mg->staging) cudaFree(mg->staging);
     if (mg->d_scratch) cudaFree(mg->d_scratch);
@@ -135,6 +139,7 @@ int mg3b_create(mg3b_t** out, const int finest_size_xyz[3], const double range[6
     if (!mg) return mg_fail(MG_ERR_NOMEM, "host allocation failed");
     mg->dtype = dtype;
     mg->mode = residual_mode;
+    mg->use_graphs = getenv("MG_B200_NO_GRAPH") ? 0 : 1;
     memcpy(mg->range, range, sizeof mg->range);
     int mn = finest_size_xyz[0];
     if (finest_size_xyz[1] < mn) mn = finest_size_xyz[1];
@@ -299,13 +304,21 @@ int mg3b_residual(mg3b_t* mg, int level, void* host_out)
     return MG_OK;
 }
 
+/* the norm pass of mg3b_residual_norm: {sum of r^2, max |r|} into d_scratch + 2*MG3B_NPARTS, nothing read back */
+static int residual_norm_enqueue(mg3b_t* mg, int level)
+{
+    mg_level3b* L = &mg->lv[level];
+    MG_LAUNCH(mg->launches, mgk3b_residual_norm(mg->stream, mg->dtype, L->v, L->f, L->g, L->c, mg->mode == MG_CORRECTED, mg->d_scratch, MG3B_NPARTS,
+                                                mg->d_scratch + 2 * MG3B_NPARTS));
+    return MG_OK;
+}
+
 int mg3b_residual_norm(mg3b_t* mg, int level, double* l2, double* linf)
 {
     int st = check_level(mg, level);
     if (st) return st;
-    mg_level3b* L = &mg->lv[level];
+    if ((st = residual_norm_enqueue(mg, level))) return st;
     double* out2 = mg->d_scratch + 2 * MG3B_NPARTS;
-    MG_LAUNCH(mg->launches, mgk3b_residual_norm(mg->stream, mg->dtype, L->v, L->f, L->g, L->c, mg->mode == MG_CORRECTED, mg->d_scratch, MG3B_NPARTS, out2));
     MG_CUDA(cudaMemcpyAsync(mg->h_out2, out2, 2 * sizeof(double), cudaMemcpyDeviceToHost, mg->stream));
     MG_CUDA(cudaStreamSynchronize(mg->stream));
     if (l2) *l2 = sqrt(mg->h_out2[0]);
@@ -392,6 +405,32 @@ int mg3b_vcycle(mg3b_t* mg, int level, int v1, int v2)
     if (st) return st;
     if (v1 < 0 || v2 < 0) return mg_fail(MG_ERR_ARG, "negative sweep count");
     return vcycle_rec(mg, level, v1, v2);
+}
+
+/* tolerance-driven solve (mg_host_common.c builds and runs it) */
+typedef struct {
+    mg3b_t* mg;
+    int level, v1, v2;
+} solve3b_ctx;
+
+static int s3b_norm(void* c) { solve3b_ctx* x = (solve3b_ctx*)c; return residual_norm_enqueue(x->mg, x->level); }
+static int s3b_cycle(void* c) { solve3b_ctx* x = (solve3b_ctx*)c; return vcycle_rec(x->mg, x->level, x->v1, x->v2); }
+
+int mg3b_solve(mg3b_t* mg, int level, int v1, int v2, double rtol, double atol, int max_cycles, int* cycles_out, int* converged_out,
+               double* history)
+{
+    int st = check_level(mg, level);
+    if (st) return st;
+    if ((st = mg_solve_check_args(rtol, atol, max_cycles, v1, v2))) return st;
+    solve3b_ctx x = {mg, level, v1, v2};
+    const mg_solve_ops ops = {&x, mg->stream, mg->d_scratch + 2 * MG3B_NPARTS, &mg->launches, s3b_norm, s3b_cycle, s3b_cycle, NULL, NULL};
+    mg_solve_slot* slot = NULL;
+    const long long per_cycle = 2LL * (v1 + v2) * (mg->nlevels - level);
+    if (mg->use_graphs && per_cycle <= 4096) {
+        const int key[MG_SOLVE_KEY] = {level, v1, v2, 0, 0, 0};
+        slot = mg_solve_slot_for(mg->solves, key);
+    }
+    return mg_solve_run(&ops, &mg->solver, slot, rtol, atol, max_cycles, cycles_out, converged_out, history);
 }
 
 /* FullMultiGridVCycle, N3/MultiGrid3D.cpp:569-585 */

@@ -129,6 +129,8 @@ struct mg3d_s {
     unsigned int* d_flag; /* {exactness flag of the pipelined smoother, completion counter of its fallback} */
     int no_tail;         /* MG_B200_NO_TAIL: coarse levels as separate launches */
     int full_correction; /* MG_B200_FULL_CORRECTION: correct both colours after prolongation inside a cycle */
+    mg_solver solver;    /* mg3d_solve: parameter block and history on the device */
+    mg_solve_slot solves[MG_SOLVE_SLOTS]; /* mg3d_solve graphs, apart from the cycle graphs above */
 };
 
 #define PROF_BEGIN(mg, level, op) mg_prof_begin(&(mg)->prof, (mg)->stream, (level), (op), (mg)->launches)
@@ -750,6 +752,7 @@ int mg3d_destroy(mg3d_t* mg)
     if (mg->stream) cudaStreamSynchronize(mg->stream);
     for (int i = 0; i < MG_GRAPH_SLOTS; i++)
         if (mg->graphs[i].used && mg->graphs[i].exec) cudaGraphExecDestroy(mg->graphs[i].exec);
+    mg_solve_free(&mg->solver, mg->solves);
     p2p_teardown(mg);
     if (mg->comm) mg_comm_destroy(mg->comm);
     if (mg->cstream) { cudaStreamSynchronize(mg->cstream); cudaStreamDestroy(mg->cstream); }
@@ -824,6 +827,11 @@ int mg3d_set_jacobi_weight(mg3d_t* mg, double omega)
         if (mg->graphs[i].used && mg->graphs[i].smoother == MG_SMOOTHER_JACOBI) {
             if (mg->graphs[i].exec) cudaGraphExecDestroy(mg->graphs[i].exec);
             memset(&mg->graphs[i], 0, sizeof mg->graphs[i]);
+        }
+    for (int i = 0; i < MG_SOLVE_SLOTS; i++) /* key[3] = smoother */
+        if (mg->solves[i].used && mg->solves[i].key[3] == MG_SMOOTHER_JACOBI) {
+            if (mg->solves[i].exec) cudaGraphExecDestroy(mg->solves[i].exec);
+            memset(&mg->solves[i], 0, sizeof mg->solves[i]);
         }
     return MG_OK;
 }
@@ -1234,13 +1242,16 @@ int mg3d_residual(mg3d_t* mg, int level, void* host_out)
 
 static void coarse_share(const mg3d_t* mg, int fine_level, int* czl_lo, int* czl_hi);
 
-int mg3d_residual_norm(mg3d_t* mg, int level, double* l2, double* linf)
+/* the norm pass of mg3d_residual_norm: {sum of r^2, max |r|} of `level` into norm_out2 (all-reduced over the ranks of a
+   distributed level); nothing is read back */
+static double* norm_out2(mg3d_t* mg) { return mg->d_scratch + 2 * MGK_NORM_MAX_PARTS; }
+
+static int residual_norm_enqueue(mg3d_t* mg, int level)
 {
-    int st = check_level(mg, level);
-    if (st) return st;
     mg_level3d* L = &mg->lv[level];
+    int st;
     if ((st = ensure_v_ghosts(mg, level))) return st;
-    double* out2 = mg->d_scratch + 2 * MGK_NORM_MAX_PARTS;
+    double* out2 = norm_out2(mg);
     int k = -2;
     if (L->has_tma && mg->smoother != MG_SMOOTHER_COLOUR && level + 1 < mg->nlevels) {
         /* large levels: the staging of the fused residual+restrict kernel; the coarse planes this rank restricts to
@@ -1256,7 +1267,15 @@ int mg3d_residual_norm(mg3d_t* mg, int level, double* l2, double* linf)
         MG_LAUNCH(mg->launches, mgk3d_residual_norm(mg->stream, mg->dtype, L->v, L->f, L->g, L->c, mg->mode == MG_CORRECTED,
                                                     L->own_lo, L->own_hi, mg->d_scratch, out2));
     if (L->dist && (st = mg_comm_allreduce_sum_max(mg->comm, out2, mg->stream))) return st;
-    MG_CUDA(cudaMemcpyAsync(mg->h_out2, out2, 2 * sizeof(double), cudaMemcpyDeviceToHost, mg->stream));
+    return MG_OK;
+}
+
+int mg3d_residual_norm(mg3d_t* mg, int level, double* l2, double* linf)
+{
+    int st = check_level(mg, level);
+    if (st) return st;
+    if ((st = residual_norm_enqueue(mg, level))) return st;
+    MG_CUDA(cudaMemcpyAsync(mg->h_out2, norm_out2(mg), 2 * sizeof(double), cudaMemcpyDeviceToHost, mg->stream));
     MG_CUDA(cudaStreamSynchronize(mg->stream));
     if (l2) *l2 = sqrt(mg->h_out2[0]);
     if (linf) *linf = mg->h_out2[1];
@@ -1586,6 +1605,64 @@ int mg3d_vcycle(mg3d_t* mg, int level, int v1, int v2)
     mg->launches += g->launches;
     mg->halo_bytes += g->halo_bytes;
     return MG_OK;
+}
+
+/* ---- tolerance-driven solve (mg_host_common.c builds and runs it) ---------------------------------------------- */
+
+typedef struct {
+    mg3d_t* mg;
+    int level, v1, v2;
+} solve3d_ctx;
+
+static int s3_norm(void* c) { solve3d_ctx* x = (solve3d_ctx*)c; return residual_norm_enqueue(x->mg, x->level); }
+static int s3_cycle(void* c) { solve3d_ctx* x = (solve3d_ctx*)c; return mg3d_vcycle(x->mg, x->level, x->v1, x->v2); }
+static int s3_capture(void* c) { solve3d_ctx* x = (solve3d_ctx*)c; return vcycle_rec(x->mg, x->level, x->v1, x->v2); }
+
+/* [0] = which v buffer every level works on; [1] = the ghost-validity flags.  Only [0] changes the kernels of a cycle on
+   one GPU (the flags steer the exchanges of distributed levels), so only [0] has to return to its start value; [1] is
+   restored so that later mg3d_vcycle calls find the graphs the hand-written loop would find. */
+static void s3_save(void* c, unsigned out[2])
+{
+    const mg3d_t* mg = ((solve3d_ctx*)c)->mg;
+    out[0] = out[1] = 0;
+    for (int l = 0; l < mg->nlevels && l < 32; l++) {
+        out[0] |= (unsigned)mg->lv[l].cur << l;
+        if (l < 16) out[1] |= ((unsigned)(mg->lv[l].vg_valid != 0) | ((unsigned)(mg->lv[l].vg_deep != 0) << 1)) << (2 * l);
+    }
+}
+
+static void s3_load(void* c, const unsigned in[2])
+{
+    mg3d_t* mg = ((solve3d_ctx*)c)->mg;
+    for (int l = 0; l < mg->nlevels && l < 32; l++) {
+        mg->lv[l].cur = (int)((in[0] >> l) & 1u);
+        mg->lv[l].v = mg->lv[l].vbuf[mg->lv[l].cur];
+        mg->lv[l].vg_valid = l < 16 ? (int)((in[1] >> (2 * l)) & 1u) : 1;
+        mg->lv[l].vg_deep = l < 16 ? (int)((in[1] >> (2 * l + 1)) & 1u) : 0;
+    }
+}
+
+int mg3d_solve(mg3d_t* mg, int level, int v1, int v2, double rtol, double atol, int max_cycles, int* cycles_out, int* converged_out,
+               double* history)
+{
+    int st = check_level(mg, level);
+    if (st) return st;
+    if ((st = mg_solve_check_args(rtol, atol, max_cycles, v1, v2))) return st;
+    solve3d_ctx x = {mg, level, v1, v2};
+    const mg_solve_ops ops = {&x, mg->stream, norm_out2(mg), &mg->launches, s3_norm, s3_cycle, s3_capture, s3_save, s3_load};
+    mg_solve_slot* slot = NULL;
+    /* A distributed solve stays host-driven: a conditional body may hold kernels, copies, memsets and nested graphs only,
+       and the NCCL all-reduce of the norm is not known to stay inside that set.  Every rank checks the same all-reduced
+       norm, so every rank stops after the same cycle. */
+    const long long per_cycle = 2LL * (v1 + v2) * (mg->nlevels - level) * 2;
+    if (mg->nranks == 1 && mg->use_graphs && !mg->prof.enabled && per_cycle <= 4096) {
+        unsigned state[2];
+        s3_save(&x, state);
+        const int key[MG_SOLVE_KEY] = {level, v1, v2, mg->smoother, mg->arith, (int)state[0]};
+        slot = mg_solve_slot_for(mg->solves, key);
+    }
+    st = mg_solve_run(&ops, &mg->solver, slot, rtol, atol, max_cycles, cycles_out, converged_out, history);
+    return st ? st : halo_error_check(mg);
 }
 
 /* FullMultiGridVCycle, N3/MultiGrid3D.cpp:569-585 */

@@ -176,6 +176,25 @@ int mgk_halo_exchange(cudaStream_t s, const void* const src[4], void* const dst[
 int mgk_gather_push(cudaStream_t s, const void* const src2[2], unsigned long long bytes, void* const dst[][2], unsigned int* const peer_block[],
                     int npeers, int me, unsigned int* flag_block);
 
+/* ---- tolerance-driven solve (mg_solve.cu) ---- */
+/* device parameter block of one solve: the host writes everything above `k` before each launch, k_solve_check the rest */
+typedef struct {
+    double rtol, atol;
+    double* hist;   /* device history: (l2, linf) of r_0, r_1, ...; room for hist_cap pairs */
+    int max_cycles;
+    int hist_cap;
+    int k;          /* residuals checked so far: the cycles run are k - 1 */
+    int done;       /* 1 once the stopping rule has fired */
+    int converged;
+    int pad_;
+    double thr;     /* max(atol, rtol * ||r_0||_2), fixed by the first check */
+} mg_solve_par;
+
+/* one thread: l2 = sqrt(out2[0]), linf = out2[1] of the residual the norm pass has just written; appends them to the
+   history, applies the stopping rule and, when nhandles > 0, sets the conditional handles h0 (and h1) to "continue" */
+int mgk_solve_check(cudaStream_t s, const double* out2, mg_solve_par* par, int nhandles, cudaGraphConditionalHandle h0,
+                    cudaGraphConditionalHandle h1);
+
 /* ---- 2D (pitched: element (x,y) at base[x + y*pitch]) ---- */
 typedef struct {
     int n;

@@ -5,12 +5,18 @@ Class and method names follow the reference classes MultiGrid3D / MultiGrid2D / 
 like the reference's own driver code.  This layer is plumbing only (ctypes + numpy buffers): every
 operator runs in libmg_b200.so on the GPU.
 """
+import collections
 import ctypes
 
 import numpy as np
 
 from . import _lib
 from ._lib import (MG_CORRECTED, MG_F32, MG_F64, MG_FIELD_F, MG_FIELD_V, MG_REF_COMPAT, check)
+
+
+SolveResult = collections.namedtuple("SolveResult", "cycles converged history")
+SolveResult.__doc__ = """Outcome of solve(): cycles run, whether the target was met, and a (cycles + 1, 2) float64 array
+of (l2, linf) of the residuals r_0 .. r_cycles."""
 
 
 def _dtype_code(dtype):
@@ -143,6 +149,16 @@ class _MultiGridBase:
 
     def FullMultiGridVCycle(self, gridID, v0, v1, v2):
         self._call("fmg", ctypes.c_int(gridID), ctypes.c_int(v0), ctypes.c_int(v1), ctypes.c_int(v2))
+
+    def solve(self, v1=2, v2=2, rtol=1e-8, atol=0.0, max_cycles=100, level=0):
+        """V-cycles VCycle(level, v1, v2) from the current v until ||r_k||_2 <= max(atol, rtol * ||r_0||_2) or
+        max_cycles cycles have run (mg?d_solve).  On one GPU the loop runs on the device: one wait per solve."""
+        hist = np.empty((max(int(max_cycles), 0) + 1, 2), dtype=np.float64)
+        cycles, converged = ctypes.c_int(), ctypes.c_int()
+        self._call("solve", ctypes.c_int(level), ctypes.c_int(v1), ctypes.c_int(v2), ctypes.c_double(rtol),
+                   ctypes.c_double(atol), ctypes.c_int(max_cycles), ctypes.byref(cycles), ctypes.byref(converged),
+                   hist.ctypes.data_as(ctypes.c_void_p))
+        return SolveResult(cycles.value, bool(converged.value), hist[:cycles.value + 1].copy())
 
     # ---- reference-facing operators on caller-owned HOST arrays (NOCUDA signatures) ----
     def _sizes(self, n):
