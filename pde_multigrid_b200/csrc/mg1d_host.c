@@ -26,9 +26,7 @@ struct mg1d_s {
     double* h_out2;
     long long launches;
     mg_prof prof;
-    int use_graphs;   /* 0: MG_B200_NO_GRAPH, mg1d_solve runs host-driven */
-    mg_solver solver; /* mg1d_solve: parameter block and history on the device */
-    mg_solve_slot solves[MG_SOLVE_SLOTS];
+    mg_graphs graphs; /* mg1d_solve graphs */
 };
 
 #define PROF_BEGIN(mg, level, op) mg_prof_begin(&(mg)->prof, (mg)->stream, (level), (op), (mg)->launches)
@@ -58,7 +56,7 @@ int mg1d_create(mg1d_t** out, int n, const double range[2], int dtype, int resid
     if (!mg) return mg_fail(MG_ERR_NOMEM, "host allocation failed");
     mg->dtype = dtype;
     mg->mode = residual_mode;
-    mg->use_graphs = getenv("MG_B200_NO_GRAPH") ? 0 : 1;
+    mg_graphs_init(&mg->graphs);
     mg->range[0] = range[0];
     mg->range[1] = range[1];
     mg->H.nlevels = mg_num_levels_for(n);
@@ -93,7 +91,7 @@ int mg1d_destroy(mg1d_t* mg)
 {
     if (!mg) return MG_OK;
     if (mg->stream) cudaStreamSynchronize(mg->stream);
-    mg_solve_free(&mg->solver, mg->solves);
+    mg_graphs_free(&mg->graphs);
     if (mg->stream) cudaStreamDestroy(mg->stream);
     if (mg->arena) cudaFree(mg->arena);
     if (mg->d_out2) cudaFree(mg->d_out2);
@@ -377,13 +375,11 @@ int mg1d_solve(mg1d_t* mg, int level, int v1, int v2, double rtol, double atol, 
     if (st) return st;
     if ((st = mg_solve_check_args(rtol, atol, max_cycles, v1, v2))) return st;
     solve1d_ctx x = {mg, level, v1, v2};
-    const mg_solve_ops ops = {&x, mg->stream, mg->d_out2, &mg->launches, s1_norm, s1_cycle, s1_cycle, NULL, NULL};
-    mg_solve_slot* slot = NULL;
-    if (mg->use_graphs && !mg->prof.enabled) {
-        const int key[MG_SOLVE_KEY] = {level, v1, v2, 0, 0, 0};
-        slot = mg_solve_slot_for(mg->solves, key);
-    }
-    return mg_solve_run(&ops, &mg->solver, slot, rtol, atol, max_cycles, cycles_out, converged_out, history);
+    const mg_cycle_ops ops = {&x, mg->stream, &mg->launches, NULL, s1_cycle, s1_cycle, s1_norm, mg->d_out2, NULL, NULL};
+    const int key[MG_GRAPH_KEY] = {level, v1, v2};
+    /* one launch per cycle: no bound on the sweep counts */
+    return mg_solve_run(&mg->graphs, mg_graphs_on(&mg->graphs, mg->prof.enabled, 1) ? key : NULL, &ops, rtol, atol, max_cycles,
+                        cycles_out, converged_out, history);
 }
 
 /* FullMultiGridVCycle (N1/MultiGrid1D.cpp:132-148): one launch */

@@ -20,19 +20,8 @@ typedef struct {
     void* f;
 } mg_level2d;
 
-/* CUDA-graph cache of whole V-cycles (key = level, v1, v2): at 1025^2 a V(2,2) is ~60 dependent launches on
-   L2-resident fields, i.e. pure launch latency; the second call with a key captures the cycle, later calls replay it */
-#define MG2_GRAPH_SLOTS 4
-typedef struct {
-    int used, level, v1, v2, calls;
-    cudaGraphExec_t exec;
-    long long launches;
-} mg2_graph_slot;
-
 struct mg2d_s {
     int dtype, nlevels;
-    int use_graphs;
-    mg2_graph_slot graphs[MG2_GRAPH_SLOTS];
     cudaStream_t stream;
     mg_level2d* lv;
     void* arena;
@@ -40,8 +29,9 @@ struct mg2d_s {
     double* h_out2;
     long long launches;
     mg_prof prof;
-    mg_solver solver; /* mg2d_solve: parameter block and history on the device */
-    mg_solve_slot solves[MG_SOLVE_SLOTS];
+    /* V-cycle graphs keyed (level, v1, v2): at 1025^2 a V(2,2) is ~60 dependent launches on L2-resident fields, i.e. pure
+       launch latency */
+    mg_graphs graphs;
 };
 
 #define PROF_BEGIN(mg, level, op) mg_prof_begin(&(mg)->prof, (mg)->stream, (level), (op), (mg)->launches)
@@ -94,7 +84,7 @@ int mg2d_create(mg2d_t** out, const int sz[2], const double range[4], const doub
     mg2d_t* mg = (mg2d_t*)calloc(1, sizeof *mg);
     if (!mg) return mg_fail(MG_ERR_NOMEM, "host allocation failed");
     mg->dtype = dtype;
-    mg->use_graphs = getenv("MG_B200_NO_GRAPH") ? 0 : 1;
+    mg_graphs_init(&mg->graphs);
     mg->nlevels = mg_num_levels_for(n);
     mg->lv = (mg_level2d*)calloc((size_t)mg->nlevels, sizeof(mg_level2d));
     if (!mg->lv) { free(mg); return mg_fail(MG_ERR_NOMEM, "host allocation failed"); }
@@ -137,9 +127,7 @@ int mg2d_destroy(mg2d_t* mg)
 {
     if (!mg) return MG_OK;
     if (mg->stream) cudaStreamSynchronize(mg->stream);
-    for (int i = 0; i < MG2_GRAPH_SLOTS; i++)
-        if (mg->graphs[i].used && mg->graphs[i].exec) cudaGraphExecDestroy(mg->graphs[i].exec);
-    mg_solve_free(&mg->solver, mg->solves);
+    mg_graphs_free(&mg->graphs);
     if (mg->stream) cudaStreamDestroy(mg->stream);
     if (mg->arena) cudaFree(mg->arena);
     if (mg->d_scratch) cudaFree(mg->d_scratch);
@@ -386,55 +374,39 @@ static int vcycle_rec(mg2d_t* mg, int level, int v1, int v2)
     return relax_level(mg, level, v2);
 }
 
+/* one cycle on `level` with fixed sweep counts, as the graph cache (mg_host_common.c) runs, captures and replays it */
+typedef struct {
+    mg2d_t* mg;
+    int level, v1, v2;
+} cycle2d_ctx;
+
+static int c2_cycle(void* c) { cycle2d_ctx* x = (cycle2d_ctx*)c; return vcycle_rec(x->mg, x->level, x->v1, x->v2); }
+static int c2_public(void* c) { cycle2d_ctx* x = (cycle2d_ctx*)c; return mg2d_vcycle(x->mg, x->level, x->v1, x->v2); }
+static int c2_norm(void* c) { cycle2d_ctx* x = (cycle2d_ctx*)c; return residual_norm_enqueue(x->mg, x->level); }
+
+static mg_cycle_ops cycle_ops(cycle2d_ctx* x)
+{
+    mg2d_t* mg = x->mg;
+    const mg_cycle_ops ops = {x, mg->stream, &mg->launches, NULL, c2_cycle, c2_public, c2_norm, mg->d_scratch + 2 * SCRATCH_PARTS, NULL, NULL};
+    return ops;
+}
+
+/* graphs for cycles of up to MG_GRAPH_MAX_LAUNCHES launches */
+static int graphs_on(const mg2d_t* mg, int level, int v1, int v2)
+{
+    return mg_graphs_on(&mg->graphs, mg->prof.enabled, 2LL * (v1 + v2) * (mg->nlevels - level));
+}
+
 int mg2d_vcycle(mg2d_t* mg, int level, int v1, int v2)
 {
     int st = check_level(mg, level);
     if (st) return st;
     if (v1 < 0 || v2 < 0) return mg_fail(MG_ERR_ARG, "negative sweep count");
-    const long long per_cycle = 2LL * (v1 + v2) * (mg->nlevels - level);
-    if (!mg->use_graphs || mg->prof.enabled || per_cycle > 4096) return vcycle_rec(mg, level, v1, v2);
-    mg2_graph_slot* g = NULL;
-    for (int i = 0; i < MG2_GRAPH_SLOTS && !g; i++)
-        if (mg->graphs[i].used && mg->graphs[i].level == level && mg->graphs[i].v1 == v1 && mg->graphs[i].v2 == v2) g = &mg->graphs[i];
-    if (!g) {
-        for (int i = 0; i < MG2_GRAPH_SLOTS && !g; i++)
-            if (!mg->graphs[i].used) g = &mg->graphs[i];
-        if (!g) return vcycle_rec(mg, level, v1, v2); /* cache full: run eagerly */
-        memset(g, 0, sizeof *g);
-        g->used = 1; g->level = level; g->v1 = v1; g->v2 = v2;
-    }
-    if (++g->calls == 1) return vcycle_rec(mg, level, v1, v2); /* first call eager: kernel attributes, lazy loading */
-    if (!g->exec) {
-        const long long l0 = mg->launches;
-        cudaGraph_t graph = NULL;
-        MG_CUDA(cudaStreamBeginCapture(mg->stream, cudaStreamCaptureModeThreadLocal));
-        st = vcycle_rec(mg, level, v1, v2);
-        cudaError_t e = cudaStreamEndCapture(mg->stream, &graph);
-        g->launches = mg->launches - l0;
-        mg->launches = l0; /* nothing ran during the capture */
-        if (!st && e == cudaSuccess && graph) e = cudaGraphInstantiate(&g->exec, graph, 0);
-        if (graph) cudaGraphDestroy(graph);
-        if (st || e != cudaSuccess || !g->exec) {
-            g->exec = NULL;
-            cudaGetLastError();
-            mg->use_graphs = 0; /* capture is not possible here: stay eager */
-            return st ? st : vcycle_rec(mg, level, v1, v2);
-        }
-    }
-    MG_CUDA(cudaGraphLaunch(g->exec, mg->stream));
-    mg->launches += g->launches;
-    return MG_OK;
+    cycle2d_ctx x = {mg, level, v1, v2};
+    const mg_cycle_ops ops = cycle_ops(&x);
+    const int key[MG_GRAPH_KEY] = {level, v1, v2};
+    return mg_graph_cycle(&mg->graphs, graphs_on(mg, level, v1, v2) ? key : NULL, &ops);
 }
-
-/* tolerance-driven solve (mg_host_common.c builds and runs it) */
-typedef struct {
-    mg2d_t* mg;
-    int level, v1, v2;
-} solve2d_ctx;
-
-static int s2_norm(void* c) { solve2d_ctx* x = (solve2d_ctx*)c; return residual_norm_enqueue(x->mg, x->level); }
-static int s2_cycle(void* c) { solve2d_ctx* x = (solve2d_ctx*)c; return mg2d_vcycle(x->mg, x->level, x->v1, x->v2); }
-static int s2_capture(void* c) { solve2d_ctx* x = (solve2d_ctx*)c; return vcycle_rec(x->mg, x->level, x->v1, x->v2); }
 
 int mg2d_solve(mg2d_t* mg, int level, int v1, int v2, double rtol, double atol, int max_cycles, int* cycles_out, int* converged_out,
                double* history)
@@ -442,15 +414,11 @@ int mg2d_solve(mg2d_t* mg, int level, int v1, int v2, double rtol, double atol, 
     int st = check_level(mg, level);
     if (st) return st;
     if ((st = mg_solve_check_args(rtol, atol, max_cycles, v1, v2))) return st;
-    solve2d_ctx x = {mg, level, v1, v2};
-    const mg_solve_ops ops = {&x, mg->stream, mg->d_scratch + 2 * SCRATCH_PARTS, &mg->launches, s2_norm, s2_cycle, s2_capture, NULL, NULL};
-    mg_solve_slot* slot = NULL;
-    const long long per_cycle = 2LL * (v1 + v2) * (mg->nlevels - level);
-    if (mg->use_graphs && !mg->prof.enabled && per_cycle <= 4096) {
-        const int key[MG_SOLVE_KEY] = {level, v1, v2, 0, 0, 0};
-        slot = mg_solve_slot_for(mg->solves, key);
-    }
-    return mg_solve_run(&ops, &mg->solver, slot, rtol, atol, max_cycles, cycles_out, converged_out, history);
+    cycle2d_ctx x = {mg, level, v1, v2};
+    const mg_cycle_ops ops = cycle_ops(&x);
+    const int key[MG_GRAPH_KEY] = {level, v1, v2};
+    return mg_solve_run(&mg->graphs, graphs_on(mg, level, v1, v2) ? key : NULL, &ops, rtol, atol, max_cycles, cycles_out,
+                        converged_out, history);
 }
 
 /* FullMultiGridVCycle, N2/MultiGrid2D.cpp:296-312 */

@@ -40,9 +40,7 @@ struct mg3b_s {
     double* d_tables;  /* sin tables of InitF: nx + ny + nz doubles of the finest level */
     double* h_out2;    /* pinned */
     long long launches;
-    int use_graphs;    /* 0: MG_B200_NO_GRAPH, mg3b_solve runs host-driven */
-    mg_solver solver;  /* mg3b_solve: parameter block and history on the device */
-    mg_solve_slot solves[MG_SOLVE_SLOTS];
+    mg_graphs graphs;  /* mg3b_solve graphs */
 };
 
 static size_t level_count(const mg_level3b* L) { return (size_t)L->n[0] * (size_t)L->n[1] * (size_t)L->n[2]; }
@@ -108,7 +106,7 @@ int mg3b_destroy(mg3b_t* mg)
 {
     if (!mg) return MG_OK;
     if (mg->stream) cudaStreamSynchronize(mg->stream);
-    mg_solve_free(&mg->solver, mg->solves);
+    mg_graphs_free(&mg->graphs);
     if (mg->arena) cudaFree(mg->arena);
     if (mg->staging) cudaFree(mg->staging);
     if (mg->d_scratch) cudaFree(mg->d_scratch);
@@ -139,7 +137,7 @@ int mg3b_create(mg3b_t** out, const int finest_size_xyz[3], const double range[6
     if (!mg) return mg_fail(MG_ERR_NOMEM, "host allocation failed");
     mg->dtype = dtype;
     mg->mode = residual_mode;
-    mg->use_graphs = getenv("MG_B200_NO_GRAPH") ? 0 : 1;
+    mg_graphs_init(&mg->graphs);
     memcpy(mg->range, range, sizeof mg->range);
     int mn = finest_size_xyz[0];
     if (finest_size_xyz[1] < mn) mn = finest_size_xyz[1];
@@ -423,14 +421,10 @@ int mg3b_solve(mg3b_t* mg, int level, int v1, int v2, double rtol, double atol, 
     if (st) return st;
     if ((st = mg_solve_check_args(rtol, atol, max_cycles, v1, v2))) return st;
     solve3b_ctx x = {mg, level, v1, v2};
-    const mg_solve_ops ops = {&x, mg->stream, mg->d_scratch + 2 * MG3B_NPARTS, &mg->launches, s3b_norm, s3b_cycle, s3b_cycle, NULL, NULL};
-    mg_solve_slot* slot = NULL;
-    const long long per_cycle = 2LL * (v1 + v2) * (mg->nlevels - level);
-    if (mg->use_graphs && per_cycle <= 4096) {
-        const int key[MG_SOLVE_KEY] = {level, v1, v2, 0, 0, 0};
-        slot = mg_solve_slot_for(mg->solves, key);
-    }
-    return mg_solve_run(&ops, &mg->solver, slot, rtol, atol, max_cycles, cycles_out, converged_out, history);
+    const mg_cycle_ops ops = {&x, mg->stream, &mg->launches, NULL, s3b_cycle, s3b_cycle, s3b_norm, mg->d_scratch + 2 * MG3B_NPARTS, NULL, NULL};
+    const int key[MG_GRAPH_KEY] = {level, v1, v2};
+    return mg_solve_run(&mg->graphs, mg_graphs_on(&mg->graphs, 0, 2LL * (v1 + v2) * (mg->nlevels - level)) ? key : NULL, &ops,
+                        rtol, atol, max_cycles, cycles_out, converged_out, history);
 }
 
 /* FullMultiGridVCycle, N3/MultiGrid3D.cpp:569-585 */

@@ -83,18 +83,6 @@ typedef struct {
     int gather_p2p;               /* 1: gather_level stores directly into the peers (MG_B200_GATHER=nccl switches it off) */
 } mg_p2p;
 
-/* CUDA-graph cache of whole V-cycles: the cycle is ~100 dependent launches, most of them tiny (coarse
-   levels, halo kernels); replaying them from a graph removes the per-launch gaps that dominate at 257^3
-   and on the 8-GPU slabs.  Key = (level, v1, v2, smoother). */
-#define MG_GRAPH_SLOTS 16
-typedef struct {
-    int used, level, v1, v2, smoother, arith, calls;
-    unsigned cur_start, cur_end; /* bit l = which v buffer level l works on when the graph starts / has finished */
-    unsigned vg_start, vg_end;   /* bits 2l, 2l+1 = mg_level3d.vg_valid, vg_deep */
-    cudaGraphExec_t exec;
-    long long launches, halo_bytes;
-} mg_graph_slot;
-
 struct mg3d_s {
     int dtype, mode, nlevels;
     int rank, nranks;
@@ -119,8 +107,6 @@ struct mg3d_s {
     long long launches;
     long long halo_bytes; /* bytes sent by this rank in halo exchanges / gathers */
     mg_prof prof;
-    int use_graphs;
-    mg_graph_slot graphs[MG_GRAPH_SLOTS];
     double omega;   /* weight of MG_SMOOTHER_JACOBI */
     int arith;           /* MG_ARITH_EXACT / MG_ARITH_FAST */
     int no_pipe;         /* MG_B200_NO_PIPE: MG_SMOOTHER_AUTO without temporal blocking (the round-1 default) */
@@ -129,8 +115,9 @@ struct mg3d_s {
     unsigned int* d_flag; /* {exactness flag of the pipelined smoother, completion counter of its fallback} */
     int no_tail;         /* MG_B200_NO_TAIL: coarse levels as separate launches */
     int full_correction; /* MG_B200_FULL_CORRECTION: correct both colours after prolongation inside a cycle */
-    mg_solver solver;    /* mg3d_solve: parameter block and history on the device */
-    mg_solve_slot solves[MG_SOLVE_SLOTS]; /* mg3d_solve graphs, apart from the cycle graphs above */
+    /* V-cycle graphs: the cycle is ~100 dependent launches, most of them tiny (coarse levels, halo kernels); replaying
+       them removes the per-launch gaps that dominate at 257^3 and on the 8-GPU slabs */
+    mg_graphs graphs;
 };
 
 #define PROF_BEGIN(mg, level, op) mg_prof_begin(&(mg)->prof, (mg)->stream, (level), (op), (mg)->launches)
@@ -622,7 +609,7 @@ static int create_common(mg3d_t** out, const int sz[3], const double range[6], i
     mg->nranks = nranks;
     mg->smoother = MG_SMOOTHER_AUTO;
     mg->sweeps_per_pass = 1;
-    mg->use_graphs = getenv("MG_B200_NO_GRAPH") ? 0 : 1;
+    mg_graphs_init(&mg->graphs);
     mg->omega = 6.0 / 7.0;
     mg->no_tail = getenv("MG_B200_NO_TAIL") != NULL;
     mg->no_pipe = getenv("MG_B200_NO_PIPE") != NULL;
@@ -750,9 +737,7 @@ int mg3d_destroy(mg3d_t* mg)
 {
     if (!mg) return MG_OK;
     if (mg->stream) cudaStreamSynchronize(mg->stream);
-    for (int i = 0; i < MG_GRAPH_SLOTS; i++)
-        if (mg->graphs[i].used && mg->graphs[i].exec) cudaGraphExecDestroy(mg->graphs[i].exec);
-    mg_solve_free(&mg->solver, mg->solves);
+    mg_graphs_free(&mg->graphs);
     p2p_teardown(mg);
     if (mg->comm) mg_comm_destroy(mg->comm);
     if (mg->cstream) { cudaStreamSynchronize(mg->cstream); cudaStreamDestroy(mg->cstream); }
@@ -823,16 +808,7 @@ int mg3d_set_jacobi_weight(mg3d_t* mg, double omega)
     if (!mg) return mg_fail(MG_ERR_ARG, "null handle");
     if (!(omega > 0.0 && omega <= 1.0)) return mg_fail(MG_ERR_ARG, "Jacobi weight %g outside (0,1]", omega);
     mg->omega = mg->dtype == MG_F32 ? (double)(float)omega : omega;
-    for (int i = 0; i < MG_GRAPH_SLOTS; i++) /* captured cycles carry the old weight as a kernel argument */
-        if (mg->graphs[i].used && mg->graphs[i].smoother == MG_SMOOTHER_JACOBI) {
-            if (mg->graphs[i].exec) cudaGraphExecDestroy(mg->graphs[i].exec);
-            memset(&mg->graphs[i], 0, sizeof mg->graphs[i]);
-        }
-    for (int i = 0; i < MG_SOLVE_SLOTS; i++) /* key[3] = smoother */
-        if (mg->solves[i].used && mg->solves[i].key[3] == MG_SMOOTHER_JACOBI) {
-            if (mg->solves[i].exec) cudaGraphExecDestroy(mg->solves[i].exec);
-            memset(&mg->solves[i], 0, sizeof mg->solves[i]);
-        }
+    mg_graphs_drop(&mg->graphs, MG_GRAPH_KEY_SMOOTHER, MG_SMOOTHER_JACOBI); /* captured cycles carry the old weight as a kernel argument */
     return MG_OK;
 }
 
@@ -1525,105 +1501,25 @@ static int vcycle_rec(mg3d_t* mg, int level, int v1, int v2)
     return relax_level(mg, level, v2);
 }
 
-/* The second call with the same (level, v1, v2, smoother) captures the cycle into a CUDA graph; later calls
-   replay it.  The first call runs eagerly (kernel attributes are set, lazy module loading is done).  The
-   P2P halo kernels keep their sequence counters in device memory, so their arguments are capture-stable;
-   NCCL collectives are graph-capturable.  Per-operator timers need eager launches: profiling disables it. */
-int mg3d_vcycle(mg3d_t* mg, int level, int v1, int v2)
-{
-    int st = check_level(mg, level);
-    if (st) return st;
-    if (v1 < 0 || v2 < 0) return mg_fail(MG_ERR_ARG, "negative sweep count");
-    const long long per_cycle = 2LL * (v1 + v2) * (mg->nlevels - level) * 2;
-    if (!mg->use_graphs || mg->prof.enabled || per_cycle > 4096) return vcycle_rec(mg, level, v1, v2);
-    /* a captured graph bakes in which of its two v buffers every level works on (the temporally blocked smoothers
-       ping-pong), so that state is part of the key; a cycle with an odd number of passes ends on the other buffers and
-       the next call finds (or captures) the graph that starts there */
-    unsigned cur_now = 0, vg_now = 0;
-    for (int l = 0; l < mg->nlevels && l < 32; l++) {
-        cur_now |= (unsigned)mg->lv[l].cur << l;
-        if (l < 16) vg_now |= ((unsigned)(mg->lv[l].vg_valid != 0) | ((unsigned)(mg->lv[l].vg_deep != 0) << 1)) << (2 * l);
-    }
-    mg_graph_slot* g = NULL;
-    for (int i = 0; i < MG_GRAPH_SLOTS && !g; i++)
-        if (mg->graphs[i].used && mg->graphs[i].level == level && mg->graphs[i].v1 == v1 && mg->graphs[i].v2 == v2 &&
-            mg->graphs[i].smoother == mg->smoother && mg->graphs[i].arith == mg->arith && mg->graphs[i].cur_start == cur_now &&
-            mg->graphs[i].vg_start == vg_now)
-            g = &mg->graphs[i];
-    if (!g) {
-        for (int i = 0; i < MG_GRAPH_SLOTS && !g; i++)
-            if (!mg->graphs[i].used) g = &mg->graphs[i];
-        if (!g) return vcycle_rec(mg, level, v1, v2); /* cache full: run eagerly */
-        memset(g, 0, sizeof *g);
-        g->used = 1; g->level = level; g->v1 = v1; g->v2 = v2; g->smoother = mg->smoother; g->arith = mg->arith;
-        g->cur_start = cur_now;
-        g->vg_start = vg_now;
-    }
-    g->calls++;
-    if (g->calls == 1) return vcycle_rec(mg, level, v1, v2);
-    if (!g->exec) {
-        const long long l0 = mg->launches, h0 = mg->halo_bytes;
-        cudaGraph_t graph = NULL;
-        MG_CUDA(cudaStreamBeginCapture(mg->stream, cudaStreamCaptureModeThreadLocal));
-        st = vcycle_rec(mg, level, v1, v2);
-        cudaError_t e = cudaStreamEndCapture(mg->stream, &graph);
-        g->cur_end = g->vg_end = 0;
-        for (int l = 0; l < mg->nlevels; l++) { /* nothing ran during the capture: undo the host-side state changes */
-            if (l < 32) g->cur_end |= (unsigned)mg->lv[l].cur << l;
-            if (l < 16) g->vg_end |= ((unsigned)(mg->lv[l].vg_valid != 0) | ((unsigned)(mg->lv[l].vg_deep != 0) << 1)) << (2 * l);
-            mg->lv[l].cur = (int)((cur_now >> l) & 1u);
-            mg->lv[l].v = mg->lv[l].vbuf[mg->lv[l].cur];
-            mg->lv[l].vg_valid = l < 16 ? (int)((vg_now >> (2 * l)) & 1u) : 1;
-            mg->lv[l].vg_deep = l < 16 ? (int)((vg_now >> (2 * l + 1)) & 1u) : 0;
-        }
-        g->launches = mg->launches - l0;
-        g->halo_bytes = mg->halo_bytes - h0;
-        mg->launches = l0;
-        mg->halo_bytes = h0;
-        if (st || e != cudaSuccess || !graph) {
-            if (graph) cudaGraphDestroy(graph);
-            cudaGetLastError();
-            mg->use_graphs = 0; /* capture is not possible here: stay eager */
-            return st ? st : vcycle_rec(mg, level, v1, v2);
-        }
-        e = cudaGraphInstantiate(&g->exec, graph, 0);
-        cudaGraphDestroy(graph);
-        if (e != cudaSuccess) {
-            g->exec = NULL;
-            cudaGetLastError();
-            mg->use_graphs = 0;
-            return vcycle_rec(mg, level, v1, v2);
-        }
-    }
-    MG_CUDA(cudaGraphLaunch(g->exec, mg->stream));
-    for (int l = 0; l < mg->nlevels && l < 32; l++) { /* the replay leaves every level in the state the capture ended in */
-        mg->lv[l].cur = (int)((g->cur_end >> l) & 1u);
-        mg->lv[l].v = mg->lv[l].vbuf[mg->lv[l].cur];
-        mg->lv[l].vg_valid = l < 16 ? (int)((g->vg_end >> (2 * l)) & 1u) : 1;
-        mg->lv[l].vg_deep = l < 16 ? (int)((g->vg_end >> (2 * l + 1)) & 1u) : 0;
-    }
-    mg->launches += g->launches;
-    mg->halo_bytes += g->halo_bytes;
-    return MG_OK;
-}
-
-/* ---- tolerance-driven solve (mg_host_common.c builds and runs it) ---------------------------------------------- */
+/* ---- the graph cache (mg_host_common.c) runs, captures and replays one cycle on `level` with fixed sweep counts ---- */
 
 typedef struct {
     mg3d_t* mg;
     int level, v1, v2;
-} solve3d_ctx;
+} cycle3d_ctx;
 
-static int s3_norm(void* c) { solve3d_ctx* x = (solve3d_ctx*)c; return residual_norm_enqueue(x->mg, x->level); }
-static int s3_cycle(void* c) { solve3d_ctx* x = (solve3d_ctx*)c; return mg3d_vcycle(x->mg, x->level, x->v1, x->v2); }
-static int s3_capture(void* c) { solve3d_ctx* x = (solve3d_ctx*)c; return vcycle_rec(x->mg, x->level, x->v1, x->v2); }
+static int c3_cycle(void* c) { cycle3d_ctx* x = (cycle3d_ctx*)c; return vcycle_rec(x->mg, x->level, x->v1, x->v2); }
+static int c3_public(void* c) { cycle3d_ctx* x = (cycle3d_ctx*)c; return mg3d_vcycle(x->mg, x->level, x->v1, x->v2); }
+static int c3_norm(void* c) { cycle3d_ctx* x = (cycle3d_ctx*)c; return residual_norm_enqueue(x->mg, x->level); }
 
-/* [0] = which v buffer every level works on; [1] = the ghost-validity flags.  Only [0] changes the kernels of a cycle on
-   one GPU (the flags steer the exchanges of distributed levels), so only [0] has to return to its start value; [1] is
-   restored so that later mg3d_vcycle calls find the graphs the hand-written loop would find. */
-static void s3_save(void* c, unsigned out[2])
+/* [0] = which v buffer every level works on (bit l, levels < 32); [1] = the ghost-validity flags (bits 2l and 2l+1 =
+   vg_valid, vg_deep, levels < 16; coarser levels load as valid and not deep).  A captured graph bakes in [0] (the
+   temporally blocked smoothers ping-pong); [1] steers the exchanges of distributed levels.  Both are part of the cycle
+   graph's key, and both are put back after a capture and set after a replay or a device solve, so that the next call
+   finds the graph the hand-written loop would find. */
+static void c3_save(void* c, unsigned out[2])
 {
-    const mg3d_t* mg = ((solve3d_ctx*)c)->mg;
+    const mg3d_t* mg = ((cycle3d_ctx*)c)->mg;
     out[0] = out[1] = 0;
     for (int l = 0; l < mg->nlevels && l < 32; l++) {
         out[0] |= (unsigned)mg->lv[l].cur << l;
@@ -1631,9 +1527,9 @@ static void s3_save(void* c, unsigned out[2])
     }
 }
 
-static void s3_load(void* c, const unsigned in[2])
+static void c3_load(void* c, const unsigned in[2])
 {
-    mg3d_t* mg = ((solve3d_ctx*)c)->mg;
+    mg3d_t* mg = ((cycle3d_ctx*)c)->mg;
     for (int l = 0; l < mg->nlevels && l < 32; l++) {
         mg->lv[l].cur = (int)((in[0] >> l) & 1u);
         mg->lv[l].v = mg->lv[l].vbuf[mg->lv[l].cur];
@@ -1642,26 +1538,61 @@ static void s3_load(void* c, const unsigned in[2])
     }
 }
 
+static mg_cycle_ops cycle_ops(cycle3d_ctx* x)
+{
+    mg3d_t* mg = x->mg;
+    const mg_cycle_ops ops = {x, mg->stream, &mg->launches, &mg->halo_bytes, c3_cycle, c3_public, c3_norm, norm_out2(mg), c3_save, c3_load};
+    return ops;
+}
+
+/* graphs for cycles of up to MG_GRAPH_MAX_LAUNCHES launches */
+static int graphs_on(const mg3d_t* mg, int level, int v1, int v2)
+{
+    return mg_graphs_on(&mg->graphs, mg->prof.enabled, 2LL * (v1 + v2) * (mg->nlevels - level) * 2);
+}
+
+/* (level, v1, v2, smoother, arith, buffer bits, ghost bits); a solve graph keys on the buffer bits only */
+static void graph_key(cycle3d_ctx* x, int with_ghosts, int key[MG_GRAPH_KEY])
+{
+    unsigned state[2];
+    c3_save(x, state);
+    const int k[MG_GRAPH_KEY] = {x->level, x->v1, x->v2, x->mg->smoother, x->mg->arith, (int)state[0], with_ghosts ? (int)state[1] : 0};
+    memcpy(key, k, sizeof k);
+}
+
+/* The first call with a key runs eagerly, the second captures the cycle into a CUDA graph, later calls replay it.  The
+   P2P halo kernels keep their sequence counters in device memory, so their arguments are capture-stable; NCCL
+   collectives are graph-capturable.  A cycle with an odd number of passes ends on the other buffers, and the next call
+   finds (or captures) the graph that starts there. */
+int mg3d_vcycle(mg3d_t* mg, int level, int v1, int v2)
+{
+    int st = check_level(mg, level);
+    if (st) return st;
+    if (v1 < 0 || v2 < 0) return mg_fail(MG_ERR_ARG, "negative sweep count");
+    cycle3d_ctx x = {mg, level, v1, v2};
+    const mg_cycle_ops ops = cycle_ops(&x);
+    int key[MG_GRAPH_KEY];
+    graph_key(&x, 1, key);
+    return mg_graph_cycle(&mg->graphs, graphs_on(mg, level, v1, v2) ? key : NULL, &ops);
+}
+
+/* ---- tolerance-driven solve (mg_host_common.c builds and runs it) ---------------------------------------------- */
+
 int mg3d_solve(mg3d_t* mg, int level, int v1, int v2, double rtol, double atol, int max_cycles, int* cycles_out, int* converged_out,
                double* history)
 {
     int st = check_level(mg, level);
     if (st) return st;
     if ((st = mg_solve_check_args(rtol, atol, max_cycles, v1, v2))) return st;
-    solve3d_ctx x = {mg, level, v1, v2};
-    const mg_solve_ops ops = {&x, mg->stream, norm_out2(mg), &mg->launches, s3_norm, s3_cycle, s3_capture, s3_save, s3_load};
-    mg_solve_slot* slot = NULL;
+    cycle3d_ctx x = {mg, level, v1, v2};
+    const mg_cycle_ops ops = cycle_ops(&x);
+    int key[MG_GRAPH_KEY];
+    graph_key(&x, 0, key);
     /* A distributed solve stays host-driven: a conditional body may hold kernels, copies, memsets and nested graphs only,
        and the NCCL all-reduce of the norm is not known to stay inside that set.  Every rank checks the same all-reduced
        norm, so every rank stops after the same cycle. */
-    const long long per_cycle = 2LL * (v1 + v2) * (mg->nlevels - level) * 2;
-    if (mg->nranks == 1 && mg->use_graphs && !mg->prof.enabled && per_cycle <= 4096) {
-        unsigned state[2];
-        s3_save(&x, state);
-        const int key[MG_SOLVE_KEY] = {level, v1, v2, mg->smoother, mg->arith, (int)state[0]};
-        slot = mg_solve_slot_for(mg->solves, key);
-    }
-    st = mg_solve_run(&ops, &mg->solver, slot, rtol, atol, max_cycles, cycles_out, converged_out, history);
+    const int device = mg->nranks == 1 && graphs_on(mg, level, v1, v2);
+    st = mg_solve_run(&mg->graphs, device ? key : NULL, &ops, rtol, atol, max_cycles, cycles_out, converged_out, history);
     return st ? st : halo_error_check(mg);
 }
 

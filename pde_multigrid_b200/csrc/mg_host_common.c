@@ -1,8 +1,9 @@
-/* mg_host_common.c -- error state and device probing shared by the host drivers. */
+/* mg_host_common.c -- error state, device probing and the CUDA-graph cache shared by the host drivers. */
 #include "mg_host_common.h"
 
 #include <stdarg.h>
 #include <stdio.h>
+#include <stdlib.h>
 #include <string.h>
 
 static __thread char g_err[512] = "";
@@ -30,6 +31,94 @@ int mg_device_count(void)
     return n;
 }
 
+/* ---- CUDA-graph cache ------------------------------------------------------------------------- */
+
+void mg_graphs_init(mg_graphs* gr) { gr->enabled = getenv("MG_B200_NO_GRAPH") ? 0 : 1; }
+
+static void drop_slot(mg_graph_slot* g)
+{
+    if (g->exec) cudaGraphExecDestroy(g->exec);
+    memset(g, 0, sizeof *g);
+}
+
+void mg_graphs_free(mg_graphs* gr)
+{
+    for (int i = 0; i < MG_CYCLE_SLOTS; i++) drop_slot(&gr->cycles[i]);
+    for (int i = 0; i < MG_SOLVE_SLOTS; i++) drop_slot(&gr->solves[i]);
+    if (gr->h_par) cudaFreeHost(gr->h_par);
+    if (gr->d_par) cudaFree(gr->d_par);
+    if (gr->d_hist) cudaFree(gr->d_hist);
+    memset(gr, 0, sizeof *gr);
+}
+
+int mg_graphs_on(const mg_graphs* gr, int profiling, long long launches_per_cycle)
+{
+    return gr->enabled && !profiling && launches_per_cycle <= MG_GRAPH_MAX_LAUNCHES;
+}
+
+void mg_graphs_drop(mg_graphs* gr, int pos, int value)
+{
+    for (int i = 0; i < MG_CYCLE_SLOTS; i++)
+        if (gr->cycles[i].used && gr->cycles[i].key[pos] == value) drop_slot(&gr->cycles[i]);
+    for (int i = 0; i < MG_SOLVE_SLOTS; i++)
+        if (gr->solves[i].used && gr->solves[i].key[pos] == value) drop_slot(&gr->solves[i]);
+}
+
+/* the slot with this key, or a free one claimed for it (NULL: the cache is full) */
+static mg_graph_slot* slot_for(mg_graph_slot* slots, int n, const int key[MG_GRAPH_KEY])
+{
+    for (int i = 0; i < n; i++)
+        if (slots[i].used && !memcmp(slots[i].key, key, sizeof slots[i].key)) return &slots[i];
+    for (int i = 0; i < n; i++)
+        if (!slots[i].used) {
+            memset(&slots[i], 0, sizeof slots[i]);
+            slots[i].used = 1;
+            memcpy(slots[i].key, key, sizeof slots[i].key);
+            return &slots[i];
+        }
+    return NULL;
+}
+
+int mg_graph_cycle(mg_graphs* gr, const int key[MG_GRAPH_KEY], const mg_cycle_ops* ops)
+{
+    mg_graph_slot* g = key ? slot_for(gr->cycles, MG_CYCLE_SLOTS, key) : NULL;
+    if (!g || !g->warm) { /* no graphs, the cache is full, or the first call of the key */
+        if (g) g->warm = 1;
+        return ops->cycle(ops->ctx);
+    }
+    if (!g->exec) {
+        const long long l0 = *ops->launches, h0 = ops->halo_bytes ? *ops->halo_bytes : 0;
+        cudaGraph_t graph = NULL;
+        if (ops->save) ops->save(ops->ctx, g->snap[0]);
+        MG_CUDA(cudaStreamBeginCapture(ops->stream, cudaStreamCaptureModeThreadLocal));
+        int st = ops->cycle(ops->ctx);
+        cudaError_t e = cudaStreamEndCapture(ops->stream, &graph);
+        if (ops->save) { /* nothing ran during the capture: undo the host-side state changes, keep the end state */
+            ops->save(ops->ctx, g->snap[1]);
+            ops->load(ops->ctx, g->snap[0]);
+        }
+        g->launches[0] = *ops->launches - l0;
+        *ops->launches = l0;
+        if (ops->halo_bytes) {
+            g->halo_bytes = *ops->halo_bytes - h0;
+            *ops->halo_bytes = h0;
+        }
+        if (!st && e == cudaSuccess && graph) e = cudaGraphInstantiate(&g->exec, graph, 0);
+        if (graph) cudaGraphDestroy(graph);
+        if (st || e != cudaSuccess || !g->exec) {
+            g->exec = NULL;
+            cudaGetLastError();
+            gr->enabled = 0; /* capture is not possible here: stay eager, and keep solves host-driven */
+            return st ? st : ops->cycle(ops->ctx);
+        }
+    }
+    MG_CUDA(cudaGraphLaunch(g->exec, ops->stream));
+    if (ops->load) ops->load(ops->ctx, g->snap[1]); /* the replay leaves the host-side state the capture ended in */
+    *ops->launches += g->launches[0];
+    if (ops->halo_bytes) *ops->halo_bytes += g->halo_bytes;
+    return MG_OK;
+}
+
 /* ---- tolerance-driven solve ------------------------------------------------------------------- */
 
 int mg_solve_check_args(double rtol, double atol, int max_cycles, int v1, int v2)
@@ -40,96 +129,72 @@ int mg_solve_check_args(double rtol, double atol, int max_cycles, int v1, int v2
     return MG_OK;
 }
 
-mg_solve_slot* mg_solve_slot_for(mg_solve_slot slots[MG_SOLVE_SLOTS], const int key[MG_SOLVE_KEY])
-{
-    for (int i = 0; i < MG_SOLVE_SLOTS; i++)
-        if (slots[i].used && !memcmp(slots[i].key, key, sizeof slots[i].key)) return &slots[i];
-    for (int i = 0; i < MG_SOLVE_SLOTS; i++)
-        if (!slots[i].used) {
-            memset(&slots[i], 0, sizeof slots[i]);
-            slots[i].used = 1;
-            memcpy(slots[i].key, key, sizeof slots[i].key);
-            return &slots[i];
-        }
-    return NULL;
-}
-
-void mg_solve_free(mg_solver* sv, mg_solve_slot slots[MG_SOLVE_SLOTS])
-{
-    for (int i = 0; i < MG_SOLVE_SLOTS; i++)
-        if (slots[i].used && slots[i].exec) cudaGraphExecDestroy(slots[i].exec);
-    if (sv->h_par) cudaFreeHost(sv->h_par);
-    if (sv->d_par) cudaFree(sv->d_par);
-    if (sv->d_hist) cudaFree(sv->d_hist);
-    memset(sv, 0, sizeof *sv);
-}
-
 /* writes the parameter block of the next solve (the graph reads everything it needs from it: one graph serves every
    tolerance, cycle limit and history size) */
-static int solver_begin(mg_solver* sv, cudaStream_t s, double rtol, double atol, int max_cycles, int want_history)
+static int solver_begin(mg_graphs* gr, cudaStream_t s, double rtol, double atol, int max_cycles, int want_history)
 {
-    if (!sv->h_par) {
-        MG_CUDA(cudaMallocHost((void**)&sv->h_par, sizeof *sv->h_par));
-        MG_CUDA(cudaMalloc((void**)&sv->d_par, sizeof *sv->d_par));
+    if (!gr->h_par) {
+        MG_CUDA(cudaMallocHost((void**)&gr->h_par, sizeof *gr->h_par));
+        MG_CUDA(cudaMalloc((void**)&gr->d_par, sizeof *gr->d_par));
     }
     const int need = want_history ? max_cycles + 1 : 0;
-    if (need > sv->hist_cap) {
+    if (need > gr->hist_cap) {
         MG_CUDA(cudaStreamSynchronize(s)); /* a previous solve may still write the old buffer */
-        if (sv->d_hist) cudaFree(sv->d_hist);
-        sv->d_hist = NULL;
-        sv->hist_cap = 0;
-        MG_CUDA(cudaMalloc((void**)&sv->d_hist, 2 * (size_t)need * sizeof(double)));
-        sv->hist_cap = need;
+        if (gr->d_hist) cudaFree(gr->d_hist);
+        gr->d_hist = NULL;
+        gr->hist_cap = 0;
+        MG_CUDA(cudaMalloc((void**)&gr->d_hist, 2 * (size_t)need * sizeof(double)));
+        gr->hist_cap = need;
     }
-    mg_solve_par* p = sv->h_par;
+    mg_solve_par* p = gr->h_par;
     memset(p, 0, sizeof *p);
     p->rtol = rtol;
     p->atol = atol;
-    p->hist = sv->d_hist;
+    p->hist = gr->d_hist;
     p->max_cycles = max_cycles;
     p->hist_cap = need;
-    MG_CUDA(cudaMemcpyAsync(sv->d_par, p, sizeof *p, cudaMemcpyHostToDevice, s));
+    MG_CUDA(cudaMemcpyAsync(gr->d_par, p, sizeof *p, cudaMemcpyHostToDevice, s));
     return MG_OK;
 }
 
-static int read_par(mg_solver* sv, cudaStream_t s)
+static int read_par(mg_graphs* gr, cudaStream_t s)
 {
-    MG_CUDA(cudaMemcpyAsync(sv->h_par, sv->d_par, sizeof *sv->h_par, cudaMemcpyDeviceToHost, s));
+    MG_CUDA(cudaMemcpyAsync(gr->h_par, gr->d_par, sizeof *gr->h_par, cudaMemcpyDeviceToHost, s));
     MG_CUDA(cudaStreamSynchronize(s));
     return MG_OK;
 }
 
-static int solver_finish(mg_solver* sv, cudaStream_t s, int* cycles_out, int* converged_out, double* history)
+static int solver_finish(mg_graphs* gr, cudaStream_t s, int* cycles_out, int* converged_out, double* history)
 {
-    const int k = sv->h_par->k;
+    const int k = gr->h_par->k;
     if (history && k > 0) {
-        MG_CUDA(cudaMemcpyAsync(history, sv->d_hist, 2 * (size_t)k * sizeof(double), cudaMemcpyDeviceToHost, s));
+        MG_CUDA(cudaMemcpyAsync(history, gr->d_hist, 2 * (size_t)k * sizeof(double), cudaMemcpyDeviceToHost, s));
         MG_CUDA(cudaStreamSynchronize(s));
     }
     if (cycles_out) *cycles_out = k - 1;
-    if (converged_out) *converged_out = sv->h_par->converged;
+    if (converged_out) *converged_out = gr->h_par->converged;
     return MG_OK;
 }
 
-static int launch_check(const mg_solve_ops* ops, mg_solver* sv, int nhandles, cudaGraphConditionalHandle h0,
+static int launch_check(const mg_cycle_ops* ops, mg_graphs* gr, int nhandles, cudaGraphConditionalHandle h0,
                         cudaGraphConditionalHandle h1)
 {
-    MG_LAUNCH(*ops->launches, mgk_solve_check(ops->stream, ops->out2, sv->d_par, nhandles, h0, h1));
+    MG_LAUNCH(*ops->launches, mgk_solve_check(ops->stream, ops->out2, gr->d_par, nhandles, h0, h1));
     return MG_OK;
 }
 
 /* host-driven: the family's own cycle call, the norm pass and the check kernel, one read-back per cycle */
-static int solve_host(const mg_solve_ops* ops, mg_solver* sv)
+static int solve_host(const mg_cycle_ops* ops, mg_graphs* gr)
 {
     int st;
     if ((st = ops->norm(ops->ctx))) return st;
-    if ((st = launch_check(ops, sv, 0, 0, 0))) return st;
+    if ((st = launch_check(ops, gr, 0, 0, 0))) return st;
     for (;;) {
-        if ((st = read_par(sv, ops->stream))) return st;
-        if (sv->h_par->done) return MG_OK;
-        if ((st = ops->cycle(ops->ctx))) return st;
+        if ((st = read_par(gr, ops->stream))) return st;
+        if (gr->h_par->done) return MG_OK;
+        if ((st = ops->public_cycle(ops->ctx))) return st;
         if ((st = ops->norm(ops->ctx))) return st;
-        if ((st = launch_check(ops, sv, 0, 0, 0))) return st;
+        if ((st = launch_check(ops, gr, 0, 0, 0))) return st;
     }
 }
 
@@ -176,7 +241,7 @@ static int capture_segment_end(cudaStream_t s)
 
 /* norm(r_0) -> check -> WHILE { cycle -> norm -> check [-> IF { cycle -> norm -> check }] }, instantiated into slot->exec.
    Nothing runs; the host-side state the captured cycles changed is put back, and the launch counter too. */
-static int solve_build(const mg_solve_ops* ops, mg_solve_slot* slot, mg_solver* sv)
+static int solve_build(const mg_cycle_ops* ops, mg_graph_slot* slot, mg_graphs* gr)
 {
     cudaStream_t s = ops->stream;
     const long long l0 = *ops->launches;
@@ -190,14 +255,14 @@ static int solve_build(const mg_solve_ops* ops, mg_solve_slot* slot, mg_solver* 
 
     SOLVE_TRY(cudaStreamBeginCaptureToGraph(s, g, NULL, NULL, 0, cudaStreamCaptureModeThreadLocal));
     SOLVE_STEP(ops->norm(ops->ctx));
-    SOLVE_STEP(launch_check(ops, sv, 1, hw, 0));
+    SOLVE_STEP(launch_check(ops, gr, 1, hw, 0));
     SOLVE_STEP(add_conditional(s, hw, cudaGraphCondTypeWhile, &body));
     SOLVE_STEP(capture_segment_end(s));
     slot->launches[0] = *ops->launches - mark;
     mark = *ops->launches;
 
     SOLVE_TRY(cudaStreamBeginCaptureToGraph(s, body, NULL, NULL, 0, cudaStreamCaptureModeThreadLocal));
-    SOLVE_STEP(ops->capture_cycle(ops->ctx));
+    SOLVE_STEP(ops->cycle(ops->ctx));
     if (ops->save) {
         ops->save(ops->ctx, slot->snap[1]);
         slot->two = slot->snap[1][0] != slot->snap[0][0];
@@ -206,7 +271,7 @@ static int solve_build(const mg_solve_ops* ops, mg_solve_slot* slot, mg_solver* 
     }
     if (slot->two) SOLVE_TRY(cudaGraphConditionalHandleCreate(&hi, body, 0, cudaGraphCondAssignDefault));
     SOLVE_STEP(ops->norm(ops->ctx));
-    SOLVE_STEP(launch_check(ops, sv, slot->two ? 2 : 1, hw, hi));
+    SOLVE_STEP(launch_check(ops, gr, slot->two ? 2 : 1, hw, hi));
     if (slot->two) SOLVE_STEP(add_conditional(s, hi, cudaGraphCondTypeIf, &ibody));
     SOLVE_STEP(capture_segment_end(s));
     slot->launches[1] = *ops->launches - mark;
@@ -214,10 +279,10 @@ static int solve_build(const mg_solve_ops* ops, mg_solve_slot* slot, mg_solver* 
 
     if (slot->two) {
         SOLVE_TRY(cudaStreamBeginCaptureToGraph(s, ibody, NULL, NULL, 0, cudaStreamCaptureModeThreadLocal));
-        SOLVE_STEP(ops->capture_cycle(ops->ctx));
+        SOLVE_STEP(ops->cycle(ops->ctx));
         ops->save(ops->ctx, slot->snap[2]);
         SOLVE_STEP(ops->norm(ops->ctx));
-        SOLVE_STEP(launch_check(ops, sv, 1, hw, 0));
+        SOLVE_STEP(launch_check(ops, gr, 1, hw, 0));
         SOLVE_STEP(capture_segment_end(s));
         slot->launches[2] = *ops->launches - mark;
         if (slot->snap[2][0] != slot->snap[0][0]) {
@@ -242,27 +307,28 @@ out:
     return st;
 }
 
-int mg_solve_run(const mg_solve_ops* ops, mg_solver* sv, mg_solve_slot* slot, double rtol, double atol, int max_cycles,
-                 int* cycles_out, int* converged_out, double* history)
+int mg_solve_run(mg_graphs* gr, const int key[MG_GRAPH_KEY], const mg_cycle_ops* ops, double rtol, double atol,
+                 int max_cycles, int* cycles_out, int* converged_out, double* history)
 {
     cudaStream_t s = ops->stream;
-    int st = solver_begin(sv, s, rtol, atol, max_cycles, history != NULL);
+    mg_graph_slot* slot = key ? slot_for(gr->solves, MG_SOLVE_SLOTS, key) : NULL; /* NULL: the solve runs host-driven */
+    int st = solver_begin(gr, s, rtol, atol, max_cycles, history != NULL);
     if (st) return st;
     /* like the cycle graphs: a capture only after an eager run of the same cycle (kernel attributes, lazily loaded
        modules and lazily allocated buffers must exist before it) */
-    if (slot && slot->warm && !slot->exec && !slot->failed && solve_build(ops, slot, sv) != MG_OK) slot->failed = 1;
+    if (slot && slot->warm && !slot->exec && !slot->failed && solve_build(ops, slot, gr) != MG_OK) slot->failed = 1;
     if (!slot || !slot->exec) {
-        if ((st = solve_host(ops, sv))) return st;
-        if (slot && sv->h_par->k > 1) slot->warm = 1;
-        return solver_finish(sv, s, cycles_out, converged_out, history);
+        if ((st = solve_host(ops, gr))) return st;
+        if (slot && gr->h_par->k > 1) slot->warm = 1;
+        return solver_finish(gr, s, cycles_out, converged_out, history);
     }
     MG_CUDA(cudaGraphLaunch(slot->exec, s));
-    if ((st = read_par(sv, s))) return st;
-    const int cycles = sv->h_par->k - 1;
+    if ((st = read_par(gr, s))) return st;
+    const int cycles = gr->h_par->k - 1;
     *ops->launches += slot->launches[0];
     for (int c = 1; c <= cycles; c++) *ops->launches += slot->launches[slot->two && c % 2 == 0 ? 2 : 1];
     if (ops->load) ops->load(ops->ctx, cycles == 0 ? slot->snap[0] : (slot->two && cycles % 2 == 0) ? slot->snap[2] : slot->snap[1]);
-    return solver_finish(sv, s, cycles_out, converged_out, history);
+    return solver_finish(gr, s, cycles_out, converged_out, history);
 }
 
 int mg_require_device(void)

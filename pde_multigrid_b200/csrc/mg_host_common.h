@@ -1,6 +1,6 @@
 /*
  * mg_host_common.h -- shared helpers of the C host drivers: error reporting, CUDA call checking,
- * pitched-layout arithmetic.  Internal; the public ABI is include/mg_b200.h.
+ * pitched-layout arithmetic, the CUDA-graph cache of cycles and solves.  Internal; the public ABI is include/mg_b200.h.
  */
 #ifndef MG_HOST_COMMON_H
 #define MG_HOST_COMMON_H
@@ -52,51 +52,79 @@ static inline int mg_num_levels_for(int n)
 int mg_tma_make_colour_map(void* out128, int dtype, void* base, const mg_geom3d* g, int box_i, int box_y);
 int mg_require_device(void); /* MG_OK, or MG_ERR_CUDA with a message: there is no CPU fallback */
 
-/* ---- tolerance-driven solve, shared by the four families (mg?d_solve) ----
-   Device loop: one graph  norm(r_0) -> check -> WHILE { cycle -> norm -> check }.  When a cycle does not end on the
-   buffers it started on (the 3D temporally blocked smoother ping-pongs), the body holds two cycles:
-   cycle(s0 -> s1) -> norm -> check -> IF { cycle(s1 -> s0) -> norm -> check }.
-   Host loop: the same kernels and the same check kernel, one read-back of the parameter block per cycle. */
+/* ---- CUDA-graph cache of a handle, shared by the four families ----
+   Cycle graphs (mg_graph_cycle, the public *_vcycle of 2D and 3D): a whole V-cycle is dozens to hundreds of dependent
+   launches, most of them tiny, so replaying it from a graph removes the per-launch gaps.  The first call with a key runs
+   eagerly (kernel attributes, lazily loaded modules and lazily allocated buffers must exist before a capture), the second
+   captures and launches the graph, later calls replay it.
+   Solve graphs (mg_solve_run, every *_solve): one graph  norm(r_0) -> check -> WHILE { cycle -> norm -> check }.  When a
+   cycle does not end on the buffers it started on (the 3D temporally blocked smoother ping-pongs), the body holds two
+   cycles: cycle(s0 -> s1) -> norm -> check -> IF { cycle(s1 -> s0) -> norm -> check }.  The first solve of a key runs
+   host-driven: the same kernels and the same check kernel, one read-back of the parameter block per cycle.
+   Either way nothing runs while a graph is captured, so the host-side state and the counters the captured cycle changed
+   are put back; a replay applies the end state and adds the counts an eager run would have added. */
+
+/* a cycle estimated to make more launches than this runs eagerly: it is not dominated by launch gaps, and its graph
+   would be large to capture and keep */
+#define MG_GRAPH_MAX_LAUNCHES 4096
+#define MG_GRAPH_KEY 7     /* (level, v1, v2, smoother, arith, buffer bits, ghost bits); the families use a prefix */
+#define MG_GRAPH_KEY_SMOOTHER 3
+#define MG_CYCLE_SLOTS 16
+#define MG_SOLVE_SLOTS 8
+
 typedef struct {
-    mg_solve_par* h_par; /* pinned */
+    int used, key[MG_GRAPH_KEY];
+    int warm;              /* a call with this key has run eagerly (a solve: host-driven, at least one cycle) */
+    int failed;            /* solve graphs: the build failed, the key stays host-driven */
+    int two;               /* solve graphs: the body holds two cycles */
+    unsigned snap[3][2];   /* family state (ops.save) at the start, after the first and after the second captured cycle */
+    cudaGraphExec_t exec;
+    long long launches[3]; /* cycle: [0] the cycle; solve: norm(r_0) + check; first body cycle + norm + check; second */
+    long long halo_bytes;  /* cycle graphs: what the captured cycle added to *ops.halo_bytes */
+} mg_graph_slot;
+
+typedef struct {
+    int enabled;           /* 0: MG_B200_NO_GRAPH, or a cycle could not be captured: everything runs eagerly */
+    mg_graph_slot cycles[MG_CYCLE_SLOTS];
+    mg_graph_slot solves[MG_SOLVE_SLOTS];
+    /* the solve's parameter block and history on the device */
+    mg_solve_par* h_par;   /* pinned */
     mg_solve_par* d_par;
     double* d_hist;
-    int hist_cap;        /* pairs d_hist has room for */
-} mg_solver;
+    int hist_cap;          /* pairs d_hist has room for */
+} mg_graphs;
 
-#define MG_SOLVE_SLOTS 8
-#define MG_SOLVE_KEY 6
-typedef struct {
-    int used, failed;
-    int warm;            /* a host-driven solve with this key has run a cycle: everything a capture needs exists */
-    int key[MG_SOLVE_KEY];
-    int two;             /* the body holds two cycles */
-    unsigned snap[3][2]; /* family state (ops.save) at the start, after the first and after the second body cycle */
-    cudaGraphExec_t exec;
-    long long launches[3]; /* norm(r_0) + check; first body cycle + norm + check; second */
-} mg_solve_slot;
-
+/* what the cache needs of a family to run, capture and replay one cycle on one level with fixed sweep counts */
 typedef struct {
     void* ctx;
     cudaStream_t stream;
-    const double* out2;       /* where norm() leaves {sum of squares, max} */
-    long long* launches;      /* the handle's kernel counter */
-    int (*norm)(void* ctx);   /* enqueue the norm pass of the solve's level into out2 */
-    int (*cycle)(void* ctx);  /* one cycle the way the family's public *_vcycle runs it (host loop) */
-    int (*capture_cycle)(void* ctx); /* one cycle as plain launches (device loop) */
+    long long* launches;            /* the handle's kernel counter */
+    long long* halo_bytes;          /* NULL, or a second counter the cycle advances (3D; solve graphs exist only where it
+                                       stays put, on one GPU) */
+    int (*cycle)(void* ctx);        /* one cycle as plain launches: what is captured, and what an eager call runs */
+    int (*public_cycle)(void* ctx); /* one cycle the way the family's public *_vcycle runs it (host-driven solve) */
+    int (*norm)(void* ctx);         /* enqueue the norm pass of the cycle's level into out2 */
+    const double* out2;             /* where norm() leaves {sum of squares, max} */
     /* NULL for families whose cycle always ends on the buffers it started on; otherwise the host-side state:
-       [0] = which buffer every level works on (must return to its start value), [1] = further bookkeeping */
+       [0] = which buffer every level works on, [1] = further bookkeeping */
     void (*save)(void* ctx, unsigned out[2]);
     void (*load)(void* ctx, const unsigned in[2]);
-} mg_solve_ops;
+} mg_cycle_ops;
+
+void mg_graphs_init(mg_graphs* gr); /* reads MG_B200_NO_GRAPH */
+void mg_graphs_free(mg_graphs* gr);
+/* graphs may be used: the cache is enabled, per-operator timers are off (they need eager launches) and the cycle's
+   launch estimate is at most MG_GRAPH_MAX_LAUNCHES */
+int mg_graphs_on(const mg_graphs* gr, int profiling, long long launches_per_cycle);
+/* drops every cycle and solve graph whose key[pos] == value */
+void mg_graphs_drop(mg_graphs* gr, int pos, int value);
+/* one cycle: eager when key is NULL, the cache is full or the key is new; otherwise captured on first need, then replayed */
+int mg_graph_cycle(mg_graphs* gr, const int key[MG_GRAPH_KEY], const mg_cycle_ops* ops);
 
 int mg_solve_check_args(double rtol, double atol, int max_cycles, int v1, int v2);
-/* slot with this key, or a free one (NULL: the cache is full, the solve runs host-driven) */
-mg_solve_slot* mg_solve_slot_for(mg_solve_slot slots[MG_SOLVE_SLOTS], const int key[MG_SOLVE_KEY]);
-/* the whole solve: device-driven when slot != NULL, it is warm and its graph builds; host-driven otherwise */
-int mg_solve_run(const mg_solve_ops* ops, mg_solver* sv, mg_solve_slot* slot, double rtol, double atol, int max_cycles,
-                 int* cycles_out, int* converged_out, double* history);
-void mg_solve_free(mg_solver* sv, mg_solve_slot slots[MG_SOLVE_SLOTS]);
+/* the whole solve: device-driven when key != NULL, the key is warm and its graph builds; host-driven otherwise */
+int mg_solve_run(mg_graphs* gr, const int key[MG_GRAPH_KEY], const mg_cycle_ops* ops, double rtol, double atol,
+                 int max_cycles, int* cycles_out, int* converged_out, double* history);
 
 #ifdef __cplusplus
 }
