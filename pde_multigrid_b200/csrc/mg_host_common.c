@@ -1,6 +1,7 @@
 /* mg_host_common.c -- error state, device probing and the CUDA-graph cache shared by the host drivers. */
 #include "mg_host_common.h"
 
+#include <math.h>
 #include <stdarg.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -119,10 +120,125 @@ int mg_graph_cycle(mg_graphs* gr, const int key[MG_GRAPH_KEY], const mg_cycle_op
     return MG_OK;
 }
 
+/* ---- the handle core -------------------------------------------------------------------------- */
+
+int mg_core_init(mg_core* c)
+{
+    mg_graphs_init(&c->graphs);
+    MG_CUDA(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
+    MG_CUDA(cudaMallocHost((void**)&c->h_out2, 2 * sizeof(double)));
+    return MG_OK;
+}
+
+void mg_core_free(mg_core* c)
+{
+    if (c->stream) cudaStreamSynchronize(c->stream);
+    mg_graphs_free(&c->graphs);
+    if (c->stream) cudaStreamDestroy(c->stream);
+    if (c->h_out2) cudaFreeHost(c->h_out2);
+    mg_prof_free(&c->prof);
+}
+
+int mg_check_level(const mg_core* c, int level)
+{
+    if (!c) return mg_fail(MG_ERR_ARG, "null handle");
+    if (level < 0 || level >= c->nlevels) return mg_fail(MG_ERR_ARG, "level %d out of range [0,%d)", level, c->nlevels);
+    return MG_OK;
+}
+
+int mg_check_fine_level(const mg_core* c, int level)
+{
+    int st = mg_check_level(c, level);
+    if (st) return st;
+    if (level == c->nlevels - 1) return mg_fail(MG_ERR_ARG, "level %d is the coarsest", level);
+    return MG_OK;
+}
+
+int mg_sync(mg_core* c)
+{
+    if (!c) return mg_fail(MG_ERR_ARG, "null handle");
+    MG_CUDA(cudaStreamSynchronize(c->stream));
+    return MG_OK;
+}
+
+int mg_profile_enable(mg_core* c, int enable)
+{
+    if (!c) return mg_fail(MG_ERR_ARG, "null handle");
+    return mg_prof_enable(&c->prof, c->stream, enable);
+}
+
+int mg_profile_read(mg_core* c, int level, int op, double* ms_total, long long* kernel_launches, long long* calls)
+{
+    int st = mg_check_level(c, level);
+    if (st) return st;
+    if (op < 0 || op >= MG_OP_COUNT) return mg_fail(MG_ERR_ARG, "bad op %d", op);
+    if ((st = mg_prof_collect(&c->prof, c->stream))) return st;
+    if (ms_total) *ms_total = c->prof.ms[level][op];
+    if (kernel_launches) *kernel_launches = c->prof.kl[level][op];
+    if (calls) *calls = c->prof.calls[level][op];
+    return MG_OK;
+}
+
+int mg_read_out2(mg_core* c, const double* d_out2)
+{
+    MG_CUDA(cudaMemcpyAsync(c->h_out2, d_out2, 2 * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    MG_CUDA(cudaStreamSynchronize(c->stream));
+    return MG_OK;
+}
+
+int mg_read_norm(mg_core* c, const double* d_out2, double* l2, double* linf)
+{
+    int st = mg_read_out2(c, d_out2);
+    if (st) return st;
+    if (l2) *l2 = sqrt(c->h_out2[0]);
+    if (linf) *linf = c->h_out2[1];
+    return MG_OK;
+}
+
+/* ---- the reference's operators on caller arrays ----------------------------------------------- */
+
+int mg_tmp_begin(mg_core* c, void** da, size_t na, const void* ha, void** db, size_t nb, const void* hb)
+{
+    const size_t es = mg_esize(c->dtype);
+    *da = *db = NULL;
+    cudaError_t e = cudaMalloc(da, na * es);
+    if (e == cudaSuccess && nb) e = cudaMalloc(db, nb * es);
+    if (e == cudaSuccess && ha) e = cudaMemcpyAsync(*da, ha, na * es, cudaMemcpyHostToDevice, c->stream);
+    if (e == cudaSuccess && hb && nb) e = cudaMemcpyAsync(*db, hb, nb * es, cudaMemcpyHostToDevice, c->stream);
+    if (e == cudaSuccess) return MG_OK;
+    cudaFree(*da);
+    cudaFree(*db);
+    *da = *db = NULL;
+    return mg_fail(MG_ERR_CUDA, "temporary device arrays: %s", cudaGetErrorString(e));
+}
+
+int mg_tmp_finish(mg_core* c, int k, void* host_out, const void* dev_out, size_t n, void* da, void* db)
+{
+    cudaError_t e = cudaSuccess;
+    if (k >= 0 && host_out) e = cudaMemcpyAsync(host_out, dev_out, n * mg_esize(c->dtype), cudaMemcpyDeviceToHost, c->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+    cudaFree(da);
+    if (db) cudaFree(db);
+    if (k < 0) return mg_fail(MG_ERR_CUDA, "launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+    if (e != cudaSuccess) return mg_fail(MG_ERR_CUDA, "copy failed: %s", cudaGetErrorString(e));
+    c->launches += k;
+    return MG_OK;
+}
+
+int mg_launch_done(mg_core* c, int k)
+{
+    if (k < 0) return mg_fail(MG_ERR_CUDA, "operator launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+    c->launches += k;
+    MG_CUDA(cudaStreamSynchronize(c->stream));
+    return MG_OK;
+}
+
 /* ---- tolerance-driven solve ------------------------------------------------------------------- */
 
-int mg_solve_check_args(double rtol, double atol, int max_cycles, int v1, int v2)
+int mg_solve_check_args(const mg_core* c, int level, double rtol, double atol, int max_cycles, int v1, int v2)
 {
+    int st = mg_check_level(c, level);
+    if (st) return st;
     if (!(rtol >= 0.0) || !(atol >= 0.0)) return mg_fail(MG_ERR_ARG, "rtol and atol must be >= 0 (got %g, %g)", rtol, atol);
     if (max_cycles < 0) return mg_fail(MG_ERR_ARG, "max_cycles %d < 0", max_cycles);
     if (v1 < 0 || v2 < 0) return mg_fail(MG_ERR_ARG, "negative sweep count");

@@ -1,6 +1,7 @@
 /*
  * mg_host_common.h -- shared helpers of the C host drivers: error reporting, CUDA call checking,
- * pitched-layout arithmetic, the CUDA-graph cache of cycles and solves.  Internal; the public ABI is include/mg_b200.h.
+ * pitched-layout arithmetic, the handle core every family embeds, operators on caller arrays, the CUDA-graph cache of
+ * cycles and solves.  Internal; the public ABI is include/mg_b200.h.
  */
 #ifndef MG_HOST_COMMON_H
 #define MG_HOST_COMMON_H
@@ -10,6 +11,7 @@
 
 #include "../../include/mg_b200.h"
 #include "mg_launch.h"
+#include "mg_profile.h"
 
 #ifdef __cplusplus
 extern "C" {
@@ -121,10 +123,58 @@ void mg_graphs_drop(mg_graphs* gr, int pos, int value);
 /* one cycle: eager when key is NULL, the cache is full or the key is new; otherwise captured on first need, then replayed */
 int mg_graph_cycle(mg_graphs* gr, const int key[MG_GRAPH_KEY], const mg_cycle_ops* ops);
 
-int mg_solve_check_args(double rtol, double atol, int max_cycles, int v1, int v2);
+/* what a family's mg_cycle_ops callbacks get as ctx: one cycle of handle h on `level` with fixed sweep counts */
+typedef struct {
+    void* h;
+    int level, v1, v2;
+} mg_cycle_ctx;
+
 /* the whole solve: device-driven when key != NULL, the key is warm and its graph builds; host-driven otherwise */
 int mg_solve_run(mg_graphs* gr, const int key[MG_GRAPH_KEY], const mg_cycle_ops* ops, double rtol, double atol,
                  int max_cycles, int* cycles_out, int* converged_out, double* history);
+
+/* ---- the handle core ----
+   Every family's handle (mg1d_s, mg2d_s, mg3b_s, mg3d_s) has an mg_core named `core`.  A public call passes
+   MG_CORE(handle) to the checking helpers below: NULL for a NULL handle, which they report as "null handle". */
+typedef struct {
+    int dtype, nlevels;
+    cudaStream_t stream;  /* non-blocking: every operator of the handle runs on it */
+    long long launches;   /* kernel launches, *_kernel_launches */
+    double* h_out2;       /* pinned {sum of squares, max} read-back */
+    mg_prof prof;         /* per-operator timers; the box engine never enables them */
+    mg_graphs graphs;
+} mg_core;
+
+/* the stream, h_out2 and the graph cache; dtype and nlevels are the family's to set.  On failure the family frees the
+   handle as usual: mg_core_free takes a partly initialised core, once. */
+int mg_core_init(mg_core* c);
+void mg_core_free(mg_core* c); /* synchronises the stream first */
+
+#define MG_CORE(h) ((h) ? &(h)->core : NULL)
+
+int mg_check_level(const mg_core* c, int level);
+int mg_check_fine_level(const mg_core* c, int level); /* ... and level is not the coarsest */
+int mg_sync(mg_core* c);
+int mg_profile_enable(mg_core* c, int enable);
+int mg_profile_read(mg_core* c, int level, int op, double* ms_total, long long* kernel_launches, long long* calls);
+/* the arguments of a *_solve: mg_check_level, then the tolerances and counts */
+int mg_solve_check_args(const mg_core* c, int level, double rtol, double atol, int max_cycles, int v1, int v2);
+int mg_read_out2(mg_core* c, const double* d_out2); /* d_out2[0..1] -> c->h_out2, synchronised */
+int mg_read_norm(mg_core* c, const double* d_out2, double* l2, double* linf); /* l2 = sqrt(sum of squares), linf = max */
+
+/* per-operator timers around a family operator; h is a family handle */
+#define PROF_BEGIN(h, level, op) mg_prof_begin(&(h)->core.prof, (h)->core.stream, (level), (op), (h)->core.launches)
+#define PROF_END(h) mg_prof_end(&(h)->core.prof, (h)->core.stream, (h)->core.launches)
+
+/* ---- the reference's operators on caller arrays ----
+   Host arrays: up to two dense device temporaries (*da of na elements, *db of nb, none when nb == 0), uploaded from ha /
+   hb when given; then the family launches one kernel on them and mg_tmp_finish downloads n elements of dev_out into
+   host_out, frees both temporaries and counts the launch (k: the launcher's return value).  Nothing leaks on any error
+   path.  Device arrays: the kernel runs in place and mg_launch_done counts it and synchronises the stream (the caller's
+   next access may be on any stream). */
+int mg_tmp_begin(mg_core* c, void** da, size_t na, const void* ha, void** db, size_t nb, const void* hb);
+int mg_tmp_finish(mg_core* c, int k, void* host_out, const void* dev_out, size_t n, void* da, void* db);
+int mg_launch_done(mg_core* c, int k);
 
 #ifdef __cplusplus
 }

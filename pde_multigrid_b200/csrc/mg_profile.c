@@ -1,5 +1,5 @@
 /* mg_profile.c -- see mg_profile.h */
-#include "mg_profile.h"
+#include "mg_host_common.h"
 
 #include <stdlib.h>
 #include <string.h>

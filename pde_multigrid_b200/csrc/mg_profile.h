@@ -7,7 +7,9 @@
 #ifndef MG_PROFILE_H
 #define MG_PROFILE_H
 
-#include "mg_host_common.h"
+#include <cuda_runtime_api.h>
+
+#include "../../include/mg_b200.h"
 
 #define MG_PROF_MAX_LEVELS 32
 
