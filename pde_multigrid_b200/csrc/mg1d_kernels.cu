@@ -147,11 +147,11 @@ __global__ void __launch_bounds__(1024) k_ops1d(T* arena, mg_hier1d H, int op, i
             for (int j = threadIdx.x; j < L.n; j += blockDim.x) {
                 const double r = (double)residual1d_at(L, j, corrected);
                 s += r * r;
-                m = fmax(m, fabs(r));
+                m = max_nan(m, fabs(r));
             }
             for (int o = 16; o > 0; o >>= 1) {
                 s += __shfl_xor_sync(0xffffffffu, s, o);
-                m = fmax(m, __shfl_xor_sync(0xffffffffu, m, o));
+                m = max_nan(m, __shfl_xor_sync(0xffffffffu, m, o));
             }
             const int w = threadIdx.x >> 5, l = threadIdx.x & 31, nw = (blockDim.x + 31) >> 5;
             if (l == 0) { sh[w] = s; sh[32 + w] = m; }
@@ -161,7 +161,7 @@ __global__ void __launch_bounds__(1024) k_ops1d(T* arena, mg_hier1d H, int op, i
                 m = l < nw ? sh[32 + l] : 0.0;
                 for (int o = 16; o > 0; o >>= 1) {
                     s += __shfl_xor_sync(0xffffffffu, s, o);
-                    m = fmax(m, __shfl_xor_sync(0xffffffffu, m, o));
+                    m = max_nan(m, __shfl_xor_sync(0xffffffffu, m, o));
                 }
                 if (l == 0) { out2[0] = s; out2[1] = m; }
             }
@@ -263,7 +263,7 @@ __global__ void __launch_bounds__(256) k_abs_error1(const T* __restrict__ v, con
     for (int i = threadIdx.x; i < n; i += blockDim.x) {
         const double d = fabs((double)mgx::sub(v[i], table[i]));
         s += d;
-        m = fmax(m, d);
+        m = max_nan(m, d);
     }
     ss[threadIdx.x] = s;
     sm[threadIdx.x] = m;
@@ -271,7 +271,7 @@ __global__ void __launch_bounds__(256) k_abs_error1(const T* __restrict__ v, con
     for (int o = 128; o > 0; o >>= 1) {
         if ((int)threadIdx.x < o) {
             ss[threadIdx.x] += ss[threadIdx.x + o];
-            sm[threadIdx.x] = fmax(sm[threadIdx.x], sm[threadIdx.x + o]);
+            sm[threadIdx.x] = max_nan(sm[threadIdx.x], sm[threadIdx.x + o]);
         }
         __syncthreads();
     }

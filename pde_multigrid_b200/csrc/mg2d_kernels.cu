@@ -159,7 +159,7 @@ __device__ __forceinline__ void block_reduce_sum_max(double& s, double& m, doubl
 {
     for (int o = 16; o > 0; o >>= 1) {
         s += __shfl_xor_sync(0xffffffffu, s, o);
-        m = fmax(m, __shfl_xor_sync(0xffffffffu, m, o));
+        m = max_nan(m, __shfl_xor_sync(0xffffffffu, m, o));
     }
     const int w = threadIdx.x >> 5, l = threadIdx.x & 31, nw = (blockDim.x + 31) >> 5;
     if (l == 0) { sh[w] = s; sh[32 + w] = m; }
@@ -169,7 +169,7 @@ __device__ __forceinline__ void block_reduce_sum_max(double& s, double& m, doubl
         m = (l < nw) ? sh[32 + l] : 0.0;
         for (int o = 16; o > 0; o >>= 1) {
             s += __shfl_xor_sync(0xffffffffu, s, o);
-            m = fmax(m, __shfl_xor_sync(0xffffffffu, m, o));
+            m = max_nan(m, __shfl_xor_sync(0xffffffffu, m, o));
         }
     }
 }
@@ -196,7 +196,7 @@ __global__ void k_reduce(const T* __restrict__ v, const T* __restrict__ f, mg_ge
                 d = fabs((double)sub(v[i], real));
                 s += d;
             }
-            m = fmax(m, fabs(d));
+            m = max_nan(m, fabs(d));
         }
     block_reduce_sum_max(s, m, sh);
     if (threadIdx.x == 0) { part[blockIdx.x] = s; part[gridDim.x + blockIdx.x] = m; }
@@ -208,7 +208,7 @@ __global__ void k_reduce_final(const double* __restrict__ part, int nparts, doub
     double s = 0.0, m = 0.0;
     for (int i = threadIdx.x; i < nparts; i += blockDim.x) {
         s += part[i];
-        m = fmax(m, part[nparts + i]);
+        m = max_nan(m, part[nparts + i]);
     }
     block_reduce_sum_max(s, m, sh);
     if (threadIdx.x == 0) { out2[0] = s; out2[1] = m; }

@@ -137,7 +137,7 @@ __global__ void __launch_bounds__(256) k_bs_norm(const T* __restrict__ v, const 
         const int x = (int)(i % g.nx), y = (int)((i / g.nx) % g.ny), z = (int)(i / ((long long)g.nx * g.ny));
         const double r = (double)residual_s<T, FAST>(v, f, g, x, y, z, c, corrected);
         s += r * r;
-        m = fmax(m, fabs(r));
+        m = max_nan(m, fabs(r));
     }
     block_sum_max(s, m, sh);
     if (threadIdx.x == 0) { parts[blockIdx.x] = s; parts[nparts + blockIdx.x] = m; }
@@ -147,7 +147,7 @@ __global__ void k_bs_norm_final(const double* __restrict__ parts, int nparts, do
 {
     if (threadIdx.x || blockIdx.x) return;
     double s = 0.0, m = 0.0;
-    for (int i = 0; i < nparts; i++) { s += parts[i]; m = fmax(m, parts[nparts + i]); }
+    for (int i = 0; i < nparts; i++) { s += parts[i]; m = max_nan(m, parts[nparts + i]); }
     out2[0] = s;
     out2[1] = m;
 }

@@ -72,7 +72,7 @@ __device__ __forceinline__ void block_sum_max(double& s, double& m, double* sh)
 {
     for (int o = 16; o > 0; o >>= 1) {
         s += __shfl_xor_sync(0xffffffffu, s, o);
-        m = fmax(m, __shfl_xor_sync(0xffffffffu, m, o));
+        m = max_nan(m, __shfl_xor_sync(0xffffffffu, m, o));
     }
     const int w = threadIdx.x >> 5, l = threadIdx.x & 31, nw = (blockDim.x + 31) >> 5;
     if (l == 0) { sh[w] = s; sh[32 + w] = m; }
@@ -82,7 +82,7 @@ __device__ __forceinline__ void block_sum_max(double& s, double& m, double* sh)
         m = (l < nw) ? sh[32 + l] : 0.0;
         for (int o = 16; o > 0; o >>= 1) {
             s += __shfl_xor_sync(0xffffffffu, s, o);
-            m = fmax(m, __shfl_xor_sync(0xffffffffu, m, o));
+            m = max_nan(m, __shfl_xor_sync(0xffffffffu, m, o));
         }
     }
 }

@@ -66,7 +66,7 @@ k_abs_error(const T* __restrict__ v, mg_geom3d g, const double* __restrict__ sx,
             const T real_sol = (T)__dmul_rn(__dmul_rn(sx[x], syz), szz);
             const double d = fabs((double)sub(real_sol, v[off3(g, x, y, zl)]));
             s += d;
-            m = fmax(m, d);
+            m = max_nan(m, d);
         }
     }
     block_sum_max(s, m, sh);

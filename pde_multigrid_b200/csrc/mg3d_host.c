@@ -149,7 +149,8 @@ static void level_coefs(int dtype, int n, const double* range, double h[3], mg_c
     /* exact-arithmetic shortcuts (mg_exact.cuh): a power of two has frexp mantissa 0.5; den = 6*2^e has 0.75 */
     int e;
     c->fast_h = frexp(c->hx2, &e) == 0.5 && frexp(c->hy2, &e) == 0.5 && frexp(c->hz2, &e) == 0.5;
-    c->fast_den = c->fast_h && frexp(c->den, &e) == 0.75;
+    /* ... and its reciprocal must be finite: a subnormal den (float h <= 2^-33, double h <= 2^-257) has 1/den = inf */
+    c->fast_den = c->fast_h && frexp(c->den, &e) == 0.75 && isfinite(c->rden);
     if (getenv("MG_B200_IEEE_DIV")) c->fast_h = c->fast_den = 0;
 }
 
@@ -990,7 +991,7 @@ static int relax_launch(mg3d_t* mg, mg_level3d* L, int colour, int lo, int hi, i
 static int level_takes_pipe(const mg3d_t* mg, const mg_level3d* L)
 {
     return (mg->smoother == MG_SMOOTHER_PIPE || (mg->smoother == MG_SMOOTHER_AUTO && !mg->no_pipe)) && L->has_tma && L->vbuf[1] &&
-           L->c.fast_den && L->iso && (!L->dist || L->own_hi - L->own_lo >= 8);
+           L->c.fast_den && L->iso && mgk3d_pipe_exact_range(mg->core.dtype, L->c.hx2) && (!L->dist || L->own_hi - L->own_lo >= 8);
 }
 
 static int relax_overlaps(const mg3d_t* mg, int level)

@@ -123,7 +123,7 @@ k_residual_norm(const T* __restrict__ v, const T* __restrict__ f, mg_geom3d g, C
         for (int x = 1 + threadIdx.x; x <= g.n - 2; x += blockDim.x) {
             const double rd = (double)residual_at<T, FAST>(v, f, g, x, y, zl, c, corrected);
             s += rd * rd;
-            m = fmax(m, fabs(rd));
+            m = max_nan(m, fabs(rd));
         }
     }
     block_sum_max(s, m, sh);
@@ -136,7 +136,7 @@ __global__ void k_norm_final(const double* __restrict__ part, int nparts, double
     double s = 0.0, m = 0.0;
     for (int i = threadIdx.x; i < nparts; i += blockDim.x) {
         s += part[i];
-        m = fmax(m, part[nparts + i]);
+        m = max_nan(m, part[nparts + i]);
     }
     block_sum_max(s, m, sh);
     if (threadIdx.x == 0) { out2[0] = s; out2[1] = m; }

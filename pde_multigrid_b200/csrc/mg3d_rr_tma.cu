@@ -228,7 +228,7 @@ k_residual_restrict_tma(const __grid_constant__ CUtensorMap map_c0, const __grid
                 for (int j = 0; j < 4; j++) {
                     const double rd = (double)res[j];
                     nsum += rd * rd;
-                    nmax = fmax(nmax, fabs(rd));
+                    nmax = max_nan(nmax, fabs(rd));
                 }
             }
         } else {

@@ -447,28 +447,40 @@ size_t smem_bytes_t(bool corr)
 //     of the reference is still exact, and with lo >= -697 + 2k the Markstein residual stays normal (mg_exact.cuh);
 //   * float has no exponent range to spare for that argument: every stage output is checked as well and the quotient is
 //     the IEEE division, which leaves lo >= -126 + 6k for the products;
-//   * hi: four stages of sums of six can grow a value by less than 2^7.
-template <typename T> void guard_window(double h2, unsigned* glo, unsigned* gspan);
-template <> void guard_window<double>(double h2, unsigned* glo, unsigned* gspan)
+//   * hi, h <= 1 (k >= 0): four stages of sums of six can grow a value by less than 2^7;
+//   * h > 1 (k < 0): the reference's products scale values UP, x*h^4 = x*2^(-4k) and f*h^6 = f*2^(-6k), and a stage adds
+//     f*h^2/6 = f*2^(-2k)/6 to what it passes on.  With every checked value below 2^(hi+1), a stage value stays below
+//     2^(hi+1-2k) (double: after the four stages; float checks each), so the reference's numerator
+//     6*|x|*h^4 + |f|*h^6 stays below 2^(hi+4-6k): hi = hi(k=0) + 6k keeps it under 2^1014 (double) / 2^118 (float), where
+//     neither it nor any partial sum or product can overflow.  Nothing of the reference underflows sooner than at
+//     k = 0, and f*h^2 is no finer than f, so the lower bounds of k = 0 hold: lo = lo(k=0).
+// Returns 0 when the window is empty: the pass would have nothing it may compute, so the level takes the literal kernels
+// (mgk3d_pipe_exact_range).
+template <typename T> int guard_window(double h2, unsigned* glo, unsigned* gspan);
+template <> int guard_window<double>(double h2, unsigned* glo, unsigned* gspan)
 {
     int e;
     frexp(h2, &e);  // h2 = 2^(e-1) = 2^(-2k)
-    const int k = -(e - 1) / 2;
-    const int a = -857 + 6 * k, b = -697 + 2 * k;
-    const int lo = (a > b ? a : b) + 8, hi = 1010;
+    const int k = -(e - 1) / 2, kl = k > 0 ? k : 0, kh = k < 0 ? k : 0;
+    const int a = -857 + 6 * kl, b = -697 + 2 * kl;
+    const int lo = (a > b ? a : b) + 8, hi = 1010 + 6 * kh;
+    if (lo > hi) return 0;
     const unsigned L = (unsigned)(lo + 1023) << 20, H = (((unsigned)(hi + 1023 + 1)) << 20) - 1;
     *glo = L;
     *gspan = H - L;
+    return 1;
 }
-template <> void guard_window<float>(double h2, unsigned* glo, unsigned* gspan)
+template <> int guard_window<float>(double h2, unsigned* glo, unsigned* gspan)
 {
     int e;
     frexp(h2, &e);
-    const int k = -(e - 1) / 2;
-    const int lo = -126 + 6 * k + 4, hi = 115;
+    const int k = -(e - 1) / 2, kl = k > 0 ? k : 0, kh = k < 0 ? k : 0;
+    const int lo = -126 + 6 * kl + 4, hi = 115 + 6 * kh;
+    if (lo > hi) return 0;
     const unsigned L = (unsigned)(lo + 127) << 23, H = (((unsigned)(hi + 127 + 1)) << 23) - 1;
     *glo = L;
     *gspan = H - L;
+    return 1;
 }
 
 template <typename T, int ARITH, bool CORR>
@@ -476,8 +488,8 @@ int launch_k(cudaStream_t s, const PipeMaps& m, const T* v_in, T* v_out, mg_geom
              unsigned int* flag, mg_geom3d gc)
 {
     MG_SET_SMEM_LIMIT((k_relax_pipe2<T, ARITH, CORR>), smem_bytes_t<T>(CORR));
-    unsigned glo, gspan;
-    guard_window<T>(c.hx2, &glo, &gspan);
+    unsigned glo = 0, gspan = 0;
+    if (!guard_window<T>(c.hx2, &glo, &gspan)) return -1;
     const T y6 = T(1) / T(6);
     k_relax_pipe2<T, ARITH, CORR><<<grid, NT, smem_bytes_t<T>(CORR), s>>>(m, v_in, v_out, g, (T)c.hx2, y6, zchunk, zlo, zhi, glo, gspan, flag, gc);
     return cudaPeekAtLastError() == cudaSuccess ? 1 : -1;
@@ -553,4 +565,11 @@ extern "C" int mgk3d_relax_pipe2(cudaStream_t s, int dtype, const void* const ma
     (void)f;  // f only enters through its tensor maps
     if (dtype == 0) return launch<float>(s, maps3, coarse_maps2, gc, (const float*)v_in, (float*)v_out, g, c, zl_lo, zl_hi, arith, flag);
     return launch<double>(s, maps3, coarse_maps2, gc, (const double*)v_in, (double*)v_out, g, c, zl_lo, zl_hi, arith, flag);
+}
+
+/* 1 when the bit-exact pass has a nonempty range check for h^2 = hx2 (guard_window) */
+extern "C" int mgk3d_pipe_exact_range(int dtype, double hx2)
+{
+    unsigned lo, span;
+    return dtype == 0 ? guard_window<float>(hx2, &lo, &span) : guard_window<double>(hx2, &lo, &span);
 }

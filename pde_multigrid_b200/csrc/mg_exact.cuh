@@ -21,6 +21,10 @@ __device__ __forceinline__ float div(float a, float b) { return __fdiv_rn(a, b);
 __device__ __forceinline__ double fma_(double a, double b, double c) { return __fma_rn(a, b, c); }
 __device__ __forceinline__ float fma_(float a, float b, float c) { return __fmaf_rn(a, b, c); }
 
+// max that keeps a NaN (fmax drops it): the linf of a field with a NaN is NaN, like np.max(np.abs(r)).  For the
+// linf and abs-error reductions; every finite result is fmax's.
+__device__ __forceinline__ double max_nan(double a, double b) { return (a > b || a != a) ? a : b; }
+
 // Correctly rounded a/b from a correctly rounded reciprocal y = RN(1/b) computed once on the host
 // (Markstein 1990: q = RN(a*y); r = a - b*q exactly with one FMA; q' = RN(q + r*y) is the correctly
 // rounded quotient).  Three pipe operations instead of the ~20-instruction IEEE division sequence.

@@ -101,6 +101,8 @@ int mgk3d_relax_fused2(cudaStream_t s, int dtype, const void* const maps4[4], vo
 int mgk3d_relax_pipe2(cudaStream_t s, int dtype, const void* const maps3[3], const void* v_in, const void* f, void* v_out,
                       mg_geom3d g, mg_coef3d c, int zl_lo, int zl_hi, int arith, unsigned int* flag, const void* const coarse_maps2[2],
                       const mg_geom3d* gc);
+/* 1 when mgk3d_relax_pipe2 has a nonempty exactness range for h^2 = hx2 (otherwise it refuses to launch) */
+int mgk3d_pipe_exact_range(int dtype, double hx2);
 /* the coarse tail of a V-cycle in one launch (mg3d_tail.cu): V(v1,v2) on the sub-hierarchy g[0..nlev-1], g[0].n <=
    MGK3D_TAIL_N, every level resident in one CTA's shared memory */
 #define MGK3D_TAIL_N 17
