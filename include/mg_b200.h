@@ -154,6 +154,23 @@ int mg3d_fmg(mg3d_t* mg, int level, int v0, int v1, int v2);        /* FullMulti
  * from the host, one read-back per cycle.  Both give the same bits.  The mg3b / mg2d / mg1d versions are the same. */
 int mg3d_solve(mg3d_t* mg, int level, int v1, int v2, double rtol, double atol, int max_cycles,
                int* cycles_out, int* converged_out, double* history);
+/* Conjugate gradients preconditioned by one VCycle(level, v1, v2) per iteration (flexible, Polak-Ribiere: an RB
+ * Gauss-Seidel V-cycle is not a symmetric operator), for Laplacian_h v = f on `level` with v's boundary values as the
+ * Dirichlet data -- the operator of the MG_CORRECTED residual -- starting from the current v.  The preconditioner is
+ * VCycle from v = 0 with f = r and uses the handle's smoother, arithmetic mode and Jacobi weight.  Stopping rule and
+ * history as mg3d_solve, on the TRUE residual b - Laplacian_h x_k (the reference's residual expression, recomputed every
+ * iteration): ||r_k||_2 <= max(atol, rtol * ||r_0||_2), a non-finite l2 (which is also how a breakdown such as
+ * p.Laplacian p = 0 surfaces), or max_iters.  history[0] is mg3d_residual_norm(level) bit for bit.
+ * iters_out counts iterations, one V-cycle each.  On return v of `level` holds the iterate, f of `level` is the caller's
+ * bit for bit, v and f of the coarser levels hold preconditioner scratch (as after mg3d_vcycle); max_iters = 0, or an r_0
+ * that already meets the target, leaves v and f as they were.
+ * MG_ERR_ARG as mg3d_solve; MG_ERR_STATE on an MG_REF_COMPAT handle (its residual, N3/MultiGrid3D.cpp:723, is not a
+ * symmetric operator) and on a distributed handle (nranks > 1); nothing runs in either case.
+ * Memory: six fields of `level` (b, x and p twice, d), allocated by the first call on the level (MG_ERR_NOMEM before
+ * anything runs if that fails) and freed by mg3d_destroy: 52 GB at 1025^3 fp64, on top of the 38 GB of the hierarchy.
+ * The loop runs on the device like mg3d_solve's (DESIGN.md section 6b).  mg3b_pcg is the same on a box grid. */
+int mg3d_pcg(mg3d_t* mg, int level, int v1, int v2, double rtol, double atol, int max_iters,
+             int* iters_out, int* converged_out, double* history);
 
 /* reference-facing calls on HOST arrays (NOCUDA signatures, N3/MultiGrid3D.h:16-27): upload, run, download */
 int mg3d_restrict_host(mg3d_t* mg, const void* fine, const int fsize_xyz[3], void* coarse, const int csize_xyz[3]);
@@ -204,6 +221,8 @@ int mg3b_vcycle(mg3b_t* mg, int level, int v1, int v2);              /* VCycle *
 int mg3b_fmg(mg3b_t* mg, int level, int v0, int v1, int v2);         /* FullMultiGridVCycle */
 int mg3b_solve(mg3b_t* mg, int level, int v1, int v2, double rtol, double atol, int max_cycles,
                int* cycles_out, int* converged_out, double* history); /* as mg3d_solve */
+int mg3b_pcg(mg3b_t* mg, int level, int v1, int v2, double rtol, double atol, int max_iters,
+             int* iters_out, int* converged_out, double* history);   /* as mg3d_pcg */
 int mg3b_vcycle_host(mg3b_t* mg, void* v_host, const void* f_host, int v1, int v2, int cycles);
 /* the operators on caller-owned HOST arrays (N3/MultiGrid3D.h:16-27 with three different sizes) */
 int mg3b_restrict_host(mg3b_t* mg, const void* fine, const int fsize_xyz[3], void* coarse, const int csize_xyz[3]);

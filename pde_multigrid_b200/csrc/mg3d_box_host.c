@@ -38,6 +38,7 @@ struct mg3b_s {
     void* staging;     /* one dense field of the finest level: host <-> device copies pass through it (repack) */
     double* d_scratch; /* 2 * MG3B_NPARTS partials + 2 outputs */
     double* d_tables;  /* sin tables of InitF: nx + ny + nz doubles of the finest level */
+    mg_pcg_vecs* pcg;  /* per level, allocated by the first mg3b_pcg of the level */
 };
 
 static size_t level_count(const mg_level3b* L) { return (size_t)L->n[0] * (size_t)L->n[1] * (size_t)L->n[2]; }
@@ -100,6 +101,8 @@ int mg3b_destroy(mg3b_t* mg)
     if (mg->staging) cudaFree(mg->staging);
     if (mg->d_scratch) cudaFree(mg->d_scratch);
     if (mg->d_tables) cudaFree(mg->d_tables);
+    for (int l = 0; mg->pcg && l < mg->core.nlevels; l++) mg_pcg_vecs_free(&mg->pcg[l]);
+    free(mg->pcg);
     free(mg->lv);
     free(mg);
     return MG_OK;
@@ -390,6 +393,47 @@ int mg3b_solve(mg3b_t* mg, int level, int v1, int v2, double rtol, double atol, 
     const int key[MG_GRAPH_KEY] = {level, v1, v2};
     return mg_solve_run(&mg->core.graphs, mg_graphs_on(&mg->core.graphs, 0, 2LL * (v1 + v2) * (mg->core.nlevels - level)) ? key : NULL, &ops,
                         rtol, atol, max_cycles, cycles_out, converged_out, history);
+}
+
+/* multigrid-preconditioned conjugate gradients (mg_host_common.c runs the loop, mg3d_cg.cu has the vector passes) */
+static void* p3b_v(mg_cycle_ctx* x) { return ((mg3b_t*)x->h)->lv[x->level].v; }
+static int p3b_vcycle(mg_cycle_ctx* x) { return vcycle_rec(x->h, x->level, x->v1, x->v2); }
+static int p3b_norm0(mg_cycle_ctx* x) { return residual_norm_enqueue(x->h, x->level); }
+static int p3b_zero_v(mg_cycle_ctx* x)
+{
+    mg3b_t* mg = x->h;
+    mg_level3b* L = &mg->lv[x->level];
+    MG_LAUNCH(mg->core.launches, mgk3b_set(mg->core.stream, mg->core.dtype, L->v, L->g, 0.0, 1));
+    return MG_OK;
+}
+
+int mg3b_pcg(mg3b_t* mg, int level, int v1, int v2, double rtol, double atol, int max_iters, int* iters_out, int* converged_out,
+             double* history)
+{
+    int st = mg_solve_check_args(MG_CORE(mg), level, rtol, atol, max_iters, v1, v2);
+    if (st) return st;
+    if (mg->mode != MG_CORRECTED) return mg_fail(MG_ERR_STATE, "pcg needs MG_CORRECTED: the MG_REF_COMPAT residual is not a symmetric operator");
+    if (!mg->pcg && !(mg->pcg = (mg_pcg_vecs*)calloc((size_t)mg->core.nlevels, sizeof *mg->pcg)))
+        return mg_fail(MG_ERR_NOMEM, "host allocation failed");
+    mg_level3b* L = &mg->lv[level];
+    if ((st = mg_pcg_vecs_alloc(&mg->pcg[level], field_bytes(L, mg->core.dtype), mg->core.stream))) return st;
+    mg_pcg_ctx pc;
+    memset(&pc, 0, sizeof pc);
+    pc.cx.h = mg; pc.cx.level = level; pc.cx.v1 = v1; pc.cx.v2 = v2;
+    pc.P = &mg->pcg[level];
+    pc.dtype = mg->core.dtype;
+    pc.stream = mg->core.stream;
+    pc.launches = &mg->core.launches;
+    pc.g.nx = L->g.nx; pc.g.ny = L->g.ny; pc.g.nz = L->g.nz;
+    pc.g.hp = L->g.hp; pc.g.plane = L->g.plane; pc.g.cstride = L->g.cstride;
+    pc.g.z0 = 0; pc.g.nzl = L->g.nz;
+    pc.c = L->c;
+    pc.f = L->f;
+    pc.out2 = mg->d_scratch + 2 * MG3B_NPARTS;
+    pc.v = p3b_v; pc.zero_v = p3b_zero_v; pc.vcycle = p3b_vcycle; pc.norm0 = p3b_norm0;
+    const int key[MG_GRAPH_KEY] = {level, v1, v2, 0, 0, 0, 0, MG_GRAPH_PCG};
+    return mg_pcg_run(&pc, &mg->core.graphs, mg_graphs_on(&mg->core.graphs, 0, 2LL * (v1 + v2) * (mg->core.nlevels - level)) ? key : NULL, rtol,
+                      atol, max_iters, iters_out, converged_out, history);
 }
 
 /* FullMultiGridVCycle, N3/MultiGrid3D.cpp:569-585 */

@@ -114,6 +114,7 @@ struct mg3d_s {
     unsigned int* d_flag; /* {exactness flag of the pipelined smoother, completion counter of its fallback} */
     int no_tail;         /* MG_B200_NO_TAIL: coarse levels as separate launches */
     int full_correction; /* MG_B200_FULL_CORRECTION: correct both colours after prolongation inside a cycle */
+    mg_pcg_vecs* pcg;    /* per level, allocated by the first mg3d_pcg of the level */
 };
 
 /* h = range/(real)(n-1) (N3/Grid3D.cpp:31-45) and the products of N3/MultiGrid3D.cpp:498-500,532,
@@ -743,6 +744,8 @@ int mg3d_destroy(mg3d_t* mg)
     if (mg->staging) cudaFree(mg->staging);
     for (int l = 0; mg->lv && l < mg->core.nlevels; l++)
         if (mg->lv[l].jscratch) cudaFree(mg->lv[l].jscratch);
+    for (int l = 0; mg->pcg && l < mg->core.nlevels; l++) mg_pcg_vecs_free(&mg->pcg[l]);
+    free(mg->pcg);
     free(mg->lv);
     free(mg);
     return MG_OK;
@@ -1550,6 +1553,54 @@ int mg3d_solve(mg3d_t* mg, int level, int v1, int v2, double rtol, double atol, 
        norm, so every rank stops after the same cycle. */
     const int device = mg->nranks == 1 && graphs_on(mg, level, v1, v2);
     st = mg_solve_run(&mg->core.graphs, device ? key : NULL, &ops, rtol, atol, max_cycles, cycles_out, converged_out, history);
+    return st ? st : halo_error_check(mg);
+}
+
+/* ---- multigrid-preconditioned conjugate gradients (mg_host_common.c runs the loop, mg3d_cg.cu has the vector passes) ---- */
+
+static void* p3_v(mg_cycle_ctx* x) { return ((mg3d_t*)x->h)->lv[x->level].v; }
+static int p3_vcycle(mg_cycle_ctx* x) { return vcycle_rec(x->h, x->level, x->v1, x->v2); }
+static int p3_norm0(mg_cycle_ctx* x) { return residual_norm_enqueue(x->h, x->level); }
+/* setToValue(v, 0, true) on the buffer the V-cycle starts from */
+static int p3_zero_v(mg_cycle_ctx* x)
+{
+    mg3d_t* mg = x->h;
+    mg_level3d* L = &mg->lv[x->level];
+    MG_LAUNCH(mg->core.launches, mgk3d_set(mg->core.stream, mg->core.dtype, L->v, L->g, 0.0, 1, 0, L->g.nzl));
+    L->vg_valid = L->vg_deep = 1;
+    return MG_OK;
+}
+
+int mg3d_pcg(mg3d_t* mg, int level, int v1, int v2, double rtol, double atol, int max_iters, int* iters_out, int* converged_out,
+             double* history)
+{
+    int st = mg_solve_check_args(MG_CORE(mg), level, rtol, atol, max_iters, v1, v2);
+    if (st) return st;
+    if (mg->mode != MG_CORRECTED) return mg_fail(MG_ERR_STATE, "pcg needs MG_CORRECTED: the MG_REF_COMPAT residual is not a symmetric operator");
+    if (mg->nranks > 1) return mg_fail(MG_ERR_STATE, "pcg runs on one GPU (distributed handle of %d ranks)", mg->nranks);
+    if (!mg->pcg && !(mg->pcg = (mg_pcg_vecs*)calloc((size_t)mg->core.nlevels, sizeof *mg->pcg)))
+        return mg_fail(MG_ERR_NOMEM, "host allocation failed");
+    mg_level3d* L = &mg->lv[level];
+    if ((st = mg_pcg_vecs_alloc(&mg->pcg[level], field_bytes(L, mg->core.dtype), mg->core.stream))) return st;
+    mg_pcg_ctx pc;
+    memset(&pc, 0, sizeof pc);
+    pc.cx.h = mg; pc.cx.level = level; pc.cx.v1 = v1; pc.cx.v2 = v2;
+    pc.P = &mg->pcg[level];
+    pc.dtype = mg->core.dtype;
+    pc.stream = mg->core.stream;
+    pc.launches = &mg->core.launches;
+    pc.g.nx = pc.g.ny = pc.g.nz = L->g.n;
+    pc.g.hp = L->g.hp; pc.g.plane = L->g.plane; pc.g.cstride = L->g.cstride;
+    pc.g.z0 = L->g.z0; pc.g.nzl = L->g.nzl;
+    pc.c = L->c;
+    pc.f = L->f;
+    pc.out2 = norm_out2(mg);
+    pc.v = p3_v; pc.zero_v = p3_zero_v; pc.vcycle = p3_vcycle; pc.norm0 = p3_norm0;
+    pc.save = c3_save; pc.load = c3_load;
+    int key[MG_GRAPH_KEY];
+    graph_key(&pc.cx, 0, key);
+    key[MG_GRAPH_KEY_KIND] = MG_GRAPH_PCG;
+    st = mg_pcg_run(&pc, &mg->core.graphs, graphs_on(mg, level, v1, v2) ? key : NULL, rtol, atol, max_iters, iters_out, converged_out, history);
     return st ? st : halo_error_check(mg);
 }
 

@@ -300,10 +300,12 @@ static int launch_check(const mg_cycle_ops* ops, mg_graphs* gr, int nhandles, cu
 }
 
 /* host-driven: the family's own cycle call, the norm pass and the check kernel, one read-back per cycle */
+static int first_norm(const mg_cycle_ops* ops) { return ops->first ? ops->first(ops->ctx) : ops->norm(ops->ctx); }
+
 static int solve_host(const mg_cycle_ops* ops, mg_graphs* gr)
 {
     int st;
-    if ((st = ops->norm(ops->ctx))) return st;
+    if ((st = first_norm(ops))) return st;
     if ((st = launch_check(ops, gr, 0, 0, 0))) return st;
     for (;;) {
         if ((st = read_par(gr, ops->stream))) return st;
@@ -370,7 +372,7 @@ static int solve_build(const mg_cycle_ops* ops, mg_graph_slot* slot, mg_graphs* 
     SOLVE_TRY(cudaGraphConditionalHandleCreate(&hw, g, 0, cudaGraphCondAssignDefault));
 
     SOLVE_TRY(cudaStreamBeginCaptureToGraph(s, g, NULL, NULL, 0, cudaStreamCaptureModeThreadLocal));
-    SOLVE_STEP(ops->norm(ops->ctx));
+    SOLVE_STEP(first_norm(ops));
     SOLVE_STEP(launch_check(ops, gr, 1, hw, 0));
     SOLVE_STEP(add_conditional(s, hw, cudaGraphCondTypeWhile, &body));
     SOLVE_STEP(capture_segment_end(s));
@@ -445,6 +447,109 @@ int mg_solve_run(mg_graphs* gr, const int key[MG_GRAPH_KEY], const mg_cycle_ops*
     for (int c = 1; c <= cycles; c++) *ops->launches += slot->launches[slot->two && c % 2 == 0 ? 2 : 1];
     if (ops->load) ops->load(ops->ctx, cycles == 0 ? slot->snap[0] : (slot->two && cycles % 2 == 0) ? slot->snap[2] : slot->snap[1]);
     return solver_finish(gr, s, cycles_out, converged_out, history);
+}
+
+/* ---- multigrid-preconditioned conjugate gradients ------------------------------------------------ */
+
+int mg_pcg_vecs_alloc(mg_pcg_vecs* P, size_t field_bytes, cudaStream_t s)
+{
+    if (P->b) return MG_OK;
+    void** f[6] = {&P->b, &P->x[0], &P->x[1], &P->p[0], &P->p[1], &P->d};
+    cudaError_t e = cudaSuccess;
+    for (int i = 0; i < 6 && e == cudaSuccess; i++) e = cudaMalloc(f[i], field_bytes);
+    if (e == cudaSuccess) e = cudaMalloc((void**)&P->parts, (MGK_PCG_PARTS + MGK_PCG_SCALARS) * sizeof(double));
+    /* the row padding is never read for a result, but it is copied into v at the end: keep it defined */
+    for (int i = 0; i < 6 && e == cudaSuccess; i++) e = cudaMemsetAsync(*f[i], 0, field_bytes, s);
+    if (e == cudaSuccess) e = cudaMemsetAsync(P->parts, 0, (MGK_PCG_PARTS + MGK_PCG_SCALARS) * sizeof(double), s);
+    if (e == cudaSuccess) {
+        P->bytes = field_bytes;
+        return MG_OK;
+    }
+    cudaGetLastError();
+    mg_pcg_vecs_free(P);
+    return mg_fail(MG_ERR_NOMEM, "PCG vectors (6 x %zu bytes): %s", field_bytes, cudaGetErrorString(e));
+}
+
+void mg_pcg_vecs_free(mg_pcg_vecs* P)
+{
+    void* f[7] = {P->b, P->x[0], P->x[1], P->p[0], P->p[1], P->d, P->parts};
+    for (int i = 0; i < 7; i++)
+        if (f[i]) cudaFree(f[i]);
+    memset(P, 0, sizeof *P);
+}
+
+static double* pcg_sc(const mg_pcg_ctx* pc) { return pc->P->parts + MGK_PCG_PARTS; }
+
+/* norm(r_0) with the family's own pass (the same bits as mg?d_residual_norm), then b <- f, x <- v, r_0 = b - Laplacian x into f */
+static int pcg_first(void* c)
+{
+    mg_pcg_ctx* pc = (mg_pcg_ctx*)c;
+    mg_pcg_vecs* P = pc->P;
+    int st = pc->norm0(&pc->cx);
+    if (st) return st;
+    pc->par = 0;
+    MG_CUDA(cudaMemcpyAsync(P->b, pc->f, P->bytes, cudaMemcpyDeviceToDevice, pc->stream));
+    MG_CUDA(cudaMemcpyAsync(P->x[0], pc->v(&pc->cx), P->bytes, cudaMemcpyDeviceToDevice, pc->stream));
+    MG_CUDA(cudaMemsetAsync(P->p[0], 0, P->bytes, pc->stream)); /* beta = 0 multiplies it on the first iteration */
+    MG_CUDA(cudaMemsetAsync(P->d, 0, P->bytes, pc->stream));
+    MG_LAUNCH(*pc->launches, mgk3cg_residual(pc->stream, pc->dtype, P->x[0], P->b, pc->f, pc->g, pc->c, pcg_sc(pc), 0, pc->g.nzl));
+    return MG_OK;
+}
+
+/* one iteration: z = VCycle(0; r) in v, beta, p, alpha, x, r, the norm partials of the new r */
+static int pcg_step(void* c)
+{
+    mg_pcg_ctx* pc = (mg_pcg_ctx*)c;
+    mg_pcg_vecs* P = pc->P;
+    const int a = pc->par, n = a ^ 1;
+    double *part = P->parts, *sc = pcg_sc(pc);
+    int st;
+    if ((st = pc->zero_v(&pc->cx)) || (st = pc->vcycle(&pc->cx))) return st;
+    const void* z = pc->v(&pc->cx);
+    MG_LAUNCH(*pc->launches, mgk3cg_dots(pc->stream, pc->dtype, z, pc->f, P->d, pc->g, 0, pc->g.nzl, part, sc));
+    MG_LAUNCH(*pc->launches, mgk3cg_dir(pc->stream, pc->dtype, z, P->p[a], P->p[n], pc->g, pc->c, 0, pc->g.nzl, part + MGK_PCG_DIR_PARTS, sc));
+    MG_LAUNCH(*pc->launches, mgk3cg_update(pc->stream, pc->dtype, P->x[a], P->p[n], P->b, pc->f, P->x[n], P->d, pc->g, pc->c, sc, 0, pc->g.nzl,
+                                           part + MGK_PCG_UPD_PARTS));
+    pc->par = n;
+    return MG_OK;
+}
+
+static int pcg_norm(void* c)
+{
+    mg_pcg_ctx* pc = (mg_pcg_ctx*)c;
+    MG_LAUNCH(*pc->launches, mgk_norm_final(pc->stream, pc->P->parts + MGK_PCG_UPD_PARTS, MGK_PCG_BLOCKS, pc->out2));
+    return MG_OK;
+}
+
+static void pcg_save(void* c, unsigned out[2])
+{
+    mg_pcg_ctx* pc = (mg_pcg_ctx*)c;
+    out[0] = out[1] = 0;
+    if (pc->save) pc->save(&pc->cx, out);
+    out[0] = (out[0] & 0x7fffffffu) | ((unsigned)pc->par << 31);
+}
+
+static void pcg_load(void* c, const unsigned in[2])
+{
+    mg_pcg_ctx* pc = (mg_pcg_ctx*)c;
+    if (pc->load) {
+        const unsigned fam[2] = {in[0] & 0x7fffffffu, in[1]};
+        pc->load(&pc->cx, fam);
+    }
+    pc->par = (int)(in[0] >> 31);
+}
+
+int mg_pcg_run(mg_pcg_ctx* pc, mg_graphs* gr, const int key[MG_GRAPH_KEY], double rtol, double atol, int max_iters, int* iters_out,
+               int* converged_out, double* history)
+{
+    const mg_cycle_ops ops = {pc, pc->stream, pc->launches, NULL, pcg_step, pcg_step, pcg_norm, pc->out2, pcg_save, pcg_load, pcg_first};
+    int st = mg_solve_run(gr, key, &ops, rtol, atol, max_iters, iters_out, converged_out, history);
+    if (st) return st;
+    /* v of the level (the buffer the last V-cycle ended on) <- x, f <- b: the caller's f bit for bit */
+    MG_CUDA(cudaMemcpyAsync(pc->v(&pc->cx), pc->P->x[pc->par], pc->P->bytes, cudaMemcpyDeviceToDevice, pc->stream));
+    MG_CUDA(cudaMemcpyAsync(pc->f, pc->P->b, pc->P->bytes, cudaMemcpyDeviceToDevice, pc->stream));
+    MG_CUDA(cudaStreamSynchronize(pc->stream));
+    return MG_OK;
 }
 
 int mg_require_device(void)

@@ -69,8 +69,10 @@ int mg_require_device(void); /* MG_OK, or MG_ERR_CUDA with a message: there is n
 /* a cycle estimated to make more launches than this runs eagerly: it is not dominated by launch gaps, and its graph
    would be large to capture and keep */
 #define MG_GRAPH_MAX_LAUNCHES 4096
-#define MG_GRAPH_KEY 7     /* (level, v1, v2, smoother, arith, buffer bits, ghost bits); the families use a prefix */
+#define MG_GRAPH_KEY 8     /* (level, v1, v2, smoother, arith, buffer bits, ghost bits, kind); the families use a prefix */
 #define MG_GRAPH_KEY_SMOOTHER 3
+#define MG_GRAPH_KEY_KIND 7 /* 0: cycles and solves, MG_GRAPH_PCG: *_pcg graphs */
+#define MG_GRAPH_PCG 1
 #define MG_CYCLE_SLOTS 16
 #define MG_SOLVE_SLOTS 8
 
@@ -111,6 +113,8 @@ typedef struct {
        [0] = which buffer every level works on, [1] = further bookkeeping */
     void (*save)(void* ctx, unsigned out[2]);
     void (*load)(void* ctx, const unsigned in[2]);
+    /* NULL, or what runs instead of norm() for r_0: its norm into out2, then whatever the loop needs set up (the PCG prologue) */
+    int (*first)(void* ctx);
 } mg_cycle_ops;
 
 void mg_graphs_init(mg_graphs* gr); /* reads MG_B200_NO_GRAPH */
@@ -132,6 +136,45 @@ typedef struct {
 /* the whole solve: device-driven when key != NULL, the key is warm and its graph builds; host-driven otherwise */
 int mg_solve_run(mg_graphs* gr, const int key[MG_GRAPH_KEY], const mg_cycle_ops* ops, double rtol, double atol,
                  int max_cycles, int* cycles_out, int* converged_out, double* history);
+
+/* ---- multigrid-preconditioned conjugate gradients (mg3d_pcg, mg3b_pcg; DESIGN.md §6b) ----
+   The loop is mg_solve_run's: ops.first = norm(r_0) + prologue, ops.cycle = one PCG iteration (its V-cycle included),
+   ops.norm = the norm finaliser of the iteration's update pass.  x and p ping-pong between two buffers, so the iteration's
+   parity is part of the state ops.save / ops.load carry (bit 31 of [0]) and a device loop always has the two-iteration body. */
+typedef struct {
+    void* b;          /* the caller's f of the level, put back at the end */
+    void* x[2];       /* the iterate */
+    void* p[2];       /* the search direction */
+    void* d;          /* r_k - r_{k-1} */
+    double* parts;    /* MGK_PCG_PARTS partials of the three passes (mg_launch.h), then MGK_PCG_SCALARS scalars */
+    size_t bytes;     /* of one field */
+} mg_pcg_vecs;
+
+typedef struct {
+    mg_cycle_ctx cx;              /* the family's cycle context: handle, level, sweeps */
+    mg_pcg_vecs* P;
+    int par;                      /* which of x[], p[] holds the current iterate and direction */
+    int dtype;
+    cudaStream_t stream;
+    long long* launches;
+    mg_geom3cg g;
+    mg_coef3d c;
+    void* f;                      /* the level's f */
+    double* out2;                 /* where the family's norm pass leaves {sum of squares, max} */
+    void* (*v)(mg_cycle_ctx* cx); /* the level's current v buffer */
+    int (*zero_v)(mg_cycle_ctx* cx);
+    int (*vcycle)(mg_cycle_ctx* cx);
+    int (*norm0)(mg_cycle_ctx* cx); /* the family's residual-norm pass (mg?d_residual_norm without the read-back) */
+    void (*save)(void* cx, unsigned out[2]); /* NULL, or the family's host-side buffer state */
+    void (*load)(void* cx, const unsigned in[2]);
+} mg_pcg_ctx;
+
+/* allocates the vectors of one level on first use (MG_ERR_NOMEM, nothing allocated, when that fails) */
+int mg_pcg_vecs_alloc(mg_pcg_vecs* P, size_t field_bytes, cudaStream_t s);
+void mg_pcg_vecs_free(mg_pcg_vecs* P);
+/* the whole PCG: the loop through mg_solve_run (device-driven when key != NULL), then v <- x, f <- b */
+int mg_pcg_run(mg_pcg_ctx* pc, mg_graphs* gr, const int key[MG_GRAPH_KEY], double rtol, double atol, int max_iters, int* iters_out,
+               int* converged_out, double* history);
 
 /* ---- the handle core ----
    Every family's handle (mg1d_s, mg2d_s, mg3b_s, mg3d_s) has an mg_core named `core`.  A public call passes

@@ -197,6 +197,43 @@ typedef struct {
 int mgk_solve_check(cudaStream_t s, const double* out2, mg_solve_par* par, int nhandles, cudaGraphConditionalHandle h0,
                     cudaGraphConditionalHandle h1);
 
+/* ---- multigrid-preconditioned conjugate gradients (mg3d_cg.cu), cubic and box levels alike ---- */
+/* a colour-split level of either 3D engine: element (x,y,zl) of colour c = (x+y+z0+zl)&1 at base[c*cstride + zl*plane + y*hp +
+   (x>>1)]; the grid is nx*ny*nz points, local planes zl = 0..nzl-1 are the global planes z0.. (one GPU: z0 = 0, nzl = nz) */
+typedef struct {
+    int nx, ny, nz, hp;
+    long long plane, cstride;
+    int z0, nzl;
+} mg_geom3cg;
+
+/* the device scalar block of one PCG (doubles) */
+#define MGK_PCG_RHO 0   /* z.r of the current iteration (after mgk3cg_dots: the previous one's is gone) */
+#define MGK_PCG_BETA 1
+#define MGK_PCG_ALPHA 2
+#define MGK_PCG_FIRST 3 /* nonzero: the next mgk3cg_dots starts the recurrence (beta = 0) */
+#define MGK_PCG_PI 4
+#define MGK_PCG_SCALARS 8
+#define MGK_PCG_BLOCKS 296 /* the fixed grid of the passes (two blocks per SM of a B200) */
+/* partials of one iteration: the dots and the direction pass write two double-double sums per block (4*MGK_PCG_BLOCKS
+   doubles each), the update pass the {sum r^2, max|r|} pair of mgk_norm_final (2*MGK_PCG_BLOCKS) */
+#define MGK_PCG_DIR_PARTS (4 * MGK_PCG_BLOCKS)
+#define MGK_PCG_UPD_PARTS (8 * MGK_PCG_BLOCKS)
+#define MGK_PCG_PARTS (10 * MGK_PCG_BLOCKS)
+/* every launcher covers local planes [zl_lo, zl_hi) (on one GPU: all of them) */
+/* rho = z.r, sigma = z.d -> beta (two launches) */
+int mgk3cg_dots(cudaStream_t s, int dtype, const void* z, const void* r, const void* d, mg_geom3cg g, int zl_lo, int zl_hi,
+                double* part, double* sc);
+/* p_out = z + beta*p_in, pi = p_out.(Laplacian p_out) -> alpha (two launches) */
+int mgk3cg_dir(cudaStream_t s, int dtype, const void* z, const void* p_in, void* p_out, mg_geom3cg g, mg_coef3d c, int zl_lo,
+               int zl_hi, double* part, double* sc);
+/* x_out = x_in + alpha*p, r = b - Laplacian x_out (in place over the old r), d = new r - old r; {sum r^2, max|r|} partials
+   for mgk_norm_final */
+int mgk3cg_update(cudaStream_t s, int dtype, const void* x_in, const void* p, const void* b, void* r, void* x_out, void* d,
+                  mg_geom3cg g, mg_coef3d c, const double* sc, int zl_lo, int zl_hi, double* part);
+/* r = b - Laplacian x (zero on the Dirichlet points), and the scalar block marked for a first iteration */
+int mgk3cg_residual(cudaStream_t s, int dtype, const void* x, const void* b, void* r, mg_geom3cg g, mg_coef3d c, double* sc,
+                    int zl_lo, int zl_hi);
+
 /* ---- 2D (pitched: element (x,y) at base[x + y*pitch]) ---- */
 typedef struct {
     int n;

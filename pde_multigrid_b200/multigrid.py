@@ -205,7 +205,24 @@ class _MultiGridBase:
         return v_host
 
 
-class MultiGrid3D(_MultiGridBase):
+class _PCGMixin:
+    """pcg() of the 3D engines.  CG needs a symmetric operator: the 2D Lyapunov operator and the first-order 1D
+    equation are not, so the 2D and 1D classes do not have it."""
+
+    def pcg(self, v1=2, v2=2, rtol=1e-8, atol=0.0, max_iters=100, level=0):
+        """Conjugate gradients preconditioned by one VCycle(level, v1, v2) per iteration (mg3d_pcg / mg3b_pcg) on the
+        MG_CORRECTED operator, from the current v, until the true residual meets ||r_k||_2 <= max(atol, rtol * ||r_0||_2)
+        or max_iters iterations have run.  Returns a SolveResult whose `cycles` counts iterations (one V-cycle each).
+        v of `level` holds the iterate afterwards, f of `level` is unchanged."""
+        hist = np.empty((max(int(max_iters), 0) + 1, 2), dtype=np.float64)
+        iters, converged = ctypes.c_int(), ctypes.c_int()
+        self._call("pcg", ctypes.c_int(level), ctypes.c_int(v1), ctypes.c_int(v2), ctypes.c_double(rtol),
+                   ctypes.c_double(atol), ctypes.c_int(max_iters), ctypes.byref(iters), ctypes.byref(converged),
+                   hist.ctypes.data_as(ctypes.c_void_p))
+        return SolveResult(iters.value, bool(converged.value), hist[:iters.value + 1].copy())
+
+
+class MultiGrid3D(_PCGMixin, _MultiGridBase):
     """MultiGrid3D(finestGridSizeXYZ, range) -- N3/MultiGrid3D.h:12."""
     dim = 3
     prefix = "mg3d"
@@ -276,7 +293,7 @@ class MultiGrid3D(_MultiGridBase):
         return dict(zip(("dist", "z0", "nzl", "own_lo", "own_hi"), list(out)))
 
 
-class MultiGrid3DBox(_MultiGridBase):
+class MultiGrid3DBox(_PCGMixin, _MultiGridBase):
     """MultiGrid3D(finestGridSizeXYZ, range) with sizeX != sizeY != sizeZ (mg3b_* of the C ABI): the grids the reference
     asserts away at N3/Grid3D.cpp:10-11.  Host arrays have numpy shape (sizeZ, sizeY, sizeX) -- the dense x-fastest layout."""
     dim = 3
