@@ -80,10 +80,10 @@ static void box_coefs(int dtype, const int n[3], const double* range, double h[3
         c->ihx2 = 1.0 / hx2; c->ihy2 = 1.0 / hy2; c->ihz2 = 1.0 / hz2;
     }
     /* three different mesh widths: the smoother's divisor is not of the 6*2^e form, IEEE division there; the residual's x / h^2
-       becomes the exact x * (1/h^2) when every h^2 is a power of two (mg_exact.cuh; MG_B200_IEEE_DIV switches it off) */
+       becomes the exact x * (1/h^2) when every h^2 is a power of two (mg_exact.cuh) */
     int e;
     c->fast_den = 0;
-    c->fast_h = frexp(c->hx2, &e) == 0.5 && frexp(c->hy2, &e) == 0.5 && frexp(c->hz2, &e) == 0.5 && !getenv("MG_B200_IEEE_DIV");
+    c->fast_h = frexp(c->hx2, &e) == 0.5 && frexp(c->hy2, &e) == 0.5 && frexp(c->hz2, &e) == 0.5;
 }
 
 static int pow2_plus_1(int n)

@@ -80,7 +80,7 @@ typedef struct {
     char** all_arena;
     unsigned int** all_flags;
     size_t* all_off;              /* byte offset of field fi of level l inside rank p's arena: [(p*nlevels + l)*3 + fi] */
-    int gather_p2p;               /* 1: gather_level stores directly into the peers (MG_B200_GATHER=nccl switches it off) */
+    int gather_p2p;               /* 1: gather_level stores directly into the peers (at most MG_GATHER_MAX_PEERS of them) */
 } mg_p2p;
 
 /* core.graphs holds the V-cycle graphs: the cycle is ~100 dependent launches, most of them tiny (coarse levels, halo
@@ -93,7 +93,6 @@ struct mg3d_s {
     double range[6];
     cudaStream_t cstream;       /* side stream: halo exchange of the boundary planes overlapping the interior sweep */
     cudaEvent_t ev_fork, ev_join;
-    int overlap;
     mg_comm* comm;
     mg_p2p p2p;
     mg_level3d* lv;
@@ -108,11 +107,7 @@ struct mg3d_s {
     long long halo_bytes; /* bytes sent by this rank in halo exchanges / gathers */
     double omega;   /* weight of MG_SMOOTHER_JACOBI */
     int arith;           /* MG_ARITH_EXACT / MG_ARITH_FAST */
-    int no_pipe;         /* MG_B200_NO_PIPE: MG_SMOOTHER_AUTO without temporal blocking (the round-1 default) */
-    int no_deep_merge;   /* MG_B200_NO_DEEP_MERGE: the post-smoothing pass fetches its colour-1 ghosts itself (one more exchange) */
-    int no_corr_fuse;    /* MG_B200_NO_CORR_FUSE: prolongation + correction as a kernel of their own even where the pass could take them */
     unsigned int* d_flag; /* {exactness flag of the pipelined smoother, completion counter of its fallback} */
-    int no_tail;         /* MG_B200_NO_TAIL: coarse levels as separate launches */
     int full_correction; /* MG_B200_FULL_CORRECTION: correct both colours after prolongation inside a cycle */
     mg_pcg_vecs* pcg;    /* per level, allocated by the first mg3d_pcg of the level */
 };
@@ -152,7 +147,6 @@ static void level_coefs(int dtype, int n, const double* range, double h[3], mg_c
     c->fast_h = frexp(c->hx2, &e) == 0.5 && frexp(c->hy2, &e) == 0.5 && frexp(c->hz2, &e) == 0.5;
     /* ... and its reciprocal must be finite: a subnormal den (float h <= 2^-33, double h <= 2^-257) has 1/den = inf */
     c->fast_den = c->fast_h && frexp(c->den, &e) == 0.75 && isfinite(c->rden);
-    if (getenv("MG_B200_IEEE_DIV")) c->fast_h = c->fast_den = 0;
 }
 
 static void set_geom(mg_geom3d* g, int n, int dtype, int z0, int nzl)
@@ -196,7 +190,7 @@ static size_t field_bytes(const mg_level3d* L, int dtype)
     return mg_align256(2 * (size_t)L->g.cstride * mg_esize(dtype));
 }
 
-static int level_uses_tma(int n) { return (n - 1) / 2 >= MGK3D_TMA_IT && !getenv("MG_B200_NO_TMA"); }
+static int level_uses_tma(int n) { return (n - 1) / 2 >= MGK3D_TMA_IT; }
 
 /* fields a level keeps in the arena: v, f and, where the temporally blocked smoothers can run (the large levels), a second v */
 static int level_fields_for(int n, int dist) { (void)dist; return level_uses_tma(n) ? 3 : 2; }
@@ -430,9 +424,8 @@ static int gather_level(mg3d_t* mg, int level, void* field, int top_mode)
  * CUDA IPC mapping of the z-neighbours' arenas and flag words (enables exchange_p2p).  Handles travel
  * through an NCCL all-gather.  If IPC / peer access is not available the NCCL send/recv path stays.
  * ---------------------------------------------------------------------------------------------- */
-static int p2p_setup(mg3d_t* mg, size_t arena_bytes)
+static int p2p_setup(mg3d_t* mg)
 {
-    (void)arena_bytes;
     mg_p2p* q = &mg->p2p;
     const int r = mg->rank, P = mg->nranks;
     /* what the neighbours' arenas look like: replay the allocation arithmetic for rank-1 and rank+1 */
@@ -530,7 +523,7 @@ static int p2p_setup(mg3d_t* mg, size_t arena_bytes)
     MG_CUDA(cudaMemcpyAsync(h2, d2, sizeof h2, cudaMemcpyDeviceToHost, mg->core.stream));
     MG_CUDA(cudaStreamSynchronize(mg->core.stream));
     q->enabled = h2[0] == 0.0;
-    q->gather_p2p = q->enabled && P - 1 <= MG_GATHER_MAX_PEERS && !(getenv("MG_B200_GATHER") && !strcmp(getenv("MG_B200_GATHER"), "nccl"));
+    q->gather_p2p = q->enabled && P - 1 <= MG_GATHER_MAX_PEERS;
     return MG_OK;
 }
 
@@ -598,10 +591,6 @@ static int create_common(mg3d_t** out, const int sz[3], const double range[6], i
     mg->smoother = MG_SMOOTHER_AUTO;
     mg->sweeps_per_pass = 1;
     mg->omega = 6.0 / 7.0;
-    mg->no_tail = getenv("MG_B200_NO_TAIL") != NULL;
-    mg->no_pipe = getenv("MG_B200_NO_PIPE") != NULL;
-    mg->no_corr_fuse = getenv("MG_B200_NO_CORR_FUSE") != NULL;
-    mg->no_deep_merge = getenv("MG_B200_NO_DEEP_MERGE") != NULL;
     mg->arith = MG_ARITH_EXACT;
     mg->full_correction = getenv("MG_B200_FULL_CORRECTION") != NULL;
     memcpy(mg->range, range, sizeof mg->range);
@@ -655,9 +644,8 @@ static int create_common(mg3d_t** out, const int sz[3], const double range[6], i
             mg3d_destroy(mg);
             return code;
         }
-        mg->overlap = getenv("MG_B200_NO_OVERLAP") ? 0 : 1;
         st = mg_comm_create(&mg->comm, rank, nranks, uid);
-        if (!st && !(getenv("MG_B200_HALO") && !strcmp(getenv("MG_B200_HALO"), "nccl"))) st = p2p_setup(mg, total);
+        if (!st) st = p2p_setup(mg);
         if (st) { mg3d_destroy(mg); return st; }
     }
     /* TMA tensor maps for the levels large enough to fill the z-marching tiles */
@@ -993,7 +981,7 @@ static int relax_launch(mg3d_t* mg, mg_level3d* L, int colour, int lo, int hi, i
    run on the side stream while the interior planes are swept; every half-sweep ends with a join */
 static int level_takes_pipe(const mg3d_t* mg, const mg_level3d* L)
 {
-    return (mg->smoother == MG_SMOOTHER_PIPE || (mg->smoother == MG_SMOOTHER_AUTO && !mg->no_pipe)) && L->has_tma && L->vbuf[1] &&
+    return (mg->smoother == MG_SMOOTHER_PIPE || mg->smoother == MG_SMOOTHER_AUTO) && L->has_tma && L->vbuf[1] &&
            L->c.fast_den && L->iso && mgk3d_pipe_exact_range(mg->core.dtype, L->c.hx2) && (!L->dist || L->own_hi - L->own_lo >= 8);
 }
 
@@ -1003,7 +991,7 @@ static int relax_overlaps(const mg3d_t* mg, int level)
     int lo, hi;
     interior_range(L, &lo, &hi);
     /* (a level the temporally blocked smoother handles exchanges once per pass, in front of it, on the main stream) */
-    return L->dist && mg->overlap && !mg->core.prof.enabled && hi - lo >= 4 && mg->smoother != MG_SMOOTHER_JACOBI && !level_takes_pipe(mg, L);
+    return L->dist && !mg->core.prof.enabled && hi - lo >= 4 && mg->smoother != MG_SMOOTHER_JACOBI && !level_takes_pipe(mg, L);
 }
 
 /* A halo exchange whose ghost planes are first read by the boundary-plane kernel of the smoothing call that follows
@@ -1067,7 +1055,7 @@ static int relax_level(mg3d_t* mg, int level, int ncycles) { return relax_level_
 static int correction_fuses(const mg3d_t* mg, int level, int v2)
 {
     const mg_level3d* L = &mg->lv[level];
-    return v2 >= 2 && level + 1 < mg->core.nlevels && level_takes_pipe(mg, L) && mg->lv[level + 1].has_pc && !mg->full_correction && !mg->no_corr_fuse;
+    return v2 >= 2 && level + 1 < mg->core.nlevels && level_takes_pipe(mg, L) && mg->lv[level + 1].has_pc && !mg->full_correction;
 }
 
 /* correct_first: the first two-sweep pass starts from v + Interpolate(v of level+1) on the colour-1 points (the caller has
@@ -1329,7 +1317,7 @@ static int residual_restrict_level(mg3d_t* mg, int fine_level, int defer_f_halo)
     coarse_share(mg, fine_level, &lo, &hi);
     /* the fused kernel reads v two planes below the slab: only plane a-2 is stale after the smoother's exchanges */
     if (F->dist) {
-        if (level_takes_pipe(mg, F) && !F->vg_deep && !mg->no_deep_merge) {
+        if (level_takes_pipe(mg, F) && !F->vg_deep) {
             /* v does not change between here and the first pass of the post-smoothing (prolongation and correction ride on that
                pass), so the four colour-1 planes that pass needs from each neighbour travel now, in the same launch: one
                exchange fewer on the way up */
@@ -1345,7 +1333,7 @@ static int residual_restrict_level(mg3d_t* mg, int fine_level, int defer_f_halo)
     {
         const void* fmaps[2] = {F->tmap_pf[0], F->tmap_pf[1]};
         MG_LAUNCH(mg->core.launches, mgk3d_residual_restrict_tma(mg->core.stream, mg->core.dtype, F->tmap_rr[F->cur][0], F->tmap_rr[F->cur][1],
-                                                            getenv("MG_B200_RR_NO_PREFETCH") ? NULL : fmaps, F->f, F->g, F->c,
+                                                            fmaps, F->f, F->g, F->c,
                                                             mg->mode == MG_CORRECTED, C->f, C->v, C->g, lo, hi));
     }
     else
@@ -1435,8 +1423,7 @@ static int vcycle_rec(mg3d_t* mg, int level, int v1, int v2)
 {
     int st;
     mg_level3d* L0 = &mg->lv[level];
-    if (L0->g.n <= MGK3D_TAIL_N && !L0->dist && mg->core.nlevels - level <= MGK3D_TAIL_MAX_LEVELS && mg->smoother != MG_SMOOTHER_JACOBI &&
-        !mg->no_tail) {
+    if (L0->g.n <= MGK3D_TAIL_N && !L0->dist && mg->core.nlevels - level <= MGK3D_TAIL_MAX_LEVELS && mg->smoother != MG_SMOOTHER_JACOBI) {
         /* the coarse tail: the whole recursion from here down in one launch of one CTA */
         mg_geom3d g[MGK3D_TAIL_MAX_LEVELS];
         mg_coef3d c[MGK3D_TAIL_MAX_LEVELS];

@@ -290,17 +290,6 @@ k_interp_octet(T* __restrict__ fine, mg_geom3d gf, const T* __restrict__ coarse,
     }
 }
 
-template <typename T>
-__global__ void k_apply_correction(T* __restrict__ fine, const T* __restrict__ err, mg_geom3d g, int zl_lo)
-{
-    const int x = 1 + blockIdx.x * blockDim.x + threadIdx.x;
-    const int y = 1 + blockIdx.y * blockDim.y + threadIdx.y;
-    const int zl = zl_lo + blockIdx.z;
-    if (x > g.n - 2 || y > g.n - 2) return;
-    const long long i = off3(g, x, y, zl);
-    fine[i] = add(fine[i], err[i]);
-}
-
 // zl_skip_lo < zl_skip_hi: the planes [zl_skip_lo, zl_skip_hi) are left out (a slab's own planes: only its ghost planes are set)
 template <typename T>
 __global__ void k_set(T* __restrict__ a, mg_geom3d g, T value, int modify_boundaries, int zl_lo, int zl_skip_lo, int zl_skip_hi)
@@ -515,17 +504,6 @@ int mgk3d_interpolate(cudaStream_t s, int dtype, void* fine, mg_geom3d gf, const
     else
         if (colour_mask == 2) k_interp_octet<double, 2><<<grid, block, 0, s>>>((double*)fine, gf, (const double*)coarse, gc, add, zl_lo, zl_hi, cz_first, cz_last, kchunk, cond);
         else k_interp_octet<double, 3><<<grid, block, 0, s>>>((double*)fine, gf, (const double*)coarse, gc, add, zl_lo, zl_hi, cz_first, cz_last, kchunk, cond);
-    return launch_ok();
-}
-
-int mgk3d_apply_correction(cudaStream_t s, int dtype, void* fine, const void* err, mg_geom3d g, int zl_lo, int zl_hi)
-{
-    if (zl_hi <= zl_lo || g.n < 3) return 0;
-    dim3 block = block2d(g.n), grid((g.n - 2 + block.x - 1) / block.x, (g.n - 2 + block.y - 1) / block.y, zl_hi - zl_lo);
-    if (dtype == 0)
-        k_apply_correction<float><<<grid, block, 0, s>>>((float*)fine, (const float*)err, g, zl_lo);
-    else
-        k_apply_correction<double><<<grid, block, 0, s>>>((double*)fine, (const double*)err, g, zl_lo);
     return launch_ok();
 }
 

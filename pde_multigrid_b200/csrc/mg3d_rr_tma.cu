@@ -25,8 +25,6 @@
 // profiles/r1_residual_restrict_tma_ncu_full.txt).
 // HBM traffic per fine point: v and f once (+ 19/16 x 36/32 halo re-reads that hit L2) and 2/8 coarse
 // writes: the algorithmic 2*B*N_l + 2*B*N_{l+1} of SURVEY.md 8(d).
-#include <stdlib.h>
-
 #include "mg3d_device.cuh"
 #include "mg_tma.cuh"
 
@@ -44,6 +42,7 @@ constexpr int RCOLS = CXT + 2;          // per-parity columns of a residual row 
 constexpr int RING = 6;   // v planes: z-1 .. z+2 live during a pair of planes + two in flight
 constexpr int RRING = 3;  // residual planes: 2k-1, 2k, 2k+1
 constexpr int NT = 256;
+constexpr int RR_ZCHUNK_MAX = 16;  // coarse planes per CTA before tile_grid halves it to fill the SMs
 
 template <typename T> struct VBox {
     static constexpr int A = 16 / sizeof(T);                      // TMA inner-coordinate alignment in elements
@@ -337,13 +336,9 @@ static void tile_grid(const mg_geom3d& gc, int czl_lo, int czl_hi, dim3& grid, i
 {
     const int planes = czl_hi - czl_lo;
     const int tiles_xy = ((gc.n + CXT - 1) / CXT) * ((gc.n + CYT - 1) / CYT);
-    static int zmax = -1;  // MG_B200_RR_ZCHUNK: coarse planes per CTA (every chunk re-reads two fine planes of halo and refills its ring)
-    if (zmax < 0) {
-        const char* env = getenv("MG_B200_RR_ZCHUNK");
-        zmax = env ? atoi(env) : 16;  // 16-24 measured best at 1025^3 (3.80 ms against 3.87 at 32, 4.28 at 64, 5.46 at 256: short chunks keep neighbouring tiles in step, and their shared halo rows in L2)
-        if (zmax < 8) zmax = 32;
-    }
-    zchunk = zmax;
+    // coarse planes per CTA: every chunk re-reads two fine planes of halo and refills its ring.  16-24 measured best at 1025^3
+    // (3.80 ms against 3.87 at 32, 4.28 at 64, 5.46 at 256: short chunks keep neighbouring tiles in step, and their shared halo rows in L2)
+    zchunk = RR_ZCHUNK_MAX;
     while (zchunk > 8 && (long long)tiles_xy * ((planes + zchunk - 1) / zchunk) < 148 * 4) zchunk /= 2;
     grid = dim3((gc.n + CXT - 1) / CXT, (gc.n + CYT - 1) / CYT, (planes + zchunk - 1) / zchunk);
 }

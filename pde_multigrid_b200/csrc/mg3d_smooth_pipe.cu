@@ -527,16 +527,7 @@ int launch(cudaStream_t s, const void* const maps3[3], const void* const cmaps2[
         const double cost = (double)((ctas + sms - 1) / sms) * (zc + 2 * ZH + 3);
         if (cost < best) { best = cost; nchunk = k; }
     }
-    int zchunk = (nz + nchunk - 1) / nchunk;
-    {
-        static int zforce = -1;  // MG_B200_PIPE_ZCHUNK: planes per z chunk (diagnostic; 0 = the cost model above)
-        if (zforce < 0) {
-            const char* env = getenv("MG_B200_PIPE_ZCHUNK");
-            zforce = env ? atoi(env) : 0;
-            if (zforce < 0) zforce = 0;
-        }
-        if (zforce >= 8) zchunk = zforce < nz ? zforce : nz;
-    }
+    const int zchunk = (nz + nchunk - 1) / nchunk;
     dim3 grid(tx, ty, (nz + zchunk - 1) / zchunk);
     if constexpr (R != 2) {
         if (corr) return -1;

@@ -8,7 +8,7 @@
 
 struct mg_comm_s {
     ncclComm_t comm;
-    int rank, nranks;
+    int rank;
 };
 
 static struct {
@@ -86,7 +86,6 @@ int mg_comm_create(mg_comm** out, int rank, int nranks, const void* unique_id128
         return mg_fail(MG_ERR_COMM, "ncclCommInitRank failed: %s", N.GetErrorString(r));
     }
     c->rank = rank;
-    c->nranks = nranks;
     *out = c;
     return MG_OK;
 }
@@ -97,9 +96,6 @@ void mg_comm_destroy(mg_comm* c)
     if (c->comm) N.CommDestroy(c->comm);
     free(c);
 }
-
-int mg_comm_rank(const mg_comm* c) { return c ? c->rank : 0; }
-int mg_comm_size(const mg_comm* c) { return c ? c->nranks : 1; }
 
 int mg_comm_group_start(mg_comm* c) { (void)c; MG_NCCL(N.GroupStart()); return MG_OK; }
 int mg_comm_group_end(mg_comm* c) { (void)c; MG_NCCL(N.GroupEnd()); return MG_OK; }

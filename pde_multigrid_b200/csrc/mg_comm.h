@@ -13,8 +13,6 @@ typedef struct mg_comm_s mg_comm;
 
 int mg_comm_create(mg_comm** out, int rank, int nranks, const void* unique_id128);
 void mg_comm_destroy(mg_comm* c);
-int mg_comm_rank(const mg_comm* c);
-int mg_comm_size(const mg_comm* c);
 
 int mg_comm_group_start(mg_comm* c);
 int mg_comm_group_end(mg_comm* c);

@@ -147,8 +147,6 @@ int mgk3d_residual_restrict_tma(cudaStream_t s, int dtype, const void* tmap_v_c0
 /* cond: NULL, or a device word: the launch does nothing unless it is nonzero (the exact fallback of mgk3d_relax_pipe2) */
 int mgk3d_interpolate(cudaStream_t s, int dtype, void* fine, mg_geom3d gf, const void* coarse, mg_geom3d gc, int add,
                       int colour_mask, int zl_lo, int zl_hi, const unsigned int* cond);
-/* fine interior += err interior (ApplyCorrection on two fine arrays) */
-int mgk3d_apply_correction(cudaStream_t s, int dtype, void* fine, const void* err, mg_geom3d g, int zl_lo, int zl_hi);
 /* setToValue */
 int mgk3d_set(cudaStream_t s, int dtype, void* a, mg_geom3d g, double value, int modify_boundaries, int zl_lo,
               int zl_hi);

@@ -4,7 +4,6 @@
  * library does not link against libcuda directly.
  */
 #include <cuda.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include "mg_host_common.h"
@@ -38,18 +37,10 @@ int mg_tma_make_colour_map(void* out128, int dtype, void* base, const mg_geom3d*
     cuuint64_t strides[2] = {(cuuint64_t)g->hp * es, (cuuint64_t)g->plane * es};
     cuuint32_t box[3] = {(cuuint32_t)box_i, (cuuint32_t)box_y, 1};
     cuuint32_t estr[3] = {1, 1, 1};
-    /* L2 promotion of the TMA requests: MG_B200_TMA_PROMO = 0 none, 1 64 B, 2 128 B, 3 256 B (diagnostic switch) */
-    static int promo = -1;
-    if (promo < 0) {
-        const char* env = getenv("MG_B200_TMA_PROMO");
-        promo = env ? atoi(env) & 3 : 3;
-    }
-    const CUtensorMapL2promotion promos[4] = {CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_64B,
-                                              CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B};
     CUtensorMap map;
     CUresult r = g_encode(&map, dtype == MG_F32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 3, base, dims,
                           strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                          promos[promo], CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+                          CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) return mg_fail(MG_ERR_CUDA, "cuTensorMapEncodeTiled failed with CUresult %d (hp=%d n=%d nzl=%d box=%dx%d)", (int)r, g->hp, g->n, g->nzl, box_i, box_y);
     memcpy(out128, &map, sizeof map);
     return MG_OK;
