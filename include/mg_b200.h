@@ -165,10 +165,16 @@ int mg3d_solve(mg3d_t* mg, int level, int v1, int v2, double rtol, double atol, 
  * bit for bit, v and f of the coarser levels hold preconditioner scratch (as after mg3d_vcycle); max_iters = 0, or an r_0
  * that already meets the target, leaves v and f as they were.
  * MG_ERR_ARG as mg3d_solve; MG_ERR_STATE on an MG_REF_COMPAT handle (its residual, N3/MultiGrid3D.cpp:723, is not a
- * symmetric operator) and on a distributed handle (nranks > 1); nothing runs in either case.
+ * symmetric operator); nothing runs in either case.
  * Memory: six fields of `level` (b, x and p twice, d), allocated by the first call on the level (MG_ERR_NOMEM before
  * anything runs if that fails) and freed by mg3d_destroy: 52 GB at 1025^3 fp64, on top of the 38 GB of the hierarchy.
- * The loop runs on the device like mg3d_solve's (DESIGN.md section 6b).  mg3b_pcg is the same on a box grid. */
+ * On a distributed handle every rank allocates six fields of its slab: about 54 GB per GPU at 2049^3 fp64 on 8 GPUs (a
+ * middle slab of 264 planes), on top of about 31 GB of hierarchy fields (estimates from the field sizes, not measured).
+ * The ranks agree on the outcome: a failure on any rank returns MG_ERR_NOMEM on every rank before anything runs.
+ * The loop runs on the device like mg3d_solve's (DESIGN.md section 6b).  On a distributed handle it is host-driven, one
+ * read-back per iteration, every rank returns the same iterations, converged flag and history, and the planes a rank owns
+ * hold the single-GPU bits on every level (the history's l2 agrees to rounding, as mg3d_residual_norm's does).  Collective:
+ * every rank calls it with the same arguments.  mg3b_pcg is the same on a box grid. */
 int mg3d_pcg(mg3d_t* mg, int level, int v1, int v2, double rtol, double atol, int max_iters,
              int* iters_out, int* converged_out, double* history);
 

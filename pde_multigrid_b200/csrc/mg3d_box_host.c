@@ -416,7 +416,7 @@ int mg3b_pcg(mg3b_t* mg, int level, int v1, int v2, double rtol, double atol, in
     if (!mg->pcg && !(mg->pcg = (mg_pcg_vecs*)calloc((size_t)mg->core.nlevels, sizeof *mg->pcg)))
         return mg_fail(MG_ERR_NOMEM, "host allocation failed");
     mg_level3b* L = &mg->lv[level];
-    if ((st = mg_pcg_vecs_alloc(&mg->pcg[level], field_bytes(L, mg->core.dtype), mg->core.stream))) return st;
+    if ((st = mg_pcg_vecs_alloc(&mg->pcg[level], field_bytes(L, mg->core.dtype), 0, mg->core.stream))) return st;
     mg_pcg_ctx pc;
     memset(&pc, 0, sizeof pc);
     pc.cx.h = mg; pc.cx.level = level; pc.cx.v1 = v1; pc.cx.v2 = v2;
@@ -431,6 +431,7 @@ int mg3b_pcg(mg3b_t* mg, int level, int v1, int v2, double rtol, double atol, in
     pc.f = L->f;
     pc.out2 = mg->d_scratch + 2 * MG3B_NPARTS;
     pc.v = p3b_v; pc.zero_v = p3b_zero_v; pc.vcycle = p3b_vcycle; pc.norm0 = p3b_norm0;
+    pc.own_hi = pc.wr_hi = L->g.nz;
     const int key[MG_GRAPH_KEY] = {level, v1, v2, 0, 0, 0, 0, MG_GRAPH_PCG};
     return mg_pcg_run(&pc, &mg->core.graphs, mg_graphs_on(&mg->core.graphs, 0, 2LL * (v1 + v2) * (mg->core.nlevels - level)) ? key : NULL, rtol,
                       atol, max_iters, iters_out, converged_out, history);

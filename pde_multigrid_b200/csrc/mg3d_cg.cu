@@ -23,6 +23,13 @@
 // MGK_PCG_BLOCKS blocks (two per SM) strides over the rows.  The rows in flight then span about one plane, and with the
 // planes on either side the stencil inputs stay in L2 until every point that needs them has read them (at 1025^3 fp64,
 // about 3 planes of 8.6 MB per field); each lane keeps four points in flight to cover the latency.
+//
+// Distributed levels (z-slabs, mg3d_host.c): the stencil passes take a write range [wr_lo, wr_hi) around their stencil and
+// reduction range [zl_lo, zl_hi).  p' and x' are pointwise, so they are also written on the planes next to the owned ones;
+// the next iteration reads p and x there as stencil neighbours, and no exchange of p or x is ever needed.  Each rank
+// finalises its dots into one double-double pair per dot (k_pcg_dd_local), the ranks all-gather the pairs, and
+// k_pcg_combine adds them in rank order: the value is again the correctly rounded dot product, so alpha and beta are the
+// single-GPU ones bit for bit.  One GPU passes equal ranges and finalises with k_pcg_scalars.
 #include <stdint.h>
 
 #include "mg3d_device.cuh"
@@ -40,6 +47,7 @@ namespace {
 
 constexpr int kThreads = 256;
 constexpr int kWarps = kThreads / 32;
+constexpr int kBlocksPerSm = 2; // MGK_PCG_BLOCKS on 148 SMs: a register budget of up to 128 per thread costs no occupancy
 
 // the half-row a warp works on: colour array `col`, local plane zl, row y; q = x & 1 of its points
 struct Row {
@@ -157,22 +165,30 @@ k_pcg_dots(const T* __restrict__ zv, const T* __restrict__ r, const T* __restric
     store_dd2(part, rho, rho_l, sig, sig_l);
 }
 
-// p_out = z + beta*p_in everywhere; pi = sum over the interior of p_out * (Laplacian p_out), the Laplacian taken as
-// -(CalculateResidual of p_out with f = 0), i.e. the residual expression's own grouping
+// p_out = z + beta*p_in on the write planes [wr_lo, wr_hi); pi = sum over the interior of planes [zl_lo, zl_hi) of
+// p_out * (Laplacian p_out), the Laplacian taken as -(CalculateResidual of p_out with f = 0), i.e. the residual expression's
+// own grouping
 template <typename T, bool FAST>
-__global__ void __launch_bounds__(kThreads)
+__global__ void __launch_bounds__(kThreads, kBlocksPerSm)
 k_pcg_dir(const T* __restrict__ zv, const T* __restrict__ p_in, T* __restrict__ p_out, mg_geom3cg g, Coef3<T> c,
-          const double* __restrict__ sc, int zl_lo, int zl_hi, double* __restrict__ part)
+          const double* __restrict__ sc, int wr_lo, int wr_hi, int zl_lo, int zl_hi, double* __restrict__ part)
 {
     __shared__ double sh[128];
     const T beta = (T)sc[MGK_PCG_BETA];
     double pi = 0.0, pi_l = 0.0, zero = 0.0, zero_l = 0.0;
-    const int nzr = zl_hi - zl_lo;
+    const int nzr = wr_hi - wr_lo;
     const long long rows = 2LL * nzr * g.ny;
     const int lane = threadIdx.x & 31;
     for (long long row = (long long)blockIdx.x * kWarps + (threadIdx.x >> 5); row < rows; row += (long long)gridDim.x * kWarps) {
-        const Row R = row_of(g, row, zl_lo);
+        const Row R = row_of(g, row, wr_lo);
         const long long own = (long long)R.col * g.cstride + R.base, oth = (long long)(R.col ^ 1) * g.cstride + R.base;
+        if (R.zl < zl_lo || R.zl >= zl_hi) { /* a write plane next to the reduction range: p_out only */
+            for (int i = lane; 2 * i + R.q < g.nx; i += 32) {
+                CG_CHK_SITE(g, i, R.y, R.zl);
+                p_out[own + i] = add(zv[own + i], mul(beta, p_in[own + i]));
+            }
+            continue;
+        }
 #pragma unroll 4
         for (int i = lane; 2 * i + R.q < g.nx; i += 32) {
             CG_CHK_SITE(g, i, R.y, R.zl);
@@ -194,23 +210,26 @@ k_pcg_dir(const T* __restrict__ zv, const T* __restrict__ p_in, T* __restrict__ 
     store_dd2(part, pi, pi_l, zero, zero_l);
 }
 
-// UPDATE: x_out = x_in + alpha*p, r' = b - Laplacian x_out into r (in place: a point reads only its own r), d = r' - r,
-//         {sum r'^2, max |r'|} partials in the layout of mgk_norm_final.  Dirichlet points keep x, get r' = d = 0.
-// !UPDATE (prologue): r = b - Laplacian x_in only, and the scalar block is marked "first iteration".
+// UPDATE: x_out = x_in + alpha*p on the write planes [wr_lo, wr_hi); on planes [zl_lo, zl_hi) also r' = b - Laplacian x_out
+//         into r (in place: a point reads only its own r), d = r' - r, {sum r'^2, max |r'|} partials in the layout of
+//         mgk_norm_final.  Dirichlet points keep x, get r' = d = 0.
+// !UPDATE (prologue, wr = zl): r = b - Laplacian x_in only, and the scalar block is marked "first iteration".
 template <typename T, bool FAST, bool UPDATE>
 __global__ void __launch_bounds__(kThreads)
 k_pcg_upd(const T* __restrict__ x_in, const T* __restrict__ p, const T* __restrict__ b, T* __restrict__ r, T* __restrict__ x_out,
-          T* __restrict__ d, mg_geom3cg g, Coef3<T> c, double* __restrict__ sc, int zl_lo, int zl_hi, double* __restrict__ part)
+          T* __restrict__ d, mg_geom3cg g, Coef3<T> c, double* __restrict__ sc, int wr_lo, int wr_hi, int zl_lo, int zl_hi,
+          double* __restrict__ part)
 {
     __shared__ double sh[64];
     const T alpha = UPDATE ? (T)sc[MGK_PCG_ALPHA] : T(0);
     double s = 0.0, m = 0.0;
-    const int nzr = zl_hi - zl_lo;
+    const int nzr = wr_hi - wr_lo;
     const long long rows = 2LL * nzr * g.ny;
     const int lane = threadIdx.x & 31;
     for (long long row = (long long)blockIdx.x * kWarps + (threadIdx.x >> 5); row < rows; row += (long long)gridDim.x * kWarps) {
-        const Row R = row_of(g, row, zl_lo);
+        const Row R = row_of(g, row, wr_lo);
         const long long own = (long long)R.col * g.cstride + R.base, oth = (long long)(R.col ^ 1) * g.cstride + R.base;
+        const bool reduce = R.zl >= zl_lo && R.zl < zl_hi;
 #pragma unroll 4
         for (int i = lane; 2 * i + R.q < g.nx; i += 32) {
             CG_CHK_SITE(g, i, R.y, R.zl);
@@ -218,21 +237,24 @@ k_pcg_upd(const T* __restrict__ x_in, const T* __restrict__ p, const T* __restri
             const T xo = x_in[own + i];
             T xc = xo, rn = T(0);
             if (!(R.bnd || x == 0 || x == g.nx - 1)) {
-                CG_NB(oth, i, R.q, g);
-                const T* xq = x_in + oth;
-                if (UPDATE) {
-                    const T* pq = p + oth;
-                    xc = add(xo, mul(alpha, p[own + i]));
-                    rn = residual_point<T, FAST>(add(xq[o_O], mul(alpha, pq[o_O])), add(xq[o_E], mul(alpha, pq[o_E])),
-                                                 add(xq[o_N], mul(alpha, pq[o_N])), add(xq[o_S], mul(alpha, pq[o_S])),
-                                                 add(xq[o_D], mul(alpha, pq[o_D])), add(xq[o_U], mul(alpha, pq[o_U])), xc,
-                                                 b[own + i], c, 1);
-                } else {
-                    rn = residual_point<T, FAST>(xq[o_O], xq[o_E], xq[o_N], xq[o_S], xq[o_D], xq[o_U], xo, b[own + i], c, 1);
+                if (UPDATE) xc = add(xo, mul(alpha, p[own + i]));
+                if (reduce) {
+                    CG_NB(oth, i, R.q, g);
+                    const T* xq = x_in + oth;
+                    if (UPDATE) {
+                        const T* pq = p + oth;
+                        rn = residual_point<T, FAST>(add(xq[o_O], mul(alpha, pq[o_O])), add(xq[o_E], mul(alpha, pq[o_E])),
+                                                     add(xq[o_N], mul(alpha, pq[o_N])), add(xq[o_S], mul(alpha, pq[o_S])),
+                                                     add(xq[o_D], mul(alpha, pq[o_D])), add(xq[o_U], mul(alpha, pq[o_U])), xc,
+                                                     b[own + i], c, 1);
+                    } else {
+                        rn = residual_point<T, FAST>(xq[o_O], xq[o_E], xq[o_N], xq[o_S], xq[o_D], xq[o_U], xo, b[own + i], c, 1);
+                    }
                 }
             }
+            if (UPDATE) x_out[own + i] = xc;
+            if (!reduce) continue;
             if (UPDATE) {
-                x_out[own + i] = xc;
                 d[own + i] = sub(rn, r[own + i]);
                 const double rd = (double)rn;
                 s += rd * rd;
@@ -249,19 +271,10 @@ k_pcg_upd(const T* __restrict__ x_in, const T* __restrict__ p, const T* __restri
     if (threadIdx.x == 0) { part[blockIdx.x] = s; part[gridDim.x + blockIdx.x] = m; }
 }
 
-// which 0 (after k_pcg_dots): rho, sigma -> beta = sigma / rho_prev (0 on the first iteration), rho_prev = rho;
-// which 1 (after k_pcg_dir): pi -> alpha = rho / pi.  The partials are double-double (store_dd2); each sum is rounded once.
-__global__ void __launch_bounds__(kThreads) k_pcg_scalars(const double* __restrict__ part, int nparts, double* __restrict__ sc, int which)
+// which 0 (after k_pcg_dots): rho = a, sigma = b -> beta = sigma / rho_prev (0 on the first iteration), rho_prev = rho;
+// which 1 (after k_pcg_dir): pi = a -> alpha = rho / pi
+__device__ __forceinline__ void set_scalars(double* sc, int which, double a, double b)
 {
-    __shared__ double sh[128];
-    double ah = 0.0, al = 0.0, bh = 0.0, bl = 0.0;
-    for (int i = threadIdx.x; i < nparts; i += blockDim.x) {
-        dd_add(ah, al, part[i], part[nparts + i]);
-        dd_add(bh, bl, part[2 * nparts + i], part[3 * nparts + i]);
-    }
-    block_sum_dd2(ah, al, bh, bl, sh);
-    if (threadIdx.x != 0) return;
-    const double a = __dadd_rn(ah, al), b = __dadd_rn(bh, bl);
     if (which == 0) {
         const int first = sc[MGK_PCG_FIRST] != 0.0;
         sc[MGK_PCG_BETA] = first ? 0.0 : b / sc[MGK_PCG_RHO];
@@ -273,65 +286,126 @@ __global__ void __launch_bounds__(kThreads) k_pcg_scalars(const double* __restri
     }
 }
 
+// the block partials (store_dd2) of one dot pass summed in double-double: valid in thread 0
+__device__ __forceinline__ void sum_parts(const double* __restrict__ part, int nparts, double& ah, double& al, double& bh, double& bl,
+                                          double* sh)
+{
+    for (int i = threadIdx.x; i < nparts; i += blockDim.x) {
+        dd_add(ah, al, part[i], part[nparts + i]);
+        dd_add(bh, bl, part[2 * nparts + i], part[3 * nparts + i]);
+    }
+    block_sum_dd2(ah, al, bh, bl, sh);
+}
+
+// one GPU: the partials -> the scalars; each sum is rounded once
+__global__ void __launch_bounds__(kThreads) k_pcg_scalars(const double* __restrict__ part, int nparts, double* __restrict__ sc, int which)
+{
+    __shared__ double sh[128];
+    double ah = 0.0, al = 0.0, bh = 0.0, bl = 0.0;
+    sum_parts(part, nparts, ah, al, bh, bl, sh);
+    if (threadIdx.x != 0) return;
+    set_scalars(sc, which, __dadd_rn(ah, al), __dadd_rn(bh, bl));
+}
+
+// a slab of a distributed level: the partials -> this rank's two double-double sums {a hi, a lo, b hi, b lo}, unrounded
+__global__ void __launch_bounds__(kThreads) k_pcg_dd_local(const double* __restrict__ part, int nparts, double* __restrict__ dd)
+{
+    __shared__ double sh[128];
+    double ah = 0.0, al = 0.0, bh = 0.0, bl = 0.0;
+    sum_parts(part, nparts, ah, al, bh, bl, sh);
+    if (threadIdx.x != 0) return;
+    dd[0] = ah; dd[1] = al; dd[2] = bh; dd[3] = bl;
+}
+
+// the all-gathered sums of every rank added in rank order, rounded once -> the scalars
+__global__ void k_pcg_combine(const double* __restrict__ dd, int nranks, double* __restrict__ sc, int which)
+{
+    double ah = 0.0, al = 0.0, bh = 0.0, bl = 0.0;
+    for (int k = 0; k < nranks; k++) {
+        dd_add(ah, al, dd[4 * k], dd[4 * k + 1]);
+        dd_add(bh, bl, dd[4 * k + 2], dd[4 * k + 3]);
+    }
+    set_scalars(sc, which, __dadd_rn(ah, al), __dadd_rn(bh, bl));
+}
+
+// the finaliser of a dot pass: the scalars (dd == NULL), or this rank's sums into dd
+void finalise(cudaStream_t s, const double* part, double* sc, int which, double* dd)
+{
+    if (dd)
+        k_pcg_dd_local<<<1, kThreads, 0, s>>>(part, MGK_PCG_BLOCKS, dd);
+    else
+        k_pcg_scalars<<<1, kThreads, 0, s>>>(part, MGK_PCG_BLOCKS, sc, which);
+}
+
 template <typename T>
-int launch_dots(cudaStream_t s, const void* z, const void* r, const void* d, mg_geom3cg g, int zl_lo, int zl_hi, double* part, double* sc)
+int launch_dots(cudaStream_t s, const void* z, const void* r, const void* d, mg_geom3cg g, int zl_lo, int zl_hi, double* part, double* sc,
+                double* dd)
 {
     k_pcg_dots<T><<<MGK_PCG_BLOCKS, kThreads, 0, s>>>((const T*)z, (const T*)r, (const T*)d, g, zl_lo, zl_hi, part);
-    k_pcg_scalars<<<1, kThreads, 0, s>>>(part, MGK_PCG_BLOCKS, sc, 0);
+    finalise(s, part, sc, 0, dd);
     return cudaPeekAtLastError() == cudaSuccess ? 2 : -1;
 }
 
 template <typename T>
-int launch_dir(cudaStream_t s, const void* z, const void* p_in, void* p_out, mg_geom3cg g, mg_coef3d c, int zl_lo, int zl_hi, double* part,
-               double* sc)
+int launch_dir(cudaStream_t s, const void* z, const void* p_in, void* p_out, mg_geom3cg g, mg_coef3d c, int wr_lo, int wr_hi, int zl_lo,
+               int zl_hi, double* part, double* sc, double* dd)
 {
     if (c.fast_h)
-        k_pcg_dir<T, true><<<MGK_PCG_BLOCKS, kThreads, 0, s>>>((const T*)z, (const T*)p_in, (T*)p_out, g, narrow<T>(c), sc, zl_lo, zl_hi, part);
+        k_pcg_dir<T, true><<<MGK_PCG_BLOCKS, kThreads, 0, s>>>((const T*)z, (const T*)p_in, (T*)p_out, g, narrow<T>(c), sc, wr_lo, wr_hi, zl_lo,
+                                                                zl_hi, part);
     else
-        k_pcg_dir<T, false><<<MGK_PCG_BLOCKS, kThreads, 0, s>>>((const T*)z, (const T*)p_in, (T*)p_out, g, narrow<T>(c), sc, zl_lo, zl_hi, part);
-    k_pcg_scalars<<<1, kThreads, 0, s>>>(part, MGK_PCG_BLOCKS, sc, 1);
+        k_pcg_dir<T, false><<<MGK_PCG_BLOCKS, kThreads, 0, s>>>((const T*)z, (const T*)p_in, (T*)p_out, g, narrow<T>(c), sc, wr_lo, wr_hi, zl_lo,
+                                                                 zl_hi, part);
+    finalise(s, part, sc, 1, dd);
     return cudaPeekAtLastError() == cudaSuccess ? 2 : -1;
 }
 
 template <typename T, bool UPDATE>
 int launch_upd(cudaStream_t s, const void* x_in, const void* p, const void* b, void* r, void* x_out, void* d, mg_geom3cg g, mg_coef3d c,
-               double* sc, int zl_lo, int zl_hi, double* part)
+               double* sc, int wr_lo, int wr_hi, int zl_lo, int zl_hi, double* part)
 {
     if (c.fast_h)
         k_pcg_upd<T, true, UPDATE><<<MGK_PCG_BLOCKS, kThreads, 0, s>>>((const T*)x_in, (const T*)p, (const T*)b, (T*)r, (T*)x_out, (T*)d,
-                                                                        g, narrow<T>(c), sc, zl_lo, zl_hi, part);
+                                                                        g, narrow<T>(c), sc, wr_lo, wr_hi, zl_lo, zl_hi, part);
     else
         k_pcg_upd<T, false, UPDATE><<<MGK_PCG_BLOCKS, kThreads, 0, s>>>((const T*)x_in, (const T*)p, (const T*)b, (T*)r, (T*)x_out, (T*)d,
-                                                                         g, narrow<T>(c), sc, zl_lo, zl_hi, part);
+                                                                         g, narrow<T>(c), sc, wr_lo, wr_hi, zl_lo, zl_hi, part);
     return cudaPeekAtLastError() == cudaSuccess ? 1 : -1;
 }
 
 }  // namespace
 
 extern "C" int mgk3cg_dots(cudaStream_t s, int dtype, const void* z, const void* r, const void* d, mg_geom3cg g, int zl_lo, int zl_hi,
-                           double* part, double* sc)
+                           double* part, double* sc, double* dd)
 {
-    return dtype == 0 ? launch_dots<float>(s, z, r, d, g, zl_lo, zl_hi, part, sc) : launch_dots<double>(s, z, r, d, g, zl_lo, zl_hi, part, sc);
+    return dtype == 0 ? launch_dots<float>(s, z, r, d, g, zl_lo, zl_hi, part, sc, dd)
+                      : launch_dots<double>(s, z, r, d, g, zl_lo, zl_hi, part, sc, dd);
 }
 
-extern "C" int mgk3cg_dir(cudaStream_t s, int dtype, const void* z, const void* p_in, void* p_out, mg_geom3cg g, mg_coef3d c, int zl_lo,
-                          int zl_hi, double* part, double* sc)
+extern "C" int mgk3cg_dir(cudaStream_t s, int dtype, const void* z, const void* p_in, void* p_out, mg_geom3cg g, mg_coef3d c, int wr_lo,
+                          int wr_hi, int zl_lo, int zl_hi, double* part, double* sc, double* dd)
 {
-    return dtype == 0 ? launch_dir<float>(s, z, p_in, p_out, g, c, zl_lo, zl_hi, part, sc)
-                      : launch_dir<double>(s, z, p_in, p_out, g, c, zl_lo, zl_hi, part, sc);
+    return dtype == 0 ? launch_dir<float>(s, z, p_in, p_out, g, c, wr_lo, wr_hi, zl_lo, zl_hi, part, sc, dd)
+                      : launch_dir<double>(s, z, p_in, p_out, g, c, wr_lo, wr_hi, zl_lo, zl_hi, part, sc, dd);
+}
+
+extern "C" int mgk3cg_combine(cudaStream_t s, const double* dd, int nranks, double* sc, int which)
+{
+    k_pcg_combine<<<1, 1, 0, s>>>(dd, nranks, sc, which);
+    return cudaPeekAtLastError() == cudaSuccess ? 1 : -1;
 }
 
 extern "C" int mgk3cg_update(cudaStream_t s, int dtype, const void* x_in, const void* p, const void* b, void* r, void* x_out, void* d,
-                             mg_geom3cg g, mg_coef3d c, const double* sc, int zl_lo, int zl_hi, double* part)
+                             mg_geom3cg g, mg_coef3d c, const double* sc, int wr_lo, int wr_hi, int zl_lo, int zl_hi, double* part)
 {
     double* scw = const_cast<double*>(sc);
-    return dtype == 0 ? launch_upd<float, true>(s, x_in, p, b, r, x_out, d, g, c, scw, zl_lo, zl_hi, part)
-                      : launch_upd<double, true>(s, x_in, p, b, r, x_out, d, g, c, scw, zl_lo, zl_hi, part);
+    return dtype == 0 ? launch_upd<float, true>(s, x_in, p, b, r, x_out, d, g, c, scw, wr_lo, wr_hi, zl_lo, zl_hi, part)
+                      : launch_upd<double, true>(s, x_in, p, b, r, x_out, d, g, c, scw, wr_lo, wr_hi, zl_lo, zl_hi, part);
 }
 
 extern "C" int mgk3cg_residual(cudaStream_t s, int dtype, const void* x, const void* b, void* r, mg_geom3cg g, mg_coef3d c, double* sc,
                                int zl_lo, int zl_hi)
 {
-    return dtype == 0 ? launch_upd<float, false>(s, x, nullptr, b, r, nullptr, nullptr, g, c, sc, zl_lo, zl_hi, nullptr)
-                      : launch_upd<double, false>(s, x, nullptr, b, r, nullptr, nullptr, g, c, sc, zl_lo, zl_hi, nullptr);
+    return dtype == 0 ? launch_upd<float, false>(s, x, nullptr, b, r, nullptr, nullptr, g, c, sc, zl_lo, zl_hi, zl_lo, zl_hi, nullptr)
+                      : launch_upd<double, false>(s, x, nullptr, b, r, nullptr, nullptr, g, c, sc, zl_lo, zl_hi, zl_lo, zl_hi, nullptr);
 }

@@ -1546,16 +1546,49 @@ int mg3d_solve(mg3d_t* mg, int level, int v1, int v2, double rtol, double atol, 
 /* ---- multigrid-preconditioned conjugate gradients (mg_host_common.c runs the loop, mg3d_cg.cu has the vector passes) ---- */
 
 static void* p3_v(mg_cycle_ctx* x) { return ((mg3d_t*)x->h)->lv[x->level].v; }
-static int p3_vcycle(mg_cycle_ctx* x) { return vcycle_rec(x->h, x->level, x->v1, x->v2); }
+/* a slab runs the V-cycle through the cycle-graph cache, as the host-driven distributed solve does */
+static int p3_vcycle(mg_cycle_ctx* x)
+{
+    mg3d_t* mg = x->h;
+    return mg->lv[x->level].dist ? mg3d_vcycle(mg, x->level, x->v1, x->v2) : vcycle_rec(mg, x->level, x->v1, x->v2);
+}
 static int p3_norm0(mg_cycle_ctx* x) { return residual_norm_enqueue(x->h, x->level); }
-/* setToValue(v, 0, true) on the buffer the V-cycle starts from */
-static int p3_zero_v(mg_cycle_ctx* x)
+/* setToValue(v, 0, true) on the buffer the V-cycle starts from; on a slab the ghost planes too, behind the handshake
+   exchange, and those of the other buffer (mirror_v_ghosts): the preconditioner's Dirichlet values are 0 */
+static int p3_zero_v(mg_cycle_ctx* x) { return mg3d_set_to_value(x->h, x->level, MG_FIELD_V, 0.0, 1); }
+
+/* ---- the slab hooks: the only communication of a distributed PCG outside its V-cycles ---- */
+/* r' on the owned planes of f: the temporally blocked pass sweeps halo planes and reads f there, four deep */
+static int p3_r_written(mg_cycle_ctx* x) { mg3d_t* mg = x->h; return exchange(mg, x->level, mg->lv[x->level].f, 3, MG_GHOST_LO, MG_GHOST_HI); }
+/* the direction pass reads z on the planes next to the owned ones */
+static int p3_z_ready(mg_cycle_ctx* x) { return ensure_v_ghosts(x->h, x->level); }
+static int p3_allgather(mg_cycle_ctx* x, double* dd) { mg3d_t* mg = x->h; return mg_comm_allgather_inplace(mg->comm, dd, 4, MG_F64, mg->core.stream); }
+static int p3_allreduce(mg_cycle_ctx* x, double* out2) { mg3d_t* mg = x->h; return mg_comm_allreduce_sum_max(mg->comm, out2, mg->core.stream); }
+/* as mg3d_set_field_device after the owned planes of v are written: the caller's boundary values are back in every ghost
+   plane of both buffers */
+static int p3_v_restored(mg_cycle_ctx* x)
 {
     mg3d_t* mg = x->h;
     mg_level3d* L = &mg->lv[x->level];
-    MG_LAUNCH(mg->core.launches, mgk3d_set(mg->core.stream, mg->core.dtype, L->v, L->g, 0.0, 1, 0, L->g.nzl));
+    int st = exchange(mg, x->level, L->v, 3, MG_GHOST_LO, MG_GHOST_HI);
+    if (st) return st;
     L->vg_valid = L->vg_deep = 1;
-    return MG_OK;
+    return mirror_v_ghosts(mg, x->level);
+}
+
+/* The first pcg on a level allocates on every rank.  A rank that failed alone would leave its peers waiting in the first
+   exchange, so the ranks agree on the outcome first (one all-reduce); if any failed, every rank frees its vectors. */
+static int pcg_alloc_agree(mg3d_t* mg, int level, int st)
+{
+    double* d = norm_out2(mg);
+    mg->core.h_out2[0] = mg->core.h_out2[1] = st ? 1.0 : 0.0;
+    MG_CUDA(cudaMemcpyAsync(d, mg->core.h_out2, 2 * sizeof(double), cudaMemcpyHostToDevice, mg->core.stream));
+    int st2 = mg_comm_allreduce_sum_max(mg->comm, d, mg->core.stream);
+    if (!st2) st2 = mg_read_out2(&mg->core, d);
+    if (st2) return st2;
+    if (mg->core.h_out2[1] == 0.0) return MG_OK;
+    if (!st) mg_pcg_vecs_free(&mg->pcg[level]);
+    return st ? st : mg_fail(MG_ERR_NOMEM, "PCG vectors: %g of %d ranks could not allocate theirs", mg->core.h_out2[0], mg->nranks);
 }
 
 int mg3d_pcg(mg3d_t* mg, int level, int v1, int v2, double rtol, double atol, int max_iters, int* iters_out, int* converged_out,
@@ -1564,11 +1597,13 @@ int mg3d_pcg(mg3d_t* mg, int level, int v1, int v2, double rtol, double atol, in
     int st = mg_solve_check_args(MG_CORE(mg), level, rtol, atol, max_iters, v1, v2);
     if (st) return st;
     if (mg->mode != MG_CORRECTED) return mg_fail(MG_ERR_STATE, "pcg needs MG_CORRECTED: the MG_REF_COMPAT residual is not a symmetric operator");
-    if (mg->nranks > 1) return mg_fail(MG_ERR_STATE, "pcg runs on one GPU (distributed handle of %d ranks)", mg->nranks);
-    if (!mg->pcg && !(mg->pcg = (mg_pcg_vecs*)calloc((size_t)mg->core.nlevels, sizeof *mg->pcg)))
-        return mg_fail(MG_ERR_NOMEM, "host allocation failed");
     mg_level3d* L = &mg->lv[level];
-    if ((st = mg_pcg_vecs_alloc(&mg->pcg[level], field_bytes(L, mg->core.dtype), mg->core.stream))) return st;
+    const int fresh = !mg->pcg || !mg->pcg[level].b;
+    if (!mg->pcg) mg->pcg = (mg_pcg_vecs*)calloc((size_t)mg->core.nlevels, sizeof *mg->pcg);
+    st = mg->pcg ? mg_pcg_vecs_alloc(&mg->pcg[level], field_bytes(L, mg->core.dtype), L->dist ? mg->nranks : 0, mg->core.stream)
+                 : mg_fail(MG_ERR_NOMEM, "host allocation failed");
+    if (fresh && mg->nranks > 1) st = pcg_alloc_agree(mg, level, st);
+    if (st) return st;
     mg_pcg_ctx pc;
     memset(&pc, 0, sizeof pc);
     pc.cx.h = mg; pc.cx.level = level; pc.cx.v1 = v1; pc.cx.v2 = v2;
@@ -1584,10 +1619,23 @@ int mg3d_pcg(mg3d_t* mg, int level, int v1, int v2, double rtol, double atol, in
     pc.out2 = norm_out2(mg);
     pc.v = p3_v; pc.zero_v = p3_zero_v; pc.vcycle = p3_vcycle; pc.norm0 = p3_norm0;
     pc.save = c3_save; pc.load = c3_load;
+    pc.own_lo = pc.wr_lo = 0;
+    pc.own_hi = pc.wr_hi = L->g.nzl;
+    if (L->dist) {
+        pc.own_lo = L->own_lo; pc.own_hi = L->own_hi;
+        pc.wr_lo = L->own_lo > 0 ? L->own_lo - 1 : 0;
+        pc.wr_hi = L->own_hi < L->g.nzl ? L->own_hi + 1 : L->g.nzl;
+        pc.rank = mg->rank; pc.nranks = mg->nranks;
+        pc.r_written = p3_r_written; pc.z_ready = p3_z_ready; pc.allgather = p3_allgather; pc.allreduce = p3_allreduce;
+        pc.v_restored = p3_v_restored;
+    }
     int key[MG_GRAPH_KEY];
     graph_key(&pc.cx, 0, key);
     key[MG_GRAPH_KEY_KIND] = MG_GRAPH_PCG;
-    st = mg_pcg_run(&pc, &mg->core.graphs, graphs_on(mg, level, v1, v2) ? key : NULL, rtol, atol, max_iters, iters_out, converged_out, history);
+    /* a distributed handle stays host-driven, as mg3d_solve does (the NCCL collectives are not known to be legal inside a
+       conditional body); every rank checks the same all-reduced norm and stops after the same iteration */
+    const int device = mg->nranks == 1 && graphs_on(mg, level, v1, v2);
+    st = mg_pcg_run(&pc, &mg->core.graphs, device ? key : NULL, rtol, atol, max_iters, iters_out, converged_out, history);
     return st ? st : halo_error_check(mg);
 }
 

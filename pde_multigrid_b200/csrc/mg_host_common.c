@@ -451,16 +451,17 @@ int mg_solve_run(mg_graphs* gr, const int key[MG_GRAPH_KEY], const mg_cycle_ops*
 
 /* ---- multigrid-preconditioned conjugate gradients ------------------------------------------------ */
 
-int mg_pcg_vecs_alloc(mg_pcg_vecs* P, size_t field_bytes, cudaStream_t s)
+int mg_pcg_vecs_alloc(mg_pcg_vecs* P, size_t field_bytes, int nranks, cudaStream_t s)
 {
     if (P->b) return MG_OK;
     void** f[6] = {&P->b, &P->x[0], &P->x[1], &P->p[0], &P->p[1], &P->d};
+    const size_t nparts = MGK_PCG_PARTS + MGK_PCG_SCALARS + 4 * (size_t)nranks;
     cudaError_t e = cudaSuccess;
     for (int i = 0; i < 6 && e == cudaSuccess; i++) e = cudaMalloc(f[i], field_bytes);
-    if (e == cudaSuccess) e = cudaMalloc((void**)&P->parts, (MGK_PCG_PARTS + MGK_PCG_SCALARS) * sizeof(double));
+    if (e == cudaSuccess) e = cudaMalloc((void**)&P->parts, nparts * sizeof(double));
     /* the row padding is never read for a result, but it is copied into v at the end: keep it defined */
     for (int i = 0; i < 6 && e == cudaSuccess; i++) e = cudaMemsetAsync(*f[i], 0, field_bytes, s);
-    if (e == cudaSuccess) e = cudaMemsetAsync(P->parts, 0, (MGK_PCG_PARTS + MGK_PCG_SCALARS) * sizeof(double), s);
+    if (e == cudaSuccess) e = cudaMemsetAsync(P->parts, 0, nparts * sizeof(double), s);
     if (e == cudaSuccess) {
         P->bytes = field_bytes;
         return MG_OK;
@@ -479,6 +480,19 @@ void mg_pcg_vecs_free(mg_pcg_vecs* P)
 }
 
 static double* pcg_sc(const mg_pcg_ctx* pc) { return pc->P->parts + MGK_PCG_PARTS; }
+/* slabs: the all-gathered dot sums, and where this rank's go (NULL on one GPU: the passes' own finaliser forms the scalars) */
+static double* pcg_dd(const mg_pcg_ctx* pc) { return pc->allgather ? pc->P->parts + MGK_PCG_PARTS + MGK_PCG_SCALARS : NULL; }
+static double* pcg_dd_mine(const mg_pcg_ctx* pc) { return pc->allgather ? pcg_dd(pc) + 4 * pc->rank : NULL; }
+
+/* slabs: every rank's sums of the dot pass just enqueued -> beta (which 0) or alpha (which 1) */
+static int pcg_combine(mg_pcg_ctx* pc, int which)
+{
+    if (!pc->allgather) return MG_OK;
+    int st = pc->allgather(&pc->cx, pcg_dd(pc));
+    if (st) return st;
+    MG_LAUNCH(*pc->launches, mgk3cg_combine(pc->stream, pcg_dd(pc), pc->nranks, pcg_sc(pc), which));
+    return MG_OK;
+}
 
 /* norm(r_0) with the family's own pass (the same bits as mg?d_residual_norm), then b <- f, x <- v, r_0 = b - Laplacian x into f */
 static int pcg_first(void* c)
@@ -492,8 +506,8 @@ static int pcg_first(void* c)
     MG_CUDA(cudaMemcpyAsync(P->x[0], pc->v(&pc->cx), P->bytes, cudaMemcpyDeviceToDevice, pc->stream));
     MG_CUDA(cudaMemsetAsync(P->p[0], 0, P->bytes, pc->stream)); /* beta = 0 multiplies it on the first iteration */
     MG_CUDA(cudaMemsetAsync(P->d, 0, P->bytes, pc->stream));
-    MG_LAUNCH(*pc->launches, mgk3cg_residual(pc->stream, pc->dtype, P->x[0], P->b, pc->f, pc->g, pc->c, pcg_sc(pc), 0, pc->g.nzl));
-    return MG_OK;
+    MG_LAUNCH(*pc->launches, mgk3cg_residual(pc->stream, pc->dtype, P->x[0], P->b, pc->f, pc->g, pc->c, pcg_sc(pc), pc->own_lo, pc->own_hi));
+    return pc->r_written ? pc->r_written(&pc->cx) : MG_OK;
 }
 
 /* one iteration: z = VCycle(0; r) in v, beta, p, alpha, x, r, the norm partials of the new r */
@@ -505,20 +519,24 @@ static int pcg_step(void* c)
     double *part = P->parts, *sc = pcg_sc(pc);
     int st;
     if ((st = pc->zero_v(&pc->cx)) || (st = pc->vcycle(&pc->cx))) return st;
+    if (pc->z_ready && (st = pc->z_ready(&pc->cx))) return st;
     const void* z = pc->v(&pc->cx);
-    MG_LAUNCH(*pc->launches, mgk3cg_dots(pc->stream, pc->dtype, z, pc->f, P->d, pc->g, 0, pc->g.nzl, part, sc));
-    MG_LAUNCH(*pc->launches, mgk3cg_dir(pc->stream, pc->dtype, z, P->p[a], P->p[n], pc->g, pc->c, 0, pc->g.nzl, part + MGK_PCG_DIR_PARTS, sc));
-    MG_LAUNCH(*pc->launches, mgk3cg_update(pc->stream, pc->dtype, P->x[a], P->p[n], P->b, pc->f, P->x[n], P->d, pc->g, pc->c, sc, 0, pc->g.nzl,
-                                           part + MGK_PCG_UPD_PARTS));
+    MG_LAUNCH(*pc->launches, mgk3cg_dots(pc->stream, pc->dtype, z, pc->f, P->d, pc->g, pc->own_lo, pc->own_hi, part, sc, pcg_dd_mine(pc)));
+    if ((st = pcg_combine(pc, 0))) return st;
+    MG_LAUNCH(*pc->launches, mgk3cg_dir(pc->stream, pc->dtype, z, P->p[a], P->p[n], pc->g, pc->c, pc->wr_lo, pc->wr_hi, pc->own_lo, pc->own_hi,
+                                        part + MGK_PCG_DIR_PARTS, sc, pcg_dd_mine(pc)));
+    if ((st = pcg_combine(pc, 1))) return st;
+    MG_LAUNCH(*pc->launches, mgk3cg_update(pc->stream, pc->dtype, P->x[a], P->p[n], P->b, pc->f, P->x[n], P->d, pc->g, pc->c, sc, pc->wr_lo,
+                                           pc->wr_hi, pc->own_lo, pc->own_hi, part + MGK_PCG_UPD_PARTS));
     pc->par = n;
-    return MG_OK;
+    return pc->r_written ? pc->r_written(&pc->cx) : MG_OK;
 }
 
 static int pcg_norm(void* c)
 {
     mg_pcg_ctx* pc = (mg_pcg_ctx*)c;
     MG_LAUNCH(*pc->launches, mgk_norm_final(pc->stream, pc->P->parts + MGK_PCG_UPD_PARTS, MGK_PCG_BLOCKS, pc->out2));
-    return MG_OK;
+    return pc->allreduce ? pc->allreduce(&pc->cx, pc->out2) : MG_OK;
 }
 
 static void pcg_save(void* c, unsigned out[2])
@@ -539,6 +557,17 @@ static void pcg_load(void* c, const unsigned in[2])
     pc->par = (int)(in[0] >> 31);
 }
 
+/* planes [lo, hi) of both colours of a field, src -> dst */
+static int copy_planes(const mg_pcg_ctx* pc, void* dst, const void* src, int lo, int hi)
+{
+    const size_t es = mg_esize(pc->dtype), pb = (size_t)pc->g.plane * es;
+    for (int col = 0; col < 2; col++) {
+        const size_t off = ((size_t)col * (size_t)pc->g.cstride + (size_t)lo * (size_t)pc->g.plane) * es;
+        MG_CUDA(cudaMemcpyAsync((char*)dst + off, (const char*)src + off, pb * (size_t)(hi - lo), cudaMemcpyDeviceToDevice, pc->stream));
+    }
+    return MG_OK;
+}
+
 int mg_pcg_run(mg_pcg_ctx* pc, mg_graphs* gr, const int key[MG_GRAPH_KEY], double rtol, double atol, int max_iters, int* iters_out,
                int* converged_out, double* history)
 {
@@ -546,8 +575,17 @@ int mg_pcg_run(mg_pcg_ctx* pc, mg_graphs* gr, const int key[MG_GRAPH_KEY], doubl
     int st = mg_solve_run(gr, key, &ops, rtol, atol, max_iters, iters_out, converged_out, history);
     if (st) return st;
     /* v of the level (the buffer the last V-cycle ended on) <- x, f <- b: the caller's f bit for bit */
-    MG_CUDA(cudaMemcpyAsync(pc->v(&pc->cx), pc->P->x[pc->par], pc->P->bytes, cudaMemcpyDeviceToDevice, pc->stream));
-    MG_CUDA(cudaMemcpyAsync(pc->f, pc->P->b, pc->P->bytes, cudaMemcpyDeviceToDevice, pc->stream));
+    if (!pc->v_restored) {
+        MG_CUDA(cudaMemcpyAsync(pc->v(&pc->cx), pc->P->x[pc->par], pc->P->bytes, cudaMemcpyDeviceToDevice, pc->stream));
+        MG_CUDA(cudaMemcpyAsync(pc->f, pc->P->b, pc->P->bytes, cudaMemcpyDeviceToDevice, pc->stream));
+    } else {
+        /* a slab: x and b hold current values on the owned planes only (x also on the next plane each way); the ghost planes
+           of v and f come from the neighbours, and those exchanges are also the handshake behind which a neighbour may
+           store into them again */
+        if ((st = copy_planes(pc, pc->v(&pc->cx), pc->P->x[pc->par], pc->own_lo, pc->own_hi)) || (st = pc->v_restored(&pc->cx)) ||
+            (st = copy_planes(pc, pc->f, pc->P->b, pc->own_lo, pc->own_hi)) || (st = pc->r_written(&pc->cx)))
+            return st;
+    }
     MG_CUDA(cudaStreamSynchronize(pc->stream));
     return MG_OK;
 }

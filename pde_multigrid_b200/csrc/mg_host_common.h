@@ -140,13 +140,15 @@ int mg_solve_run(mg_graphs* gr, const int key[MG_GRAPH_KEY], const mg_cycle_ops*
 /* ---- multigrid-preconditioned conjugate gradients (mg3d_pcg, mg3b_pcg; DESIGN.md §6b) ----
    The loop is mg_solve_run's: ops.first = norm(r_0) + prologue, ops.cycle = one PCG iteration (its V-cycle included),
    ops.norm = the norm finaliser of the iteration's update pass.  x and p ping-pong between two buffers, so the iteration's
-   parity is part of the state ops.save / ops.load carry (bit 31 of [0]) and a device loop always has the two-iteration body. */
+   parity is part of the state ops.save / ops.load carry (bit 31 of [0]) and a device loop always has the two-iteration body.
+   A slab of a distributed level (DESIGN.md section 6b) adds the hooks and plane ranges of mg_pcg_ctx; its loop is host-driven. */
 typedef struct {
     void* b;          /* the caller's f of the level, put back at the end */
     void* x[2];       /* the iterate */
     void* p[2];       /* the search direction */
     void* d;          /* r_k - r_{k-1} */
-    double* parts;    /* MGK_PCG_PARTS partials of the three passes (mg_launch.h), then MGK_PCG_SCALARS scalars */
+    double* parts;    /* MGK_PCG_PARTS partials of the three passes (mg_launch.h), MGK_PCG_SCALARS scalars, then (slabs) the
+                         all-gathered double-double dot sums, 4 per rank */
     size_t bytes;     /* of one field */
 } mg_pcg_vecs;
 
@@ -167,10 +169,20 @@ typedef struct {
     int (*norm0)(mg_cycle_ctx* cx); /* the family's residual-norm pass (mg?d_residual_norm without the read-back) */
     void (*save)(void* cx, unsigned out[2]); /* NULL, or the family's host-side buffer state */
     void (*load)(void* cx, const unsigned in[2]);
+    /* local planes: the dots, residual and norm cover [own_lo, own_hi), the pointwise updates of p and x [wr_lo, wr_hi).
+       One GPU (and a level every rank holds whole): both are all planes and the hooks below are NULL. */
+    int own_lo, own_hi, wr_lo, wr_hi;
+    int rank, nranks;
+    int (*r_written)(mg_cycle_ctx* cx);    /* f (= r) holds new owned planes: bring its ghost planes up to date */
+    int (*z_ready)(mg_cycle_ctx* cx);      /* the preconditioner has left z in v: at least one ghost plane of v each way */
+    int (*allgather)(mg_cycle_ctx* cx, double* dd); /* dd[4*rank .. 4*rank+3] of every rank into every rank's dd, in place */
+    int (*allreduce)(mg_cycle_ctx* cx, double* out2); /* {sum, max} over the ranks, in place */
+    int (*v_restored)(mg_cycle_ctx* cx);   /* v holds the iterate on the owned planes: refresh its ghost planes as after set_field */
 } mg_pcg_ctx;
 
-/* allocates the vectors of one level on first use (MG_ERR_NOMEM, nothing allocated, when that fails) */
-int mg_pcg_vecs_alloc(mg_pcg_vecs* P, size_t field_bytes, cudaStream_t s);
+/* allocates the vectors of one level on first use (MG_ERR_NOMEM, nothing allocated, when that fails); nranks: room for the
+   dot sums of that many ranks (0 where the level is not distributed) */
+int mg_pcg_vecs_alloc(mg_pcg_vecs* P, size_t field_bytes, int nranks, cudaStream_t s);
 void mg_pcg_vecs_free(mg_pcg_vecs* P);
 /* the whole PCG: the loop through mg_solve_run (device-driven when key != NULL), then v <- x, f <- b */
 int mg_pcg_run(mg_pcg_ctx* pc, mg_graphs* gr, const int key[MG_GRAPH_KEY], double rtol, double atol, int max_iters, int* iters_out,

@@ -217,17 +217,23 @@ typedef struct {
 #define MGK_PCG_DIR_PARTS (4 * MGK_PCG_BLOCKS)
 #define MGK_PCG_UPD_PARTS (8 * MGK_PCG_BLOCKS)
 #define MGK_PCG_PARTS (10 * MGK_PCG_BLOCKS)
-/* every launcher covers local planes [zl_lo, zl_hi) (on one GPU: all of them) */
+/* every launcher reduces over local planes [zl_lo, zl_hi) (on one GPU: all of them).  The stencil passes write their
+   pointwise output on [wr_lo, wr_hi), which contains [zl_lo, zl_hi) (a slab: the owned planes and one more on each side
+   inside the stored ones; one GPU: the same range).  dd: NULL on one GPU, where the dot passes' finaliser forms beta / alpha;
+   on a slab it receives this rank's unrounded double-double sums {a hi, a lo, b hi, b lo}, and mgk3cg_combine forms the
+   scalars once the ranks have all-gathered them. */
 /* rho = z.r, sigma = z.d -> beta (two launches) */
 int mgk3cg_dots(cudaStream_t s, int dtype, const void* z, const void* r, const void* d, mg_geom3cg g, int zl_lo, int zl_hi,
-                double* part, double* sc);
+                double* part, double* sc, double* dd);
 /* p_out = z + beta*p_in, pi = p_out.(Laplacian p_out) -> alpha (two launches) */
-int mgk3cg_dir(cudaStream_t s, int dtype, const void* z, const void* p_in, void* p_out, mg_geom3cg g, mg_coef3d c, int zl_lo,
-               int zl_hi, double* part, double* sc);
+int mgk3cg_dir(cudaStream_t s, int dtype, const void* z, const void* p_in, void* p_out, mg_geom3cg g, mg_coef3d c, int wr_lo,
+               int wr_hi, int zl_lo, int zl_hi, double* part, double* sc, double* dd);
+/* dd[4*k .. 4*k+3] of ranks k = 0..nranks-1 added in rank order -> beta (which 0, after mgk3cg_dots) or alpha (which 1) */
+int mgk3cg_combine(cudaStream_t s, const double* dd, int nranks, double* sc, int which);
 /* x_out = x_in + alpha*p, r = b - Laplacian x_out (in place over the old r), d = new r - old r; {sum r^2, max|r|} partials
    for mgk_norm_final */
 int mgk3cg_update(cudaStream_t s, int dtype, const void* x_in, const void* p, const void* b, void* r, void* x_out, void* d,
-                  mg_geom3cg g, mg_coef3d c, const double* sc, int zl_lo, int zl_hi, double* part);
+                  mg_geom3cg g, mg_coef3d c, const double* sc, int wr_lo, int wr_hi, int zl_lo, int zl_hi, double* part);
 /* r = b - Laplacian x (zero on the Dirichlet points), and the scalar block marked for a first iteration */
 int mgk3cg_residual(cudaStream_t s, int dtype, const void* x, const void* b, void* r, mg_geom3cg g, mg_coef3d c, double* sc,
                     int zl_lo, int zl_hi);

@@ -213,7 +213,9 @@ class _PCGMixin:
         """Conjugate gradients preconditioned by one VCycle(level, v1, v2) per iteration (mg3d_pcg / mg3b_pcg) on the
         MG_CORRECTED operator, from the current v, until the true residual meets ||r_k||_2 <= max(atol, rtol * ||r_0||_2)
         or max_iters iterations have run.  Returns a SolveResult whose `cycles` counts iterations (one V-cycle each).
-        v of `level` holds the iterate afterwards, f of `level` is unchanged."""
+        v of `level` holds the iterate afterwards, f of `level` is unchanged.  On a distributed handle every rank calls it
+        with the same arguments; the loop is host-driven there, every rank gets the same result, and the planes a rank owns
+        hold the bits of the single-GPU pcg."""
         hist = np.empty((max(int(max_iters), 0) + 1, 2), dtype=np.float64)
         iters, converged = ctypes.c_int(), ctypes.c_int()
         self._call("pcg", ctypes.c_int(level), ctypes.c_int(v1), ctypes.c_int(v2), ctypes.c_double(rtol),

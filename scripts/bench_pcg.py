@@ -12,9 +12,17 @@ For each configuration, one JSON line with the card's name and power limit (read
 Every key is warmed up first: the first solve()/pcg() of a key runs host-driven, the second builds the graph.
 
     python scripts/bench_pcg.py [--reps 5] [--only cube1025,box1025x513x257,...]
+
+--gpus N (N > 1) runs the distributed engine on N z-slabs instead, relaunching itself under torchrun with one rank per GPU:
+cube 1025^3 with the default smoother and with weighted Jacobi, and 2049^3 on 8 GPUs.  Both loops are host-driven there
+(one read-back per cycle or iteration).  solve_ms / pcg_ms are the medians of each rank's alternating calls, then the
+maximum over the ranks; halo_bytes_per_iter is what rank 0 sends per PCG iteration (its V-cycle included).
+
+    python scripts/bench_pcg.py --gpus 8 [--reps 3] [--only cube1025,cube1025_jacobi,cube2049]
 """
 import argparse
 import json
+import os
 import statistics
 import subprocess
 import sys
@@ -23,7 +31,7 @@ import time
 import numpy as np
 import torch
 
-sys.path.insert(0, ".")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import pde_multigrid_b200 as mg  # noqa: E402
 
 COPY_PEAK_GBS = 6451.8
@@ -31,10 +39,10 @@ COPY_PEAK_GBS = 6451.8
 PASS_FIELDS = {"k_pcg_dots": 3, "k_pcg_dir": 3, "k_pcg_upd": 7}
 
 
-def card():
-    name = torch.cuda.get_device_name(0)
+def card(device=0):
+    name = torch.cuda.get_device_name(device)
     try:
-        out = subprocess.run(["nvidia-smi", "-i", "0", "--query-gpu=power.limit", "--format=csv,noheader,nounits"],
+        out = subprocess.run(["nvidia-smi", "-i", str(device), "--query-gpu=power.limit", "--format=csv,noheader,nounits"],
                              capture_output=True, text=True, timeout=30).stdout.strip()
         power = float(out.splitlines()[0])
     except Exception:
@@ -124,13 +132,89 @@ def measure(eng, v1, v2, rtol, cap, reps, points):
                 solve_ms_all=t_solve, pcg_ms_all=t_pcg, kernels=kernels)
 
 
+def dist_configs(world):
+    out = [("cube1025", 1025, None), ("cube1025_jacobi", 1025, mg.MG_SMOOTHER_JACOBI)]
+    if world == 8:
+        out.append(("cube2049", 2049, None))
+    return out
+
+
+def dist_main(args):
+    """one rank of the --gpus run (under torchrun)"""
+    import ctypes
+
+    import torch.distributed as dist
+    rank, world, local = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"]), int(os.environ["LOCAL_RANK"])
+    torch.cuda.set_device(local)
+    dist.init_process_group("nccl", device_id=torch.device("cuda", local))
+    name, power = card(local)
+    only = set(filter(None, args.only.split(",")))
+    rtol, cap, (v1, v2) = 1e-9, 200, (2, 2)
+
+    def rank_max(x):
+        t = torch.tensor([x], dtype=torch.float64, device="cuda")
+        dist.all_reduce(t, op=dist.ReduceOp.MAX)
+        return t.item()
+
+    for tag, n, smoother in dist_configs(world):
+        if only and tag not in only:
+            continue
+        buf = torch.zeros(128, dtype=torch.uint8, device="cuda")
+        if rank == 0:
+            raw = (ctypes.c_ubyte * 128)()
+            mg._lib.check(mg.lib().mg_comm_unique_id(raw))
+            buf.copy_(torch.tensor(list(raw), dtype=torch.uint8))
+        dist.broadcast(buf, 0)
+        eng = mg.MultiGrid3D(n, dtype=np.float64, residual_mode=mg.MG_CORRECTED, rank=rank, nranks=world,
+                             nccl_unique_id=bytes(buf.cpu().tolist()))
+        if smoother is not None:
+            eng.set_smoother(smoother)
+        for _ in range(2):  # cycle graphs, PCG vectors, Jacobi scratch
+            eng.init_problem()
+            eng.solve(v1, v2, rtol=0.0, max_cycles=2)
+            eng.init_problem()
+            eng.pcg(v1, v2, rtol=0.0, max_iters=2)
+        t_solve, t_pcg, s = [], [], None
+        for _ in range(args.reps):
+            eng.init_problem()
+            eng.sync()
+            t0 = time.perf_counter()
+            s = eng.solve(v1, v2, rtol=rtol, max_cycles=cap)
+            t_solve.append((time.perf_counter() - t0) * 1e3)
+            eng.init_problem()
+            eng.sync()
+            h0 = eng.halo_bytes
+            t0 = time.perf_counter()
+            p = eng.pcg(v1, v2, rtol=rtol, max_iters=cap)
+            t_pcg.append((time.perf_counter() - t0) * 1e3)
+            halo = (eng.halo_bytes - h0) / max(p.cycles, 1)
+        solve_ms, pcg_ms = rank_max(statistics.median(t_solve)), rank_max(statistics.median(t_pcg))
+        eng.close()
+        if rank == 0:
+            print(json.dumps(dict(config=tag, shape=(n,) * 3, gpus=world, v1=v1, v2=v2, rtol=rtol, dtype="float64", gpu=name,
+                                  power_limit_w=power, cycles=s.cycles, iters=p.cycles, solve_converged=s.converged,
+                                  pcg_converged=p.converged, solve_ms=solve_ms, pcg_ms=pcg_ms, speedup=solve_ms / pcg_ms,
+                                  solve_ms_per_cycle=solve_ms / max(s.cycles, 1), pcg_ms_per_iter=pcg_ms / max(p.cycles, 1),
+                                  halo_bytes_per_iter=halo)), flush=True)
+    dist.destroy_process_group()
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--reps", type=int, default=5)
     ap.add_argument("--only", default="")
+    ap.add_argument("--gpus", type=int, default=1)
     args = ap.parse_args()
     if not torch.cuda.is_available():
         sys.exit("bench_pcg: no CUDA device (there is no CPU path)")
+    if args.gpus > 1:
+        if "RANK" in os.environ:
+            return dist_main(args)
+        if torch.cuda.device_count() < args.gpus:
+            sys.exit("bench_pcg: --gpus %d but %d devices" % (args.gpus, torch.cuda.device_count()))
+        cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", str(args.gpus), "--master-addr",
+               "127.0.0.1", "--master-port", "29563", os.path.abspath(__file__)] + sys.argv[1:]
+        sys.exit(subprocess.run(cmd).returncode)
     torch.cuda.init()
     name, power = card()
     only = set(filter(None, args.only.split(",")))
