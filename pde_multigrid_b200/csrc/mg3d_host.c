@@ -44,7 +44,6 @@ typedef struct {
     int dist;       /* 1: slab-distributed over the ranks; 0: the whole level lives on this rank */
     int own_lo;     /* local plane range [own_lo, own_hi) owned by this rank */
     int own_hi;
-    int has_tma;    /* tensor maps of the two colour arrays of v are valid */
     /* temporally blocked smoother: it works out of place, v ping-pongs between two buffers */
     void* vbuf[2];  /* vbuf[cur] == v; vbuf[1] is NULL when the level has no second buffer */
     int cur;
@@ -56,8 +55,6 @@ typedef struct {
     unsigned char tmap_pp[2][128] __attribute__((aligned(64)));    /* pipelined smoother: colour-1 array of v, [buffer] */
     unsigned char tmap_pf[2][128] __attribute__((aligned(64)));    /* pipelined smoother: f, [colour] */
     unsigned char tmap_pc[2][2][128] __attribute__((aligned(64))); /* this level's v as the COARSE operand of the finer level's pass: [buffer][colour] */
-    int has_pc;
-    int iso;        /* hx2 == hy2 == hz2 */
     /* distributed levels: 1 = the ghost planes of v (both colours, 2 below / 1 above) hold the neighbours' current values.
        Every operator leaves it 1 except the temporally blocked smoother, whose pass only writes the planes a rank owns;
        whoever reads ghost planes of v calls ensure_v_ghosts() first. */
@@ -89,7 +86,7 @@ struct mg3d_s {
     mg_core core;
     int mode;
     int rank, nranks;
-    int smoother, sweeps_per_pass;
+    int smoother;
     double range[6];
     cudaStream_t cstream;       /* side stream: halo exchange of the boundary planes overlapping the interior sweep */
     cudaEvent_t ev_fork, ev_join;
@@ -190,11 +187,9 @@ static size_t field_bytes(const mg_level3d* L, int dtype)
     return mg_align256(2 * (size_t)L->g.cstride * mg_esize(dtype));
 }
 
+/* the levels with tensor maps (create_common makes them or fails).  The temporally blocked smoothers run there only, so
+   these are the levels that keep a second v in the arena behind v and f. */
 static int level_uses_tma(int n) { return (n - 1) / 2 >= MGK3D_TMA_IT; }
-
-/* fields a level keeps in the arena: v, f and, where the temporally blocked smoothers can run (the large levels), a second v */
-static int level_fields_for(int n, int dist) { (void)dist; return level_uses_tma(n) ? 3 : 2; }
-static int level_fields(const mg_level3d* L) { return level_fields_for(L->g.n, L->dist); }
 
 static void* field_ptr(mg_level3d* L, int field) { return field == MG_FIELD_V ? L->v : L->f; }
 
@@ -447,7 +442,7 @@ static int p2p_setup(mg3d_t* mg)
             q->nb_off[k][3 * l] = off; off += fb;
             q->nb_off[k][3 * l + 1] = off; off += fb;
             q->nb_off[k][3 * l + 2] = off;
-            if (level_fields_for(mg->lv[l].g.n, plan[0]) == 3) off += fb;
+            if (level_uses_tma(mg->lv[l].g.n)) off += fb;
         }
     }
     q->all_arena = (char**)calloc((size_t)P, sizeof(char*));
@@ -466,7 +461,7 @@ static int p2p_setup(mg3d_t* mg)
             o[0] = off; off += fb;
             o[1] = off; off += fb;
             o[2] = off;
-            if (level_fields_for(mg->lv[l].g.n, plan[0]) == 3) off += fb;
+            if (level_uses_tma(mg->lv[l].g.n)) off += fb;
         }
     }
     MG_CUDA(cudaMalloc((void**)&q->flags, MG_HALO_FLAG_WORDS * sizeof(unsigned int)));
@@ -589,7 +584,6 @@ static int create_common(mg3d_t** out, const int sz[3], const double range[6], i
     mg->rank = rank;
     mg->nranks = nranks;
     mg->smoother = MG_SMOOTHER_AUTO;
-    mg->sweeps_per_pass = 1;
     mg->omega = 6.0 / 7.0;
     mg->arith = MG_ARITH_EXACT;
     mg->full_correction = getenv("MG_B200_FULL_CORRECTION") != NULL;
@@ -611,7 +605,7 @@ static int create_common(mg3d_t** out, const int sz[3], const double range[6], i
         L->vg_valid = 1;
         L->vg_deep = 1;
         level_coefs(dtype, nl, range, L->h, &L->c);
-        total += (size_t)level_fields(L) * field_bytes(L, dtype);
+        total += (size_t)(level_uses_tma(nl) ? 3 : 2) * field_bytes(L, dtype);
         nl = (nl - 1) / 2 + 1; /* N3/MultiGrid3D.cpp:40-42 */
     }
     cudaError_t e = cudaMalloc(&mg->arena_raw, total + 2 * MG_ARENA_SLACK);
@@ -626,7 +620,7 @@ static int create_common(mg3d_t** out, const int sz[3], const double range[6], i
         L->v = p; p += field_bytes(L, dtype);
         L->f = p; p += field_bytes(L, dtype);
         L->vbuf[0] = L->v;
-        if (level_fields(L) == 3) { L->vbuf[1] = p; p += field_bytes(L, dtype); }
+        if (level_uses_tma(L->g.n)) { L->vbuf[1] = p; p += field_bytes(L, dtype); }
     }
     if ((st = mg_core_init(&mg->core))) { mg3d_destroy(mg); return st; }
     if (cudaMalloc((void**)&mg->d_scratch, (2 * MGK_NORM_MAX_PARTS + 2) * sizeof(double)) != cudaSuccess ||
@@ -654,7 +648,6 @@ static int create_common(mg3d_t** out, const int sz[3], const double range[6], i
         if (!level_uses_tma(L->g.n)) continue;
         const int es = (int)mg_esize(dtype);
         for (int b = 0; b < 2 && !st; b++) {
-            if (!L->vbuf[b]) continue;
             for (int col = 0; col < 2 && !st; col++) {
                 char* base = plane_ptr(mg, L, L->vbuf[b], col, 0);
                 st = mg_tma_make_colour_map(L->tmap_v[b][col], dtype, base, &L->g, MGK3D_TMA_BOX_I(es), MGK3D_TMA_BOX_Y);
@@ -667,14 +660,12 @@ static int create_common(mg3d_t** out, const int sz[3], const double range[6], i
             st = mg_tma_make_colour_map(L->tmap_ff[col], dtype, plane_ptr(mg, L, L->f, col, 0), &L->g, MGK3D_FU_BOX_I(es), MGK3D_FU_BOX_Y);
             if (!st) st = mg_tma_make_colour_map(L->tmap_pf[col], dtype, plane_ptr(mg, L, L->f, col, 0), &L->g, MGK3D_PP_BOX_I(es), MGK3D_PP_BOX_Y);
         }
-        L->iso = L->c.hx2 == L->c.hy2 && L->c.hy2 == L->c.hz2;
         if (st) { mg3d_destroy(mg); return st; }
-        L->has_tma = 1;
     }
     /* a level below one with tensor maps is the coarse operand of that level's fused prolongation */
     for (int l = 1; l < mg->core.nlevels && !st; l++) {
         mg_level3d* L = &mg->lv[l];
-        if (!mg->lv[l - 1].has_tma) continue;
+        if (!level_uses_tma(mg->lv[l - 1].g.n)) continue;
         const int es = (int)mg_esize(dtype);
         for (int b = 0; b < 2 && !st; b++) {
             if (!L->vbuf[b]) continue;
@@ -682,7 +673,6 @@ static int create_common(mg3d_t** out, const int sz[3], const double range[6], i
                 st = mg_tma_make_colour_map(L->tmap_pc[b][col], dtype, plane_ptr(mg, L, L->vbuf[b], col, 0), &L->g, MGK3D_PP_CBOX_I(es), MGK3D_PP_CBOX_Y);
         }
         if (st) { mg3d_destroy(mg); return st; }
-        L->has_pc = 1;
     }
     /* pad elements of the layout are never used by a kernel, but keep them defined */
     if (cudaMemsetAsync(mg->arena_raw, 0, total + 2 * MG_ARENA_SLACK, mg->core.stream) != cudaSuccess) {
@@ -767,7 +757,6 @@ int mg3d_set_smoother(mg3d_t* mg, int smoother, int sweeps_per_pass)
         return mg_fail(MG_ERR_ARG, "sweeps_per_pass %d is not what smoother %d does (%s)", sweeps_per_pass, smoother,
                        smoother == MG_SMOOTHER_AUTO ? "1 or 2" : two ? "2" : "1");
     mg->smoother = smoother;
-    mg->sweeps_per_pass = sweeps_per_pass;
     return MG_OK;
 }
 
@@ -977,21 +966,45 @@ static int relax_launch(mg3d_t* mg, mg_level3d* L, int colour, int lo, int hi, i
     return MG_OK;
 }
 
-/* 1 when relax_level(level, n > 0) takes the overlapped path: the boundary planes of the slab and their halo exchange
-   run on the side stream while the interior planes are swept; every half-sweep ends with a join */
-static int level_takes_pipe(const mg3d_t* mg, const mg_level3d* L)
+/* the kernel family that relaxes a level: PIPE (register-tiled) and FUSED (shared memory) are the temporally blocked
+   smoothers, the COLOUR ones sweep one colour per launch */
+typedef enum { MG_RELAX_JACOBI, MG_RELAX_PIPE, MG_RELAX_FUSED, MG_RELAX_COLOUR_TMA, MG_RELAX_COLOUR } mg_relax3d;
+typedef struct {
+    mg_relax3d relax;    /* PIPE and FUSED run pairs of sweeps; an odd last sweep runs as COLOUR_TMA */
+    int tma;             /* residual+restrict, the residual norm and the one-colour sweeps read v through tensor maps */
+    int tail;            /* the V-cycle from this level down is one launch of the coarse-tail kernel */
+    int correct_colour1; /* a correction followed by red-black post-smoothing only needs the colour-1 points */
+} mg_path3d;
+
+/* The kernels that work on `level`: the only place that decides them.  Computed on every call from the smoother, the level's
+   geometry and coefficients and MG_B200_FULL_CORRECTION, so a mg3d_set_smoother between two calls takes effect. */
+static mg_path3d level_path(const mg3d_t* mg, int level)
 {
-    return (mg->smoother == MG_SMOOTHER_PIPE || mg->smoother == MG_SMOOTHER_AUTO) && L->has_tma && L->vbuf[1] &&
-           L->c.fast_den && L->iso && mgk3d_pipe_exact_range(mg->core.dtype, L->c.hx2) && (!L->dist || L->own_hi - L->own_lo >= 8);
+    const mg_level3d* L = &mg->lv[level];
+    const int s = mg->smoother;
+    mg_path3d p;
+    p.tma = level_uses_tma(L->g.n) && level + 1 < mg->core.nlevels && s != MG_SMOOTHER_COLOUR; /* the TMA residuals read level+1 */
+    /* the scaled arithmetic of the pipelined pass is exact: the same power-of-two h^2 on every axis, inside its guard's range */
+    const int pipe_exact = L->c.fast_den && L->c.hx2 == L->c.hy2 && L->c.hy2 == L->c.hz2 && mgk3d_pipe_exact_range(mg->core.dtype, L->c.hx2);
+    p.relax = s == MG_SMOOTHER_JACOBI ? MG_RELAX_JACOBI
+            : (s == MG_SMOOTHER_PIPE || s == MG_SMOOTHER_AUTO) && p.tma && pipe_exact && (!L->dist || L->own_hi - L->own_lo >= 8) ? MG_RELAX_PIPE
+            : s == MG_SMOOTHER_FUSED && p.tma && !L->dist ? MG_RELAX_FUSED
+            : p.tma ? MG_RELAX_COLOUR_TMA : MG_RELAX_COLOUR;
+    p.tail = L->g.n <= MGK3D_TAIL_N && !L->dist && mg->core.nlevels - level <= MGK3D_TAIL_MAX_LEVELS && p.relax != MG_RELAX_JACOBI;
+    p.correct_colour1 = p.relax != MG_RELAX_JACOBI && !mg->full_correction;
+    return p;
 }
 
+/* 1 when relax_level(level, n > 0) takes the overlapped path: the boundary planes of the slab and their halo exchange
+   run on the side stream while the interior planes are swept; every half-sweep ends with a join.  (A level the temporally
+   blocked smoother handles exchanges once per pass, in front of it, on the main stream.) */
 static int relax_overlaps(const mg3d_t* mg, int level)
 {
     const mg_level3d* L = &mg->lv[level];
+    const mg_relax3d r = level_path(mg, level).relax;
     int lo, hi;
     interior_range(L, &lo, &hi);
-    /* (a level the temporally blocked smoother handles exchanges once per pass, in front of it, on the main stream) */
-    return L->dist && !mg->core.prof.enabled && hi - lo >= 4 && mg->smoother != MG_SMOOTHER_JACOBI && !level_takes_pipe(mg, L);
+    return L->dist && !mg->core.prof.enabled && hi - lo >= 4 && (r == MG_RELAX_COLOUR_TMA || r == MG_RELAX_COLOUR);
 }
 
 /* A halo exchange whose ghost planes are first read by the boundary-plane kernel of the smoothing call that follows
@@ -1047,15 +1060,12 @@ static int relax_jacobi_level(mg3d_t* mg, int level, int ncycles)
     return MG_OK;
 }
 
-static int relax_level_ex(mg3d_t* mg, int level, int ncycles, int correct_first);
-
-static int relax_level(mg3d_t* mg, int level, int ncycles) { return relax_level_ex(mg, level, ncycles, 0); }
-
-/* 1 when VCycle's Interpolate + ApplyCorrection on `level` can ride on the first pass of the post-smoothing */
+/* 1 when VCycle's Interpolate + ApplyCorrection on `level` can ride on the first pass of the post-smoothing: that pass
+   corrects the colour-1 points only.  (A PIPE level has tensor maps, so the coarser level has its tmap_pc.) */
 static int correction_fuses(const mg3d_t* mg, int level, int v2)
 {
-    const mg_level3d* L = &mg->lv[level];
-    return v2 >= 2 && level + 1 < mg->core.nlevels && level_takes_pipe(mg, L) && mg->lv[level + 1].has_pc && !mg->full_correction;
+    const mg_path3d p = level_path(mg, level);
+    return v2 >= 2 && p.relax == MG_RELAX_PIPE && p.correct_colour1;
 }
 
 /* correct_first: the first two-sweep pass starts from v + Interpolate(v of level+1) on the colour-1 points (the caller has
@@ -1066,12 +1076,12 @@ static int relax_level_ex(mg3d_t* mg, int level, int ncycles, int correct_first)
     int lo, hi, st;
     interior_range(L, &lo, &hi);
     if (ncycles <= 0) return MG_OK;
-    if (mg->smoother == MG_SMOOTHER_JACOBI) return relax_jacobi_level(mg, level, ncycles);
-    const int use_tma = L->has_tma && mg->smoother != MG_SMOOTHER_COLOUR;
+    const mg_path3d p = level_path(mg, level);
+    if (p.relax == MG_RELAX_JACOBI) return relax_jacobi_level(mg, level, ncycles);
     /* register-tiled temporally blocked smoother (the default where it applies): two full sweeps per pass, out of place.
        Bit-exact mode: the pass range-checks everything it touches; the conditional literal-arithmetic pass behind it only
        runs (and then recomputes the same output buffer from the untouched input) if that check failed. */
-    if (level_takes_pipe(mg, L)) {
+    if (p.relax == MG_RELAX_PIPE) {
         while (ncycles >= 2) {
             const void* maps3[3] = {L->tmap_pp[L->cur], L->tmap_pf[0], L->tmap_pf[1]};
             const void* maps4[4] = {L->tmap_fu[L->cur][0], L->tmap_fu[L->cur][1], L->tmap_ff[0], L->tmap_ff[1]};
@@ -1115,7 +1125,7 @@ static int relax_level_ex(mg3d_t* mg, int level, int ncycles, int correct_first)
     L->vg_deep = 0; /* the sweeps below refresh one ghost plane per side only */
     /* the shared-memory version of the same idea (literal arithmetic; slower than four colour launches, kept as the
        exact fallback above and selectable for tests) */
-    if (mg->smoother == MG_SMOOTHER_FUSED && L->has_tma && L->vbuf[1] && !L->dist) {
+    if (p.relax == MG_RELAX_FUSED) {
         while (ncycles >= 2) {
             const void* maps4[4] = {L->tmap_fu[L->cur][0], L->tmap_fu[L->cur][1], L->tmap_ff[0], L->tmap_ff[1]};
             PROF_BEGIN(mg, level, MG_OP_RELAX);
@@ -1139,18 +1149,20 @@ static int relax_level_ex(mg3d_t* mg, int level, int ncycles, int correct_first)
                 MG_LAUNCH(mg->core.launches, mgk3d_relax_colour_pair(mg->cstream, mg->core.dtype, L->v, L->f, L->g, L->c, colour, lo, hi - 1));
                 if ((st = exchange_on(mg, level, L->v, 1 << colour, 1, 1, mg->cstream))) return st;
                 MG_CUDA(cudaEventRecord(mg->ev_join, mg->cstream));
-                if ((st = relax_launch(mg, L, colour, lo + 1, hi - 1, use_tma))) return st;
+                if ((st = relax_launch(mg, L, colour, lo + 1, hi - 1, p.tma))) return st;
                 MG_CUDA(cudaStreamWaitEvent(mg->core.stream, mg->ev_join, 0));
                 continue;
             }
             PROF_BEGIN(mg, level, MG_OP_RELAX);
-            st = relax_launch(mg, L, colour, lo, hi, use_tma);
+            st = relax_launch(mg, L, colour, lo, hi, p.tma);
             PROF_END(mg);
             if (st) return st;
             if ((st = exchange(mg, level, L->v, 1 << colour, 1, 1))) return st;
         }
     return MG_OK;
 }
+
+static int relax_level(mg3d_t* mg, int level, int ncycles) { return relax_level_ex(mg, level, ncycles, 0); }
 
 int mg3d_relax(mg3d_t* mg, int level, int ncycles)
 {
@@ -1191,7 +1203,7 @@ static int residual_norm_enqueue(mg3d_t* mg, int level)
     if ((st = ensure_v_ghosts(mg, level))) return st;
     double* out2 = norm_out2(mg);
     int k = -2;
-    if (L->has_tma && mg->smoother != MG_SMOOTHER_COLOUR && level + 1 < mg->core.nlevels) {
+    if (level_path(mg, level).tma) {
         /* large levels: the staging of the fused residual+restrict kernel; the coarse planes this rank restricts to
            lie over exactly the fine planes it owns */
         int clo, chi;
@@ -1313,11 +1325,12 @@ int mg3d_restrict(mg3d_t* mg, int fine_level, int field)
 static int residual_restrict_level(mg3d_t* mg, int fine_level, int defer_f_halo)
 {
     mg_level3d *F = &mg->lv[fine_level], *C = &mg->lv[fine_level + 1];
+    const mg_path3d p = level_path(mg, fine_level);
     int lo, hi, st;
     coarse_share(mg, fine_level, &lo, &hi);
     /* the fused kernel reads v two planes below the slab: only plane a-2 is stale after the smoother's exchanges */
     if (F->dist) {
-        if (level_takes_pipe(mg, F) && !F->vg_deep) {
+        if (p.relax == MG_RELAX_PIPE && !F->vg_deep) {
             /* v does not change between here and the first pass of the post-smoothing (prolongation and correction ride on that
                pass), so the four colour-1 planes that pass needs from each neighbour travel now, in the same launch: one
                exchange fewer on the way up */
@@ -1329,8 +1342,7 @@ static int residual_restrict_level(mg3d_t* mg, int fine_level, int defer_f_halo)
         F->vg_valid = 1;
     }
     PROF_BEGIN(mg, fine_level, MG_OP_RESIDUAL_RESTRICT);
-    if (F->has_tma && mg->smoother != MG_SMOOTHER_COLOUR)
-    {
+    if (p.tma) {
         const void* fmaps[2] = {F->tmap_pf[0], F->tmap_pf[1]};
         MG_LAUNCH(mg->core.launches, mgk3d_residual_restrict_tma(mg->core.stream, mg->core.dtype, F->tmap_rr[F->cur][0], F->tmap_rr[F->cur][1],
                                                             fmaps, F->f, F->g, F->c,
@@ -1374,12 +1386,11 @@ static int interpolate_level(mg3d_t* mg, int fine_level, int add, int colour_mas
     MG_LAUNCH(mg->core.launches, mgk3d_interpolate(mg->core.stream, mg->core.dtype, F->v, F->g, C->v, C->g, add, colour_mask, lo, hi, NULL));
     PROF_END(mg);
     if (!F->dist) return MG_OK;
-    /* a level the temporally blocked smoother takes next fetches its (deeper) ghost planes itself */
     /* The owned planes of the fine v changed: the neighbours' ghost copies are stale.  A level the temporally blocked
        smoother takes next fetches its (deeper) ghost planes itself, and whoever else reads ghost planes refreshes them
        first (ensure_v_ghosts); otherwise the colour that changed travels now. */
     F->vg_deep = 0;
-    if (level_takes_pipe(mg, F) || !F->vg_valid) {
+    if (level_path(mg, fine_level).relax == MG_RELAX_PIPE || !F->vg_valid) {
         F->vg_valid = 0;
         return MG_OK;
     }
@@ -1422,8 +1433,8 @@ int mg3d_set_to_value(mg3d_t* mg, int level, int field, double value, int modify
 static int vcycle_rec(mg3d_t* mg, int level, int v1, int v2)
 {
     int st;
-    mg_level3d* L0 = &mg->lv[level];
-    if (L0->g.n <= MGK3D_TAIL_N && !L0->dist && mg->core.nlevels - level <= MGK3D_TAIL_MAX_LEVELS && mg->smoother != MG_SMOOTHER_JACOBI) {
+    const mg_path3d p = level_path(mg, level);
+    if (p.tail) {
         /* the coarse tail: the whole recursion from here down in one launch of one CTA */
         mg_geom3d g[MGK3D_TAIL_MAX_LEVELS];
         mg_coef3d c[MGK3D_TAIL_MAX_LEVELS];
@@ -1443,10 +1454,8 @@ static int vcycle_rec(mg3d_t* mg, int level, int v1, int v2)
     if (level != mg->core.nlevels - 1) {
         if ((st = residual_restrict_level(mg, level, v1 > 0 && relax_overlaps(mg, level + 1)))) return st;
         if ((st = vcycle_rec(mg, level + 1, v1, v2))) return st;
-        /* prolongation + correction ride on the first pass of the post-smoothing where the temporally blocked smoother runs */
         if (correction_fuses(mg, level, v2)) return relax_level_ex(mg, level, v2, 1);
-        /* the colour-0 half of the correction is dead when a red-black post-smoothing sweep follows */
-        if ((st = interpolate_level(mg, level, 1, (v2 > 0 && mg->smoother != MG_SMOOTHER_JACOBI && !mg->full_correction) ? 2 : 3,
+        if ((st = interpolate_level(mg, level, 1, (v2 > 0 && p.correct_colour1) ? 2 : 3,
                                     v2 > 0 && relax_overlaps(mg, level))))
             return st;
     }
